@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py -- FLAC encode/decode throughput of the hot path on B200 (contract: see the task brief).
+"""bench.py -- FLAC encode/decode throughput of the hot path on B200; prints one JSON result line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--streams S] [--samples L]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): float32 detector timestreams (1000, 1M) quantised with
 quanta = 1e-4, full encode + decode.  One "step" = one encode pass + one decode pass over the batch
@@ -19,6 +20,11 @@ roofline= the slower of the two kernel groups: the encoder sequence (k_enc_analy
 cpu_baseline = the CPU oracle port (restatement of the reference's OpenMP-over-streams loops) timed on
           this box's host cores on a bounded sample of the same workload.
 `--impl reference` times that CPU implementation as the whole job (rank 0 only).
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (see dump_outputs) as DIR/<name>.npy, so
+          that two builds can be compared output for output: the inputs are seeded and identical from run to run.
+
+The benchmark writes nothing into the source tree (it may be read-only): no bytecode caches, and outputs only where
+--dump-outputs points.
 """
 import argparse
 import json
@@ -30,6 +36,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -91,6 +98,41 @@ def make_tod_torch(n_stream, n_samp, seed, device):
         out[i:j] = torch.randn((j - i, n_samp), generator=g, device=device)
         out[i:j] += dc[i:j] + scale[i:j] * wave
     return out
+
+
+# ---------------------------------------------------------------------------------------------------
+# --dump-outputs: what a caller of the timed path receives, as float32 / float64 .npy files
+# ---------------------------------------------------------------------------------------------------
+DUMP_ROWS = 4                 # streams whose decoded samples and compressed bytes are written
+DUMP_ELEMS = 1 << 22          # cap per sampled array (16 MB as float32)
+DUMP_STREAMS = 1 << 20        # cap on the per-stream arrays (24 MB for all four)
+
+
+def dump_outputs(out_dir, comp, starts, nbytes, off, gain, decoded, n_stream, n_samp):
+    """Write the last timed step's results: encode_device's (compressed bytes, stream starts, stream byte counts,
+    offsets, gains) and decode_device's float32 samples.  Large outputs are sampled with a fixed seed, so the files
+    stay below 64 MB in all and are comparable between builds: the decoded samples and compressed bytes of
+    DUMP_ROWS streams (each cut to DUMP_ELEMS // DUMP_ROWS values), and the per-stream arrays of at most
+    DUMP_STREAMS streams.  Bytes and integer offsets are stored as float32 / float64, which hold them exactly."""
+    rng = np.random.default_rng(SEED)
+    rows = np.sort(rng.choice(n_stream, min(n_stream, DUMP_ROWS), replace=False))
+    per_row = DUMP_ELEMS // len(rows)
+    streams = np.arange(n_stream) if n_stream <= DUMP_STREAMS else np.sort(rng.choice(n_stream, DUMP_STREAMS, replace=False))
+    h_starts = starts.reshape(-1).cpu().numpy()
+    h_nbytes = nbytes.reshape(-1).cpu().numpy()
+    dec = decoded.reshape(n_stream, n_samp)
+    pieces = [comp[int(h_starts[r]):int(h_starts[r]) + min(int(h_nbytes[r]), per_row)] for r in rows]
+    arrays = {
+        "decoded": dec[rows.tolist(), :min(n_samp, per_row)].cpu().numpy().astype(np.float32),
+        "compressed": np.concatenate([p.cpu().numpy() for p in pieces]).astype(np.float32),
+        "stream_starts": h_starts[streams].astype(np.float64),
+        "stream_nbytes": h_nbytes[streams].astype(np.float64),
+        "stream_offsets": off.reshape(-1).cpu().numpy()[streams].astype(np.float32),
+        "stream_gains": gain.reshape(-1).cpu().numpy()[streams].astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -400,6 +442,8 @@ def run_ours(args):
     dec_ms, dec_n = ctx.profile_ms(1)
     ctx.profile(False)
     comp_bytes = int(comp.numel())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, comp, starts, nbytes, off, gain, out, n_stream, n_samp)
     del comp, out
 
     tt = torch.tensor([t_enc, t_dec, wall], dtype=torch.float64, device=dev)
@@ -491,7 +535,7 @@ def run_ours(args):
         back = far.to_array()
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     h2d = d2h = 0
     for _ in range(e2e_steps):
         del far, back
@@ -605,7 +649,13 @@ def main():
     ap.add_argument("--samples", type=int, default=1000000)
     ap.add_argument("--e2e-streams", type=int, default=1000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (sampled, float32/float64) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

@@ -46,17 +46,31 @@ def test_sass_is_sm100(so_path):
     assert "sm_100a" in out
 
 
+_NO_CPU_FALLBACK = """
+import numpy as np
+import pytest
+import torch
+
+assert not torch.cuda.is_available()
+import flacarray_b200 as fa
+
+with pytest.raises(RuntimeError, match="no CPU fallback"):
+    fa.array_compress(np.zeros((2, 64), np.int32))
+with pytest.raises(RuntimeError, match="no CPU fallback"):
+    fa.float_to_int(np.zeros((2, 64), np.float32), quanta=1e-3)
+"""
+
+
 def test_no_cpu_fallback():
-    import torch
+    """Without a CUDA device the product path raises.  Runs in a child process that sees no device, so that it
+    checks the same on a machine with a GPU."""
+    import subprocess
+    import sys
 
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import flacarray_b200 as fa
-
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        fa.array_compress(np.zeros((2, 64), np.int32))
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        fa.float_to_int(np.zeros((2, 64), np.float32), quanta=1e-3)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-s", "-c", _NO_CPU_FALLBACK], cwd=ROOT, env=env, capture_output=True,
+                         text=True, timeout=600)
+    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-4000:]
 
 
 def test_argument_validation_matches_reference():
