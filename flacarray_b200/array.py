@@ -15,7 +15,7 @@ import copy
 import numpy as np
 
 from .compress import array_compress
-from .decompress import array_decompress_slice
+from .decompress import array_decompress_slice, array_decompress_windows
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -329,6 +329,32 @@ class FlacArray:
         if keep is not None and keep_indices:
             return (arr, indices)
         return arr
+
+    def to_windows(self, streams, first, last):
+        """Decompress many sample windows of local streams in one call.
+
+        Window i is samples [first[i], last[i]) of stream streams[i].  `streams` is either flat C-order indices over
+        the leading shape or a tuple of index arrays, one per leading axis (as np.nonzero returns); a 1-D array has the
+        single stream 0.  `first` / `last` may be scalars.  Returns (data, offsets) like array_decompress_windows:
+        window i is data[offsets[i]:offsets[i + 1]] in the array's dtype.
+        """
+        if isinstance(streams, tuple):
+            if len(streams) != len(self._leading_shape):
+                raise RuntimeError(
+                    f"streams has {len(streams)} index arrays for {len(self._leading_shape)} leading axes")
+            idx = [np.asarray(a, dtype=np.int64).reshape(-1) for a in streams]
+            if len({a.size for a in idx}) > 1:
+                raise RuntimeError("the index arrays of streams must have the same length")
+            for ax, (a, n) in enumerate(zip(idx, self._leading_shape)):
+                if a.size and (int(a.min()) < 0 or int(a.max()) >= n):
+                    raise RuntimeError(f"window stream index out of range on leading axis {ax} of length {n}")
+            streams = np.ravel_multi_index(tuple(idx), self._leading_shape) if idx and idx[0].size else np.zeros(0, np.int64)
+        starts = np.asarray(self._stream_starts).reshape(-1)
+        nbytes = np.asarray(self._stream_nbytes).reshape(-1)
+        offsets = None if self._stream_offsets is None else np.asarray(self._stream_offsets).reshape(-1)
+        gains = None if self._stream_gains is None else np.asarray(self._stream_gains).reshape(-1)
+        return array_decompress_windows(self._compressed, self._stream_size, starts, nbytes, streams, first, last,
+                                        stream_offsets=offsets, stream_gains=gains, is_int64=self._is_int64)
 
     @classmethod
     def from_array(cls, arr, level=5, quanta=None, precision=None, mpi_comm=None, use_threads=False):

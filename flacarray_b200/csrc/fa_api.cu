@@ -339,21 +339,23 @@ __global__ void __launch_bounds__(kSyncThreads) k_dec_sync(const DecParams P) {
 
 constexpr int kDecThreads = 128;
 
-__global__ void __launch_bounds__(kDecThreads) k_dec_frames(const DecParams P, int64_t nwin) {
-    // one thread per (stream, frame index inside the sample window)
+template <bool WIN>
+__global__ void __launch_bounds__(kDecThreads) k_dec_frames(const DecParams P, const WinParams W, int64_t nwin) {
+    // one thread per work item (stream, frame index inside the sample window), see resolve_item
     int64_t idx = (int64_t)blockIdx.x * kDecThreads + threadIdx.x;
-    int64_t k = idx / nwin;
-    if (k >= P.n_sel) return;
+    const WorkItem it = resolve_item<WIN>(P, W, nwin, idx);
+    const int64_t k = it.k;
+    if (k < 0) return;
     if (P.stream_flag[k] != 0) return;
     int bs = P.meta[k].blocksize;
-    int64_t j0 = P.first / bs, j1 = (P.first + P.n_decode - 1) / bs;
-    if (j1 - j0 + 1 > nwin) {  // blocksize differs from the host's hint: leave the stream to the walker
-        if (idx % nwin == 0) atomicOr(&P.stream_flag[k], 1);
+    int64_t j0 = it.first / bs, j1 = (it.first + it.n - 1) / bs;
+    if (j1 - j0 + 1 > it.nwin) {  // blocksize differs from the host's hint: leave the stream to the walker
+        if (it.jrel == 0) atomicOr(&P.stream_flag[k], 1);
         return;
     }
-    int64_t j = j0 + idx % nwin;
+    int64_t j = j0 + it.jrel;
     if (j > j1) return;
-    frame_body(P, k, j);
+    frame_body(P, k, j, it.first, it.n, it.out);
 }
 
 // throughput path: one warp = 32 (stream, frame) items, see fa_decode_tile.h.
@@ -368,18 +370,21 @@ __global__ void __launch_bounds__(kDecThreads) k_dec_frames(const DecParams P, i
 #ifndef FAB_DEC_CTAS
 #define FAB_DEC_CTAS (20 / FAB_TILE_WARPS)
 #endif
-__global__ void __launch_bounds__(kTileWarps * 32, FAB_DEC_CTAS) k_dec_tile(const TileParams P) {
+// (WIN: the item space of fab_decode_windows, `total` items)
+template <bool WIN>
+__global__ void __launch_bounds__(kTileWarps * 32, FAB_DEC_CTAS) k_dec_tile(const TileParams P, int64_t total) {
     __shared__ TileShared ws[kTileWarps];
     int64_t item0 = ((int64_t)blockIdx.x * kTileWarps + (threadIdx.x >> 5)) * 32;
-    if (item0 >= P.D.n_sel * P.nwin) return;
-    tile_warp_body(P, item0, &ws[threadIdx.x >> 5]);
+    if (item0 >= total) return;
+    tile_warp_body<WIN>(P, item0, &ws[threadIdx.x >> 5]);
 }
 
 // frame CRC-16 of every (stream, frame) item: one warp per item, see crc_frame_warp
-__global__ void __launch_bounds__(128) k_dec_crc(const TileParams P) {
+template <bool WIN>
+__global__ void __launch_bounds__(128) k_dec_crc(const TileParams P, int64_t total) {
     int64_t idx = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
-    if (idx >= P.D.n_sel * P.nwin) return;
-    crc_frame_warp(P, idx);
+    if (idx >= total) return;
+    crc_frame_warp<WIN>(P, idx);
 }
 
 // int32 -> float32 for the sample ranges that were NOT written by the fused tile path (frames left to
@@ -423,6 +428,92 @@ __global__ void __launch_bounds__(256) k_restore_fixup(const TileParams P) {
 __global__ void k_dec_walker(const DecParams P) {
     int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k < P.n_sel) walker_body(P, k);
+}
+
+// ---- fab_decode_windows ------------------------------------------------------------------------------
+// Window records -> item space: a record that names a stream slot outside [0, n_sel) or a range outside the stream
+// sets ERROR_DECODE_SAMPLE_RANGE and gets no items; W.item0 = exclusive prefix of the frame counts (hinted blocksize),
+// W.item0[n_win] = the number of items.  One CTA, chunks of 1024 windows with a running carry.
+constexpr int kWinScanThreads = 1024;
+__global__ void __launch_bounds__(kWinScanThreads) k_win_prep(const WinParams W, int64_t n_sel, int64_t stream_size, int* err) {
+    __shared__ long long wpre[kWinScanThreads / 32];
+    __shared__ long long ctot;
+    long long* item0 = const_cast<long long*>(W.item0);
+    const int ln = threadIdx.x & 31, wp = threadIdx.x >> 5;
+    long long carry = 0;
+    for (int64_t w0 = 0; w0 < W.n_win; w0 += kWinScanThreads) {
+        const int64_t w = w0 + threadIdx.x;
+        long long cnt = 0;
+        if (w < W.n_win) {
+            if (win_valid(W, w, n_sel, stream_size)) cnt = frames_in_window(W.first[w], W.last[w] - W.first[w], W.bsh);
+            else atom_or_global(err, kErrDecodeSampleRange);
+        }
+        long long inc = cnt;       // inclusive scan inside the warp, then over the warps' totals
+        for (int d = 1; d < 32; d <<= 1) {
+            long long v = __shfl_up_sync(0xffffffffu, inc, d);
+            if (ln >= d) inc += v;
+        }
+        if (ln == 31) wpre[wp] = inc;
+        __syncthreads();
+        if (wp == 0) {
+            const long long t = wpre[ln];
+            long long ti = t;
+            for (int d = 1; d < 32; d <<= 1) {
+                long long v = __shfl_up_sync(0xffffffffu, ti, d);
+                if (ln >= d) ti += v;
+            }
+            wpre[ln] = ti - t;
+            if (ln == 31) ctot = ti;
+        }
+        __syncthreads();
+        if (w < W.n_win) item0[w] = carry + wpre[wp] + inc - cnt;
+        carry += ctot;
+        __syncthreads();           // (wpre / ctot are rewritten by the next chunk)
+    }
+    if (threadIdx.x == 0) item0[W.n_win] = carry;
+}
+
+// fab_decode_windows: the frames of the windows, one thread per work item (walker-decoded streams: per window)
+__global__ void k_dec_walker_win(const DecParams P, const WinParams W) {
+    const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= W.n_win || !win_valid(W, w, P.n_sel, P.stream_size)) return;
+    const long long first = W.first[w], n = W.last[w] - first;
+    if (n > 0) walker_body(P, W.stream[w], first, n, W.out[w]);
+}
+
+// Windowed int -> float, one warp per work item over the item's samples.  F64: every sample (the decoders wrote int64
+// everywhere).  float32: only what the fused tile path did not restore -- frames flagged for the general decoder, and the
+// whole window of a stream left to the walker (there the items cover the window in hinted-blocksize pieces).
+template <bool F64>
+__global__ void __launch_bounds__(128) k_restore_win(const TileParams P, int64_t total) {
+    const int64_t idx = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (idx >= total) return;
+    const DecParams& D = P.D;
+    const WorkItem it = resolve_item<true>(D, P.W, P.nwin, idx);
+    const int64_t k = it.k;
+    if (k < 0) return;
+    const int sflag = D.stream_flag[k];
+    const bool whole = F64 || sflag != 0;
+    if (!whole && D.meta[k].blocksize <= 0) return;
+    if (!F64 && sflag == 4) return;
+    const int64_t bs = whole ? P.W.bsh : D.meta[k].blocksize;
+    const int64_t j = it.first / bs + it.jrel;
+    if (!whole && (j >= D.nframes_cap || !P.frame_flag[k * (int64_t)D.nframes_cap + j])) return;
+    int64_t lo = j * bs - it.first, hi = lo + bs;
+    if (lo < 0) lo = 0;
+    if (hi > it.n) hi = it.n;
+    const int ln = threadIdx.x & 31;
+    if constexpr (F64) {
+        const double off = ((const double*)P.offsets)[k], coeff = restore_coeff_f64(((const double*)P.gains)[k]);
+        const long long* in = (const long long*)D.data + it.out;
+        double* out = (double*)D.data + it.out;
+        for (int64_t i = lo + ln; i < hi; i += 32) out[i] = restore_f64(in[i], off, coeff);
+    } else {
+        const float off = P.offsets[k], coeff = restore_coeff_f32(P.gains[k]);
+        const int32_t* in = D.data + it.out;
+        float* out = (float*)D.data + it.out;
+        for (int64_t i = lo + ln; i < hi; i += 32) out[i] = restore_f32(in[i], off, coeff);
+    }
 }
 
 __global__ void k_max_i64(const long long* __restrict__ v, int64_t n, long long* __restrict__ out) {
@@ -949,6 +1040,52 @@ extern "C" int64_t fab_decode_workspace_bytes(int64_t n_stream, int64_t stream_s
     return (int64_t)dec_workspace(n_stream, cap).total;
 }
 
+// Stages 1 and 2 of a decode, once per stream slot: metadata + frame offsets (k_dec_meta), then the sync scan of the
+// streams without a frame-size table (k_dec_sync, grid.y split at 65535 streams).
+static void dec_index_streams(fab_ctx* ctx, const DecParams& P, int64_t max_nbytes, cudaStream_t st) {
+    const int64_t n_stream = P.n_sel;
+    k_dec_meta<<<(unsigned)((n_stream + 3) / 4), 128, 0, st>>>(P);
+    ctx->launches++;
+    int64_t per_cta = (int64_t)kSyncThreads * kSyncBytesPerThread;
+    int64_t gx = (max_nbytes + per_cta - 1) / per_cta;
+    // streams carrying a frame-size table leave at once: keep the grid near one wave-set of CTAs and
+    // let the CTAs of a foreign stream stride over its chunks
+    gx = std::max<int64_t>(1, std::min<int64_t>(gx, (148 * 32 + n_stream - 1) / n_stream));
+    for (int64_t s0 = 0; s0 < n_stream; s0 += 65535) {
+        int64_t ns = std::min<int64_t>(65535, n_stream - s0);
+        DecParams Q = P;
+        Q.starts += s0; Q.nbytes += s0; Q.meta += s0; Q.frame_off += s0 * (int64_t)(P.nframes_cap + 1); Q.stream_flag += s0;
+        Q.n_sel = ns;
+        dim3 grid((unsigned)gx, (unsigned)ns);
+        k_dec_sync<<<grid, kSyncThreads, 0, st>>>(Q);
+        ctx->launches++;
+    }
+}
+
+// Stage 3 over `total` work items (resolve_item): warp-tile decoder, its CRC pass next to it on the second stream, then
+// the general per-thread decoder on the frames the tile path flagged.  TP.frame_flag must be cleared.
+template <bool WIN>
+static int dec_items(fab_ctx* ctx, const TileParams& TP, int64_t total, cudaStream_t st) {
+    int64_t per_cta = (int64_t)kTileWarps * 32;
+    prof_begin(ctx, 1, st);
+    FAB_CUDA(ctx, cudaEventRecord(ctx->ev_fork, st));
+    k_dec_tile<WIN><<<(unsigned)((total + per_cta - 1) / per_cta), kTileWarps * 32, 0, st>>>(TP, total);
+    // the CRC pass only needs the frame table: it runs on the second stream, queued behind the tile
+    // kernel's launch so that its CTAs fill the SMs the decoder's last partial wave leaves idle
+    FAB_CUDA(ctx, cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
+    k_dec_crc<WIN><<<(unsigned)((total + 3) / 4), 128, 0, ctx->aux>>>(TP, total);
+    FAB_CUDA(ctx, cudaEventRecord(ctx->ev_join, ctx->aux));
+    FAB_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
+    prof_end(ctx, st);
+    ctx->launches += 2;
+    // general per-thread decoder: only the frames the tile path flagged
+    DecParams P = TP.D;
+    P.frame_flag = TP.frame_flag;
+    k_dec_frames<WIN><<<(unsigned)((total + kDecThreads - 1) / kDecThreads), kDecThreads, 0, st>>>(P, TP.W, TP.nwin);
+    ctx->launches++;
+    return 0;
+}
+
 extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
                           int64_t n_stream, int64_t stream_size, int is_int64, int64_t first_sample, int64_t last_sample,
                           void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes,
@@ -995,24 +1132,7 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
     P.meta = (StreamMeta*)scr; P.frame_off = (long long*)(scr + meta_b); P.nframes_cap = nframes_cap;
     P.stream_flag = (int*)(scr + meta_b + fo_b); P.err = ctx->d_err; P.verify_crc16 = 1; P.frame_flag = frame_flag;
 
-    k_dec_meta<<<(unsigned)((n_stream + 3) / 4), 128, 0, st>>>(P);
-    ctx->launches++;
-    {
-        int64_t per_cta = (int64_t)kSyncThreads * kSyncBytesPerThread;
-        int64_t gx = (max_nbytes + per_cta - 1) / per_cta;
-        // streams carrying a frame-size table leave at once: keep the grid near one wave-set of CTAs and
-        // let the CTAs of a foreign stream stride over its chunks
-        gx = std::max<int64_t>(1, std::min<int64_t>(gx, (148 * 32 + n_stream - 1) / n_stream));
-        for (int64_t s0 = 0; s0 < n_stream; s0 += 65535) {
-            int64_t ns = std::min<int64_t>(65535, n_stream - s0);
-            DecParams Q = P;
-            Q.starts += s0; Q.nbytes += s0; Q.meta += s0; Q.frame_off += s0 * (int64_t)(nframes_cap + 1); Q.stream_flag += s0;
-            Q.n_sel = ns;
-            dim3 grid((unsigned)gx, (unsigned)ns);
-            k_dec_sync<<<grid, kSyncThreads, 0, st>>>(Q);
-            ctx->launches++;
-        }
-    }
+    dec_index_streams(ctx, P, max_nbytes, st);
     const bool fuse_restore = d_offsets && d_gains && !is_int64;
     TileParams TP;
     {
@@ -1023,21 +1143,9 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
         FAB_CUDA(ctx, cudaMemsetAsync(frame_flag, 0, fflag_b, st));
         TP.D = P; TP.j0 = first_decode / bsh; TP.nwin = nwin; TP.frame_flag = frame_flag;
         TP.restore = fuse_restore ? 1 : 0; TP.offsets = (const float*)d_offsets; TP.gains = (const float*)d_gains;
-        int64_t per_cta = (int64_t)kTileWarps * 32;
-        prof_begin(ctx, 1, st);
-        FAB_CUDA(ctx, cudaEventRecord(ctx->ev_fork, st));
-        k_dec_tile<<<(unsigned)((total + per_cta - 1) / per_cta), kTileWarps * 32, 0, st>>>(TP);
-        // the CRC pass only needs the frame table: it runs on the second stream, queued behind the tile
-        // kernel's launch so that its CTAs fill the SMs the decoder's last partial wave leaves idle
-        FAB_CUDA(ctx, cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
-        k_dec_crc<<<(unsigned)((total + 3) / 4), 128, 0, ctx->aux>>>(TP);
-        FAB_CUDA(ctx, cudaEventRecord(ctx->ev_join, ctx->aux));
-        FAB_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_join, 0));
-        prof_end(ctx, st);
-        ctx->launches += 2;
-        // general per-thread decoder: only the frames the tile path flagged
-        k_dec_frames<<<(unsigned)((total + kDecThreads - 1) / kDecThreads), kDecThreads, 0, st>>>(P, nwin);
-        ctx->launches++;
+        TP.W = WinParams{};
+        int rc2 = dec_items<false>(ctx, TP, total, st);
+        if (rc2) return rc2;
     }
     k_dec_walker<<<(unsigned)((n_stream + 31) / 32), 32, 0, st>>>(P);
     ctx->launches++;
@@ -1065,6 +1173,88 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
                                                                (double*)d_out + s0 * n_decode);
             ctx->launches++;
         }
+    }
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+// Workspace of one fab_decode_windows call: fab_decode's layout for the stream slots | item0 of the windows.  The item
+// space itself needs no storage (frame flags are kept per stream slot and frame), so total_items does not change it.
+static size_t win_item0_bytes(int64_t n_win) { return align256((size_t)(n_win + 1) * 8); }
+extern "C" int64_t fab_decode_windows_workspace_bytes(int64_t n_stream, int64_t stream_size, int64_t n_win,
+                                                      int64_t total_items, int blocksize_hint) {
+    int cap = 0;
+    if (n_stream <= 0 || stream_size <= 0 || n_win < 0 || total_items < 0 || dec_frames_cap(stream_size, blocksize_hint, &cap))
+        return 0;
+    return (int64_t)(dec_workspace(n_stream, cap).total + win_item0_bytes(n_win));
+}
+
+extern "C" int fab_decode_windows(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                                  int64_t n_stream, int64_t stream_size, int is_int64, const int64_t* d_win_stream,
+                                  const int64_t* d_win_first, const int64_t* d_win_last, const int64_t* d_win_out,
+                                  int64_t n_win, void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes,
+                                  int blocksize_hint, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    if (n_win < 0) return ERROR_DECODE_SAMPLE_RANGE;
+    if (n_win == 0) return 0;
+    if (n_stream <= 0) return ERROR_ZERO_NSTREAM;
+    if (stream_size <= 0) return ERROR_ZERO_STREAMSIZE;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nch = is_int64 ? 2 : 1;
+    int nframes_cap = 0;
+    if (dec_frames_cap(stream_size, blocksize_hint, &nframes_cap)) return ERROR_ALLOC;
+    const int bsh = std::max(16, blocksize_hint > 0 ? blocksize_hint : 4096);
+
+    const DecWorkspace DW = dec_workspace(n_stream, nframes_cap);
+    unsigned char* scr;
+    int rc = ctx_scratch(ctx, DW.total + win_item0_bytes(n_win), &scr, st);
+    if (rc) return rc;
+    unsigned char* frame_flag = scr + DW.meta_b + DW.fo_b + DW.flag_b;
+    long long* d_max = (long long*)(frame_flag + DW.fflag_b);
+
+    WinParams W;
+    W.stream = (const long long*)d_win_stream; W.first = (const long long*)d_win_first; W.last = (const long long*)d_win_last;
+    W.out = (const long long*)d_win_out; W.item0 = (const long long*)(scr + DW.total); W.n_win = n_win; W.bsh = bsh;
+    k_win_prep<<<1, kWinScanThreads, 0, st>>>(W, n_stream, stream_size, ctx->d_err);
+    ctx->launches++;
+    // the grids are sized by the number of items: one round trip for it (and for the longest stream when not given)
+    long long h_total = 0, h_max = 0;
+    if (max_nbytes <= 0) {
+        k_max_i64<<<1, 256, 0, st>>>((const long long*)d_nbytes, n_stream, d_max);
+        ctx->launches++;
+        FAB_CUDA(ctx, cudaMemcpyAsync(&h_max, d_max, 8, cudaMemcpyDeviceToHost, st));
+    }
+    FAB_CUDA(ctx, cudaMemcpyAsync(&h_total, W.item0 + n_win, 8, cudaMemcpyDeviceToHost, st));
+    FAB_CUDA(ctx, cudaStreamSynchronize(st));
+    if (max_nbytes <= 0) max_nbytes = h_max;
+    const int64_t total = h_total;
+    if (total == 0) {           // every window empty (or rejected: the error mask says so)
+        FAB_CUDA(ctx, cudaGetLastError());
+        return 0;
+    }
+
+    DecParams P;
+    P.bytes = d_bytes; P.starts = (const long long*)d_starts; P.nbytes = (const long long*)d_nbytes;
+    P.n_sel = n_stream; P.stream_size = stream_size; P.nch = nch;
+    P.first = 0; P.n_decode = 0; P.data = (int32_t*)d_out; P.crc = ctx->d_crc;      // (windows carry their own ranges)
+    P.meta = (StreamMeta*)scr; P.frame_off = (long long*)(scr + DW.meta_b); P.nframes_cap = nframes_cap;
+    P.stream_flag = (int*)(scr + DW.meta_b + DW.fo_b); P.err = ctx->d_err; P.verify_crc16 = 1; P.frame_flag = frame_flag;
+    dec_index_streams(ctx, P, max_nbytes, st);
+
+    const bool fuse_restore = d_offsets && d_gains && !is_int64;
+    TileParams TP;
+    FAB_CUDA(ctx, cudaMemsetAsync(frame_flag, 0, DW.fflag_b, st));
+    TP.D = P; TP.j0 = 0; TP.nwin = 0; TP.frame_flag = frame_flag;
+    TP.restore = fuse_restore ? 1 : 0; TP.offsets = (const float*)d_offsets; TP.gains = (const float*)d_gains;
+    TP.W = W;
+    rc = dec_items<true>(ctx, TP, total, st);
+    if (rc) return rc;
+    k_dec_walker_win<<<(unsigned)((n_win + 127) / 128), 128, 0, st>>>(P, W);
+    ctx->launches++;
+    if (d_offsets && d_gains) {
+        if (fuse_restore) k_restore_win<false><<<(unsigned)((total + 3) / 4), 128, 0, st>>>(TP, total);
+        else k_restore_win<true><<<(unsigned)((total + 3) / 4), 128, 0, st>>>(TP, total);
+        ctx->launches++;
     }
     FAB_CUDA(ctx, cudaGetLastError());
     return 0;

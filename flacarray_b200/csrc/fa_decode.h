@@ -264,6 +264,69 @@ struct DecParams {
 // number of frames / size of frame j for a fixed-blocksize stream
 FA_D int64_t frames_in_stream(int64_t stream_size, int bs) { return (stream_size + bs - 1) / bs; }
 
+// Per-window sample ranges (fab_decode_windows).  Window w reads samples [first[w], last[w]) of stream slot stream[w] and
+// writes them from output element out[w] on.  Its work items are the frames the window overlaps for the hinted
+// blocksize `bsh`; item0 is the exclusive prefix of those counts, so an item finds its window by a binary search and
+// windows of any length share warps.  Records that fail win_valid have no items.
+struct WinParams {
+    const long long* stream;   // [n_win] stream slot u in [0, n_sel)
+    const long long* first;    // [n_win]
+    const long long* last;     // [n_win]
+    const long long* out;      // [n_win] output element of the window's first sample
+    const long long* item0;    // [n_win + 1] first work item of every window; item0[n_win] = number of items
+    int64_t n_win;
+    int bsh;
+};
+
+FA_D bool win_valid(const WinParams& W, int64_t w, int64_t n_sel, int64_t stream_size) {
+    const long long u = W.stream[w], a = W.first[w], b = W.last[w];
+    return u >= 0 && u < n_sel && a >= 0 && b <= stream_size && a <= b;
+}
+
+// frames of [first, first + n) for blocksize bs (0 for an empty window)
+FA_D int64_t frames_in_window(int64_t first, int64_t n, int64_t bs) {
+    return n > 0 ? (first + n - 1) / bs - first / bs + 1 : 0;
+}
+
+// One work item of the decoder's index space: frame `jrel` (counted from the window's first frame) of the window
+// [first, first + n) of stream slot k, whose sample `first` goes to output element `out`.  k < 0: no item.
+struct WorkItem {
+    int64_t k, jrel, first, n, out, nwin;
+};
+
+// WIN = false: fab_decode's uniform case, every selected stream with the same window and nwin items each, packed rows.
+// WIN = true: the windows of W.
+template <bool WIN>
+FA_D WorkItem resolve_item(const DecParams& D, const WinParams& W, int64_t nwin, int64_t idx) {
+    WorkItem it;
+    if constexpr (!WIN) {
+        it.k = idx / nwin;
+        it.jrel = idx % nwin;
+        it.first = D.first;
+        it.n = D.n_decode;
+        it.out = it.k * D.n_decode;
+        it.nwin = nwin;
+        if (it.k >= D.n_sel) it.k = -1;
+    } else {
+        it.k = -1;
+        it.jrel = it.first = it.n = it.out = it.nwin = 0;
+        if (idx >= W.item0[W.n_win]) return it;
+        int64_t lo = 0, hi = W.n_win - 1;      // last window whose first item is <= idx (empty windows share it with the next)
+        while (lo < hi) {
+            const int64_t mid = (lo + hi + 1) >> 1;
+            if (W.item0[mid] <= idx) lo = mid;
+            else hi = mid - 1;
+        }
+        it.k = W.stream[lo];
+        it.jrel = idx - W.item0[lo];
+        it.first = W.first[lo];
+        it.n = W.last[lo] - it.first;
+        it.out = W.out[lo];
+        it.nwin = W.item0[lo + 1] - W.item0[lo];
+    }
+    return it;
+}
+
 // ---- stage 1: one thread per selected stream: metadata + (if present) the faB2 frame-size table ----
 FA_D void meta_body(const DecParams& P, int64_t k) {
     const uint8_t* buf = P.bytes + P.starts[k];
@@ -368,7 +431,8 @@ FA_D void sync_scan_warp(const DecParams& P, int64_t k, int64_t w, int64_t nw) {
 }
 
 // ---- stage 3: one thread per (selected stream, frame overlapping the sample window) ---------------
-FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) {
+// (frame j of stream k for the window [first, first + n) that starts at output element `out`)
+FA_D void frame_body(const DecParams& P, int64_t k, int64_t j, int64_t first, int64_t n, int64_t out) {
     if (P.stream_flag[k] != 0) return;
     if (P.frame_flag && !P.frame_flag[k * (int64_t)P.nframes_cap + j]) return;
     const StreamMeta m = P.meta[k];
@@ -378,8 +442,8 @@ FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) {
     const uint8_t* buf = P.bytes + P.starts[k];
     const uint8_t* end = buf + P.nbytes[k];
     int64_t s0 = j * (int64_t)m.blocksize;  // first sample of the frame
-    int32_t* base = P.data + (k * P.n_decode + (s0 - P.first)) * P.nch;
-    int64_t lo = P.first - s0, hi = P.first + P.n_decode - s0;
+    int32_t* base = P.data + (out + (s0 - first)) * P.nch;
+    int64_t lo = first - s0, hi = first + n - s0;
     FrameHdr fh;
     int64_t len = decode_frame_general(buf + off, end, P.crc, m.bps, P.nch, fh, base,
                                        (int)(lo < 0 ? 0 : lo), (int)(hi > m.blocksize ? m.blocksize : hi),
@@ -388,22 +452,24 @@ FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) {
     if (ok && next >= 0 && off + len != next) ok = false;
     if (!ok) atom_or_global(&P.stream_flag[k], 2);
 }
+FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) { frame_body(P, k, j, P.first, P.n_decode, k * P.n_decode); }
 
 // ---- stage 4: sequential walker for streams the parallel path could not index -----------------------
 // (variable blocksize, ambiguous sync candidates, failed chain check).  Always verifies CRC-16.
-FA_D void walker_body(const DecParams& P, int64_t k) {
+// Decodes the window [first, first + n) of stream k to output element `out` on.
+FA_D void walker_body(const DecParams& P, int64_t k, int64_t first, int64_t n, int64_t out) {
     int flag = P.stream_flag[k];
     if (flag == 0 || flag == 4) return;
     const StreamMeta m = P.meta[k];
     const uint8_t* buf = P.bytes + P.starts[k];
     const uint8_t* end = buf + P.nbytes[k];
-    int64_t pos = m.first_frame, sample = 0, last = P.first + P.n_decode;
+    int64_t pos = m.first_frame, sample = 0, last = first + n;
     uint64_t expect = 0;
     while (sample < last) {
         if (pos >= P.nbytes[k]) { atom_or_global(P.err, kErrDecodeProcess); return; }
         FrameHdr fh;
-        int32_t* base = P.data + (k * P.n_decode + (sample - P.first)) * P.nch;
-        int64_t lo = P.first - sample, hi = last - sample;
+        int32_t* base = P.data + (out + (sample - first)) * P.nch;
+        int64_t lo = first - sample, hi = last - sample;
         int64_t len = decode_frame_general(buf + pos, end, P.crc, m.bps, P.nch, fh, base, (int)(lo < 0 ? 0 : lo),
                                            (int)(hi > 65536 ? 65536 : hi), true);
         if (len < 0) { atom_or_global(P.err, kErrDecodeProcess); return; }
@@ -416,5 +482,6 @@ FA_D void walker_body(const DecParams& P, int64_t k) {
         pos += len;
     }
 }
+FA_D void walker_body(const DecParams& P, int64_t k) { walker_body(P, k, P.first, P.n_decode, k * P.n_decode); }
 
 }  // namespace fa

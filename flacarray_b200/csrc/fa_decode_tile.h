@@ -426,6 +426,7 @@ struct TileParams {
     int restore;                // 1: nch == 1 and D.data receives float32 (offsets/gains given)
     const float* offsets;
     const float* gains;
+    WinParams W;                // the windows (WIN instantiations only)
 };
 
 // Decode + flush all tiles of one channel pass with a compile-time upper bound on the predictor order.
@@ -522,15 +523,17 @@ FA_D void tile_channel_pass(const TileParams& P, TileShared* ws, BitRdC& br, Til
     }
 }
 
-// One warp: 32 consecutive (stream, frame) work items.  `ws` = this warp's shared storage, `T` = CRC
-// slice tables in shared memory.
+// One warp: 32 consecutive work items (resolve_item: WIN = false the (stream, frame) pairs of fab_decode, WIN = true
+// the frames of the windows of P.W).  `ws` = this warp's shared storage.
+template <bool WIN = false>
 FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
     const DecParams& D = P.D;
     const int ln = lane();
     const int nch = D.nch;
     int64_t idx = item0 + ln;
-    int64_t k = idx / P.nwin;
-    bool active = k < D.n_sel;
+    const WorkItem it = resolve_item<WIN>(D, P.W, P.nwin, idx);
+    const int64_t k = it.k;
+    bool active = k >= 0;
     int64_t j = 0;
     int bs_nom = 0, bs = 0;
     const uint8_t* fp = nullptr;
@@ -542,12 +545,12 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
     if (active) {
         const StreamMeta m = D.meta[k];
         bs_nom = m.blocksize;
-        int64_t jj0 = D.first / bs_nom, jj1 = (D.first + D.n_decode - 1) / bs_nom;
-        if (jj1 - jj0 + 1 > P.nwin) {
-            if (idx % P.nwin == 0) atom_or_global(&D.stream_flag[k], 1);
+        int64_t jj0 = it.first / bs_nom, jj1 = (it.first + it.n - 1) / bs_nom;
+        if (jj1 - jj0 + 1 > it.nwin) {
+            if (it.jrel == 0) atom_or_global(&D.stream_flag[k], 1);
             active = false;
         } else {
-            j = jj0 + idx % P.nwin;
+            j = jj0 + it.jrel;
             if (j > jj1) active = false;
         }
     }
@@ -580,8 +583,8 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
         r.out = nullptr; r.lo = 0; r.hi = 0; r.off = 0.f; r.coeff = 0.f;
         if (active) {
             int64_t s0 = j * (int64_t)bs_nom;
-            r.out = D.data + (k * D.n_decode + (s0 - D.first)) * nch;
-            int64_t lo = D.first - s0, hi = D.first + D.n_decode - s0;
+            r.out = D.data + (it.out + (s0 - it.first)) * nch;
+            int64_t lo = it.first - s0, hi = it.first + it.n - s0;
             r.lo = (int)(lo < 0 ? 0 : lo);
             r.hi = (int)(hi > bs ? bs : hi);
             if (P.restore) { r.off = P.offsets[k]; r.coeff = restore_coeff_f32(P.gains[k]); }
@@ -640,17 +643,19 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
 // and works in the trinomial domain of fa_bits.h (shifts and XORs only: no tables, no shared memory).  A
 // mismatch flags the stream for the sequential walker exactly like a mismatch found by the general decoder.
 // ------------------------------------------------------------------------------------------------------
+template <bool WIN = false>
 FA_D void crc_frame_warp(const TileParams& P, int64_t idx) {
     const DecParams& D = P.D;
     const int ln = lane();
-    const int64_t k = idx / P.nwin;
-    if (k >= D.n_sel) return;
+    const WorkItem it = resolve_item<WIN>(D, P.W, P.nwin, idx);
+    const int64_t k = it.k;
+    if (k < 0) return;
     if (D.stream_flag[k] != 0) return;
     const int bs_nom = D.meta[k].blocksize;
     if (bs_nom <= 0) return;
-    const int64_t jj0 = D.first / bs_nom, jj1 = (D.first + D.n_decode - 1) / bs_nom;
-    if (jj1 - jj0 + 1 > P.nwin) return;               // (the tile kernel hands this stream to the walker)
-    const int64_t j = jj0 + idx % P.nwin;
+    const int64_t jj0 = it.first / bs_nom, jj1 = (it.first + it.n - 1) / bs_nom;
+    if (jj1 - jj0 + 1 > it.nwin) return;              // (the tile kernel hands this stream to the walker)
+    const int64_t j = jj0 + it.jrel;
     if (j > jj1) return;
     const long long* fo = D.frame_off + k * (int64_t)(D.nframes_cap + 1);
     const long long off = fo[j], next = fo[j + 1];

@@ -1,9 +1,10 @@
 """array_decompress / array_decompress_slice: same contract as
 /root/reference/src/flacarray/decompress.py:18-205 (keep mask, sample window, single-stream
-flattening rules, error messages).  The FLAC decode and the int->float restore run on the device."""
+flattening rules, error messages); array_decompress_windows: many per-stream sample windows in one decode.
+The FLAC decode and the int->float restore run on the device."""
 import numpy as np
 
-from .libflacarray import decode_flac, decode_flac_float, is_torch
+from .libflacarray import decode_flac, decode_flac_float, decode_windows, is_torch
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -107,3 +108,41 @@ def array_decompress(
         no_flatten=no_flatten,
     )
     return arr
+
+
+@function_timer
+def array_decompress_windows(
+    compressed,
+    stream_size,
+    stream_starts,
+    stream_nbytes,
+    streams,
+    first,
+    last,
+    stream_offsets=None,
+    stream_gains=None,
+    is_int64=False,
+):
+    """Decompress many sample windows, each of its own stream, in one call.
+
+    Window i is samples [first[i], last[i]) of the stream with flat C-order index streams[i] into stream_starts;
+    `first` and `last` may be scalars (broadcast against `streams`).  Windows may be empty, overlap, repeat and come in
+    any order.  Offsets and gains -- both or neither -- restore the floats as array_decompress does.  Only the frames
+    the windows touch are decoded.
+
+    Returns (data, offsets): `data` is 1-D in the restored dtype (a CUDA tensor when `compressed` is one, else numpy)
+    and `offsets` an int64 numpy array of shape (n + 1,); window i is data[offsets[i]:offsets[i + 1]].
+    """
+    if (stream_offsets is None) != (stream_gains is None):
+        which = "gains" if stream_gains is None else "offsets"
+        given = "offsets" if stream_gains is None else "gains"
+        raise RuntimeError(f"When specifying {given}, you must also provide the {which}")
+    if not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts)):
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+        if stream_offsets is not None:
+            fdt = np.float64 if is_int64 else np.float32
+            stream_offsets = ensure_one_element(stream_offsets, fdt)
+            stream_gains = ensure_one_element(stream_gains, fdt)
+    return decode_windows(compressed, stream_starts, stream_nbytes, stream_size, streams, first, last,
+                          offsets=stream_offsets, gains=stream_gains, is_int64=is_int64)

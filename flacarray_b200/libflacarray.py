@@ -919,3 +919,165 @@ def decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, f
     out = decode_device(comp, d_starts, d_nbytes, n_stream, int(stream_size), int(first_sample), int(last_sample),
                         is_int64, max_nb, hint, off, gain)
     return out.reshape(output_shape)
+
+
+# -------------------------------------------------------------------------------------------------
+# Per-stream sample windows (fab_decode_windows; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+
+def _window_records(n_stream, stream_size, streams, first, last):
+    """Host validation of window records (flat stream indices, [first, last) each); returns three int64 arrays."""
+    s = np.asarray(streams.cpu() if is_torch(streams) else streams)
+    f = np.asarray(first.cpu() if is_torch(first) else first)
+    l_ = np.asarray(last.cpu() if is_torch(last) else last)
+    for name, a in (("streams", s), ("first", f), ("last", l_)):
+        if a.size and not np.issubdtype(a.dtype, np.integer):
+            raise RuntimeError(f"window {name} must be integers, not {a.dtype}")
+    s = s.reshape(-1).astype(np.int64)
+    f = f.reshape(-1).astype(np.int64) if f.ndim else np.full(s.size, int(f), np.int64)
+    l_ = l_.reshape(-1).astype(np.int64) if l_.ndim else np.full(s.size, int(l_), np.int64)
+    if not (s.size == f.size == l_.size):
+        raise RuntimeError(f"streams, first and last must have the same length (got {s.size}, {f.size} and {l_.size})")
+    if s.size:
+        if int(s.min()) < 0 or int(s.max()) >= n_stream:
+            bad = int(s[(s < 0) | (s >= n_stream)][0])
+            raise RuntimeError(f"window stream index {bad} is out of range for {n_stream} streams")
+        if int(f.min()) < 0 or int(l_.max()) > stream_size:
+            i = int(np.nonzero((f < 0) | (l_ > stream_size))[0][0])
+            raise RuntimeError(f"window {i} [{int(f[i])}, {int(l_[i])}) lies outside the stream of {stream_size} samples")
+        if bool((f > l_).any()):
+            i = int(np.nonzero(f > l_)[0][0])
+            raise RuntimeError(f"window {i}: first sample {int(f[i])} is larger than last sample {int(l_[i])}")
+    return s, f, l_
+
+
+def decode_windows_device(comp, starts, nbytes, n_stream, stream_size, is_int64, win_stream, win_first, win_last, win_out,
+                          out, max_nbytes, bs_hint, offsets=None, gains=None):
+    """Device-level fab_decode_windows.  Every array is a CUDA tensor; `out` receives the windows at win_out."""
+    dev = comp.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_decode_windows(ctx.handle, _ptr(comp), _ptr(starts), _ptr(nbytes), n_stream, stream_size,
+                                           1 if is_int64 else 0, _ptr(win_stream), _ptr(win_first), _ptr(win_last),
+                                           _ptr(win_out), int(win_stream.numel()), _ptr(out), _ptr(offsets), _ptr(gains),
+                                           int(max_nbytes), int(bs_hint), st)
+        _check(rc, ctx, st, "Decoding")
+    return out
+
+
+def decode_windows(compressed, starts, nbytes, stream_size, streams, first, last, offsets=None, gains=None,
+                   is_int64=False):
+    """Decode window i = samples [first[i], last[i]) of stream streams[i] for every i in one call.
+
+    streams: flat (C-order) indices into starts / nbytes; first / last: arrays or scalars broadcast against streams.
+    Windows may be empty, overlap, repeat and come in any order.  With offsets and gains (one per stream) the samples
+    are restored to float32 / float64.  Returns (data, woff): data is 1-D, window i is data[woff[i]:woff[i + 1]], and woff
+    is a host int64 array of n + 1 entries.  data is a CUDA tensor when `compressed` is one (the decode stays on the
+    device), else a numpy array.  Only the frames the windows touch are decoded, and every referenced stream is indexed
+    once however many windows it has.
+    """
+    if np_dtype(compressed) != compressed_dtype:
+        raise RuntimeError("Compressed data should be of type uint8")
+    if len(compressed.shape) != 1 or not _is_contiguous(compressed):
+        raise RuntimeError("Compressed byte array should be one dimensional and C-contiguous")
+    if stream_size <= 0:
+        raise RuntimeError("You must specify the non-zero output stream size")
+    if (offsets is None) != (gains is None):
+        raise RuntimeError("Offsets and gains must be given together")
+    h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1).astype(np.int64)
+    h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1).astype(np.int64)
+    n_stream = h_starts.size
+    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
+    s, f, l_ = _window_records(n_stream, int(stream_size), streams, first, last)
+    restore = offsets is not None
+    woff = np.zeros(s.size + 1, np.int64)
+    np.cumsum(l_ - f, out=woff[1:])
+    total = int(woff[-1])
+    if is_int64:
+        odt = torch.float64 if restore else torch.int64
+    else:
+        odt = torch.float32 if restore else torch.int32
+    idt = torch.int64 if is_int64 else torch.int32
+    on_dev = is_torch(compressed) and compressed.is_cuda
+    if s.size == 0:
+        if on_dev:
+            return torch.empty(0, dtype=odt, device=compressed.device), woff
+        return np.zeros(0, dtype=_TORCH2NP[odt]), woff
+    # the device only sees the referenced streams, each once
+    uniq, inv = np.unique(s, return_inverse=True)
+    inv = inv.reshape(-1).astype(np.int64)
+    u_starts, u_nbytes = h_starts[uniq], h_nbytes[uniq]
+    fdt = torch.float64 if is_int64 else torch.float32
+    h_off = h_gain = None
+    if restore:
+        h_off = np.asarray(offsets.cpu() if is_torch(offsets) else offsets).reshape(-1)[uniq]
+        h_gain = np.asarray(gains.cpu() if is_torch(gains) else gains).reshape(-1)[uniq]
+    hint = blocksize_hint(compressed, u_starts)
+    if on_dev:
+        dev = compressed.device
+        out = torch.empty(max(total, 1), dtype=idt, device=dev)
+        d_off = to_device(h_off, dev, fdt) if restore else None
+        d_gain = to_device(h_gain, dev, fdt) if restore else None
+        decode_windows_device(compressed, to_device(u_starts, dev, torch.int64), to_device(u_nbytes, dev, torch.int64),
+                              uniq.size, int(stream_size), is_int64, to_device(inv, dev, torch.int64),
+                              to_device(f, dev, torch.int64), to_device(l_, dev, torch.int64),
+                              to_device(woff[:-1], dev, torch.int64), out, int(u_nbytes.max()), hint, d_off, d_gain)
+        return out[:total].view(odt), woff
+    return _decode_windows_host(compressed, u_starts, u_nbytes, int(stream_size), inv, f, l_, woff, is_int64, hint, idt, odt,
+                                h_off, h_gain), woff
+
+
+def _decode_windows_host(compressed, u_starts, u_nbytes, stream_size, inv, f, l_, woff, is_int64, hint, idt, odt, h_off,
+                         h_gain):
+    """Host compressed bytes: the referenced streams' bytes go to the device in staged copies, in groups of streams
+    (_chunk_ranges) when they exceed one chunk; every group decodes its windows into one packed device output."""
+    if is_torch(compressed):
+        compressed = compressed.numpy()
+    dev = _device()
+    total = int(woff[-1])
+    n_u = u_starts.size
+    restore = h_off is not None
+    order = np.argsort(inv, kind="stable")          # windows grouped by stream slot
+    bounds = np.searchsorted(inv[order], np.arange(n_u + 1))
+    ranges = _chunk_ranges(n_u, max(1, int(u_nbytes.sum()) // n_u))
+    src = _as_host_tensor(compressed)
+    with torch.cuda.device(dev):
+        cur = torch.cuda.current_stream(dev)
+        s_in, _ = _side_streams(dev)
+        fdt = torch.float64 if is_int64 else torch.float32
+        out = torch.empty(max(total, 1), dtype=idt, device=dev)
+        d_wout = to_device(woff[:-1], dev, torch.int64)
+
+        def prep(feed, i):
+            a, b = ranges[i]
+            st, nb = u_starts[a:b], u_nbytes[a:b]
+            lo, hi = int(st.min()), int((st + nb).max())
+            if hi - lo == int(nb.sum()):                 # back to back (any order): one contiguous range
+                part, rel = src[lo:hi], st - lo
+            else:                                        # gather the streams' bytes into one buffer first
+                rel = np.zeros(b - a, np.int64)
+                np.cumsum(nb[:-1], out=rel[1:])
+                part = torch.from_numpy(np.concatenate([compressed[int(x):int(x) + int(n)] for x, n in zip(st, nb)]))
+            dc = torch.empty(max(part.numel(), 1), dtype=torch.uint8, device=dev)
+            feed.copy(dc[:part.numel()], part)
+            sel = order[bounds[a]:bounds[b]]
+            dw = [torch.from_numpy(np.ascontiguousarray(x)).to(dev, non_blocking=True)
+                  for x in (rel, nb, inv[sel] - a, f[sel], l_[sel], sel.astype(np.int64))]
+            e = torch.cuda.Event()
+            e.record(s_in)
+            return dc, dw, e, int(nb.max())
+
+        d_off = to_device(h_off, dev, fdt) if restore else None
+        d_gain = to_device(h_gain, dev, fdt) if restore else None
+        for (a, b), (dc, dw, e, max_nb) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
+            cur.wait_event(e)
+            for t in [dc] + dw:
+                t.record_stream(cur)
+            d_st, d_nb, d_ws, d_wf, d_wl, d_sel = dw
+            d_wo = d_wout[d_sel]
+            decode_windows_device(dc, d_st, d_nb, b - a, stream_size, is_int64, d_ws, d_wf, d_wl, d_wo, out, max_nb, hint,
+                                  None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b])
+            del dc, dw, d_st, d_nb, d_ws, d_wf, d_wl, d_sel, d_wo
+        host = to_host(out[:total].view(odt))
+    return host

@@ -157,6 +157,27 @@ int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_star
                void* stream);
 
 /*
+ * Decode many sample windows, each of its own stream and range, in one call (no reference equivalent).
+ * Window w = (d_win_stream[w], d_win_first[w], d_win_last[w], d_win_out[w]) decodes samples [first, last)
+ * of stream slot d_win_stream[w] in [0, n_stream) to d_out[d_win_out[w] ...] (counted in samples of the
+ * output type: packed, a row pitch, ... -- output regions must not overlap).  Windows may be empty
+ * (first == last), overlap, repeat and come in any order.  A record with the slot out of range, first < 0,
+ * last > stream_size or first > last sets ERROR_DECODE_SAMPLE_RANGE in the error mask and is skipped.
+ * Only the frames the windows touch are decoded; metadata, frame tables and the sync scan of foreign
+ * streams run once per stream slot, so give each distinct stream one slot.  Offsets and gains are indexed
+ * by slot and restore like fab_decode.  All window arrays are device memory (int64).  One host round trip
+ * per call sizes the grids.  The workspace (fab_decode_windows_workspace_bytes; total_items, the number of
+ * (window, frame) items, does not enter the present layout) grows with n_stream x frames + n_win.
+ */
+int fab_decode_windows(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                       int64_t n_stream, int64_t stream_size, int is_int64, const int64_t* d_win_stream,
+                       const int64_t* d_win_first, const int64_t* d_win_last, const int64_t* d_win_out, int64_t n_win,
+                       void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes, int blocksize_hint,
+                       void* stream);
+int64_t fab_decode_windows_workspace_bytes(int64_t n_stream, int64_t stream_size, int64_t n_win, int64_t total_items,
+                                           int blocksize_hint);
+
+/*
  * Per-stream population standard deviation of float32 / float64 streams, in the input's type: the device side of
  * `precision` -> quanta (replaces np.std(data, axis=-1) in utils.py:282-296).  One read of the input, moments
  * accumulated in double precision; differs from numpy's pairwise single-precision sum by rounding only.
