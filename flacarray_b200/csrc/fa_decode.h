@@ -190,9 +190,11 @@ FA_D bool decode_subframe_general(BitRd& br, int bs, int bps, const FrameOut& fo
     if (!residual_begin(br, bs, order, rs)) return false;
     for (int i = order; i < bs; ++i) {
         int64_t r = residual_next(br, order, rs);
-        int64_t sum = 0;
-        for (int j = 0; j < order; ++j) sum += (int64_t)coef[j] * hist[(i - 1 - j) & 31];
-        int64_t v = r + (sum >> shift);
+        // (wrapping arithmetic: a valid stream keeps |sum| < 2^53, but a damaged one can feed any history, and signed
+        // overflow is undefined behaviour; such a frame fails its CRC-16 anyway)
+        uint64_t sum = 0;
+        for (int j = 0; j < order; ++j) sum += (uint64_t)(int64_t)coef[j] * (uint64_t)hist[(i - 1 - j) & 31];
+        int64_t v = (int64_t)((uint64_t)r + (uint64_t)((int64_t)sum >> shift));
         hist[i & 31] = v;
         store_sample(fo, ca, c, i, (int64_t)((uint64_t)v << wasted));
         if (br.err) return false;

@@ -21,6 +21,7 @@ import numpy as np
 
 from . import ffmpeg_flac as ff
 from . import oracle as O
+from .flac_writer import crc8, crc16
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 SEED = 123456789  # demo.py:12
@@ -36,24 +37,6 @@ def tod(rng, shape, dtype, sigma=1.0):
     wave = 2 * sigma * np.sin(2 * np.pi * 3 * minf * t) + 6 * sigma * np.sin(2 * np.pi * minf * t)
     scale = rng.random(size=lead)
     return (dc + scale * wave + rng.normal(0.0, sigma, shape)).astype(dtype)
-
-
-def crc8(b):
-    c = 0
-    for x in b:
-        c ^= x
-        for _ in range(8):
-            c = ((c << 1) ^ 0x07) & 0xFF if c & 0x80 else (c << 1) & 0xFF
-    return c
-
-
-def crc16(b):
-    c = 0
-    for x in b:
-        c ^= x << 8
-        for _ in range(8):
-            c = ((c << 1) ^ 0x8005) & 0xFFFF if c & 0x8000 else (c << 1) & 0xFFFF
-    return c
 
 
 def handmade_verbatim(samples):

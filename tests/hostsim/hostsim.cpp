@@ -147,6 +147,15 @@ int hs_decode(const uint8_t* bytes, const long long* starts, const long long* nb
     }
     int nframes_cap = (int)((stream_size + 15) / 16) + 1;  // smallest legal blocksize is 16
     if (nframes_cap > (1 << 22)) nframes_cap = 1 << 22;
+    // mode 2 sizes the frame tables and the item space the way fab_decode does: from the blocksize hint the host
+    // reads from the FIRST stream's STREAMINFO (min blocksize; 4096 without one), clamped to >= 16
+    int bsh = 4096;
+    if (mode == 2) {
+        const uint8_t* s0 = n_sel > 0 ? bytes + starts[0] : nullptr;
+        if (s0 && nbytes[0] >= 12 && memcmp(s0, "fLaC", 4) == 0 && ((s0[8] << 8) | s0[9]) > 0) bsh = (s0[8] << 8) | s0[9];
+        if (bsh < 16) bsh = 16;
+        nframes_cap = (int)((stream_size + bsh - 1) / bsh);
+    }
     std::vector<StreamMeta> meta((size_t)n_sel);
     std::vector<long long> fo((size_t)n_sel * (size_t)(nframes_cap + 1), -1);
     std::vector<int> flag((size_t)n_sel, 0);
@@ -165,8 +174,6 @@ int hs_decode(const uint8_t* bytes, const long long* starts, const long long* nb
         });
         // the product's warp-cooperative scan (three warps striding over each stream's rows)
         fasim::launch((int)n_sel * 3, 32, 0, [&](int b) { sync_scan_warp(P, (int64_t)(b / 3), (int64_t)(b % 3), 3); });
-        int bsh = 4096;
-        for (int64_t k = 0; k < n_sel; ++k) if (meta[(size_t)k].blocksize > 0) { bsh = meta[(size_t)k].blocksize; break; }
         int64_t nwin = (first_decode + n_decode - 1) / bsh - first_decode / bsh + 1;
         TileParams TP;
         TP.D = P; TP.j0 = first_decode / bsh; TP.nwin = nwin; TP.frame_flag = fflag.data();

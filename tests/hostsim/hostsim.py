@@ -13,15 +13,17 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
 
-def lib():
+def lib(prebuilt=None):
+    """The emulator library, built next to this file when stale; `prebuilt`: load that build instead (e.g. one with
+    sanitizers)."""
     global _LIB
     if _LIB is not None:
         return _LIB
-    so = os.path.join(_HERE, "libhostsim.so")
+    so = prebuilt or os.path.join(_HERE, "libhostsim.so")
     srcs = [os.path.join(_HERE, "hostsim.cpp")] + [
         os.path.join(_HERE, "..", "..", "flacarray_b200", "csrc", f)
         for f in ("fa_simt.h", "fa_bits.h", "fa_quant.h", "fa_decode.h", "fa_decode_tile.h", "fa_encode.h", "fa_encode_fixed.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
+    if prebuilt is None and (not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs)):
         cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
         subprocess.run([cxx, "-O2", "-std=c++20", "-ffp-contract=off", "-fPIC", "-shared", "-pthread",
                         srcs[0], "-o", so], check=True, capture_output=True)
