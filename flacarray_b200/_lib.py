@@ -92,6 +92,10 @@ def lib():
         L.fab_encode.argtypes = [_vp, _vp, _i32, _i64, _i64, _u32, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]
         L.fab_decode.restype = _i32
         L.fab_decode.argtypes = [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _i64, _i64, _vp, _vp, _vp, _i64, _i32, _vp]
+        L.fab_decode_isolated.restype = _i32
+        L.fab_decode_isolated.argtypes = [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _i64, _i64, _vp, _vp, _vp, _i64, _i32, _vp, _vp]
+        L.fab_verify.restype = _i32
+        L.fab_verify.argtypes = [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _i64, _i32, _vp, _vp]
         L.fab_decode_windows.restype = _i32
         L.fab_decode_windows.argtypes = [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64,
                                          _i32, _vp]
@@ -118,7 +122,7 @@ EXPORTED = [
     "float32_to_int32", "float64_to_int64", "int64_to_float64", "int32_to_float32",
     "fab_create", "fab_destroy", "fab_last_error", "fab_launch_count", "fab_encode_bound", "fab_encode",
     "fab_encode_workspace_bytes", "fab_decode_workspace_bytes", "fab_set_workspace",
-    "fab_decode", "fab_decode_windows", "fab_decode_windows_workspace_bytes", "fab_stream_std", "fab_float_to_int", "fab_int_to_float", "fab_finish", "fab_profile", "fab_profile_ms",
+    "fab_decode", "fab_decode_isolated", "fab_verify", "fab_decode_windows", "fab_decode_windows_workspace_bytes", "fab_stream_std", "fab_float_to_int", "fab_int_to_float", "fab_finish", "fab_profile", "fab_profile_ms",
 ]
 
 

@@ -15,7 +15,7 @@ import copy
 import numpy as np
 
 from .compress import array_compress
-from .decompress import array_decompress_slice, array_decompress_windows
+from .decompress import array_decompress_slice, array_decompress_windows, array_verify
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -303,8 +303,12 @@ class FlacArray:
                 return False
         return True
 
-    def to_array(self, keep=None, stream_slice=None, keep_indices=False, use_threads=False):
-        """Decompress local data into an array (array.py:518-584)."""
+    def to_array(self, keep=None, stream_slice=None, keep_indices=False, use_threads=False, on_error="raise"):
+        """Decompress local data into an array (array.py:518-584).
+
+        on_error="fill": streams that cannot be decoded do not fail the call; returns (array, status), or (array,
+        indices, status) with `keep` and `keep_indices`, where status (int32, array.shape[:-1]) is 0 or the stream's
+        ERROR_DECODE_* bit and failed rows are 0 / NaN (see array_decompress_slice)."""
         first_samp = None
         last_samp = None
         if stream_slice is not None:
@@ -312,7 +316,7 @@ class FlacArray:
                 raise RuntimeError("Only stream slices with a step size of 1 are supported")
             first_samp = stream_slice.start
             last_samp = stream_slice.stop
-        arr, indices = array_decompress_slice(
+        res = array_decompress_slice(
             self._compressed,
             self._stream_size,
             self._stream_starts,
@@ -325,10 +329,21 @@ class FlacArray:
             is_int64=self._is_int64,
             use_threads=use_threads,
             no_flatten=(not self._flatten_single),
+            on_error=on_error,
         )
+        arr, indices = res[0], res[1]
+        if on_error == "fill":
+            return (arr, indices, res[2]) if (keep is not None and keep_indices) else (arr, res[2])
         if keep is not None and keep_indices:
             return (arr, indices)
         return arr
+
+    def verify(self):
+        """Check every local stream without decoding it out (array_verify).  Returns the int32 status of every stream
+        in the leading shape: 0, or the ERROR_DECODE_* bit of a stream a decode would reject."""
+        status = array_verify(self._compressed, self._stream_size, self._stream_starts, self._stream_nbytes,
+                              is_int64=self._is_int64)
+        return status.reshape(self._leading_shape)
 
     def to_windows(self, streams, first, last):
         """Decompress many sample windows of local streams in one call.

@@ -294,7 +294,7 @@ __global__ void __launch_bounds__(128) k_dec_meta(const DecParams P) {
     long long* fo = P.frame_off + k * (int64_t)(P.nframes_cap + 1);
     int flag = 0;
     if (m.first_frame < 0 || m.channels != P.nch || m.bps != 32) {
-        if (ln == 0) atom_or_global(P.err, kErrDecodeInit);
+        if (ln == 0) stream_failed(P, k, kErrDecodeInit);
         flag = 4;  // undecodable
     } else if (m.blocksize <= 0) {
         flag = 1;  // variable blocksize: sequential walker
@@ -324,7 +324,10 @@ __global__ void __launch_bounds__(128) k_dec_meta(const DecParams P) {
             if (ln == 0) fo[nf] = nb;
         }
     }
-    if (ln == 0) P.stream_flag[k] = flag;
+    if (ln == 0) {
+        P.stream_flag[k] = flag;
+        if (P.status && flag != 4) P.status[k] = 0;
+    }
 }
 
 constexpr int kSyncThreads = 256;
@@ -370,13 +373,13 @@ __global__ void __launch_bounds__(kDecThreads) k_dec_frames(const DecParams P, c
 #ifndef FAB_DEC_CTAS
 #define FAB_DEC_CTAS (20 / FAB_TILE_WARPS)
 #endif
-// (WIN: the item space of fab_decode_windows, `total` items)
-template <bool WIN>
+// (WIN: the item space of fab_decode_windows, `total` items; STORE = false: fab_verify, decode and check only)
+template <bool WIN, bool STORE = true>
 __global__ void __launch_bounds__(kTileWarps * 32, FAB_DEC_CTAS) k_dec_tile(const TileParams P, int64_t total) {
     __shared__ TileShared ws[kTileWarps];
     int64_t item0 = ((int64_t)blockIdx.x * kTileWarps + (threadIdx.x >> 5)) * 32;
     if (item0 >= total) return;
-    tile_warp_body<WIN>(P, item0, &ws[threadIdx.x >> 5]);
+    tile_warp_body<WIN, STORE>(P, item0, &ws[threadIdx.x >> 5]);
 }
 
 // frame CRC-16 of every (stream, frame) item: one warp per item, see crc_frame_warp
@@ -428,6 +431,23 @@ __global__ void __launch_bounds__(256) k_restore_fixup(const TileParams P) {
 __global__ void k_dec_walker(const DecParams P) {
     int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k < P.n_sel) walker_body(P, k);
+}
+
+// fab_decode_isolated / fab_verify: failures go to P.status, P.data null = discard mode
+__global__ void k_dec_walker_iso(const DecParams P) {
+    int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < P.n_sel) walker_body<true>(P, k);
+}
+
+// fab_decode_isolated: overwrite the whole output row of every stream whose status is not 0 with `fill` (0 for integer
+// output, a quiet NaN for float output), after the walker and the restore.  grid = (x, streams of one slab); W is the
+// output element (uint32_t for int32 / float32, unsigned long long for int64 / float64).
+template <typename W>
+__global__ void __launch_bounds__(256) k_dec_fill_failed(const int* __restrict__ status, W* out, int64_t n_per_stream, W fill) {
+    const int64_t s = blockIdx.y;
+    if (status[s] == 0) return;
+    W* o = out + s * n_per_stream;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n_per_stream; i += (int64_t)gridDim.x * 256) o[i] = fill;
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
@@ -1063,13 +1083,14 @@ static void dec_index_streams(fab_ctx* ctx, const DecParams& P, int64_t max_nbyt
 }
 
 // Stage 3 over `total` work items (resolve_item): warp-tile decoder, its CRC pass next to it on the second stream, then
-// the general per-thread decoder on the frames the tile path flagged.  TP.frame_flag must be cleared.
-template <bool WIN>
+// the general per-thread decoder on the frames the tile path flagged.  TP.frame_flag must be cleared.  STORE = false
+// (fab_verify, TP.D.data null): the same stages, no samples written.
+template <bool WIN, bool STORE = true>
 static int dec_items(fab_ctx* ctx, const TileParams& TP, int64_t total, cudaStream_t st) {
     int64_t per_cta = (int64_t)kTileWarps * 32;
     prof_begin(ctx, 1, st);
     FAB_CUDA(ctx, cudaEventRecord(ctx->ev_fork, st));
-    k_dec_tile<WIN><<<(unsigned)((total + per_cta - 1) / per_cta), kTileWarps * 32, 0, st>>>(TP, total);
+    k_dec_tile<WIN, STORE><<<(unsigned)((total + per_cta - 1) / per_cta), kTileWarps * 32, 0, st>>>(TP, total);
     // the CRC pass only needs the frame table: it runs on the second stream, queued behind the tile
     // kernel's launch so that its CTAs fill the SMs the decoder's last partial wave leaves idle
     FAB_CUDA(ctx, cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
@@ -1086,10 +1107,15 @@ static int dec_items(fab_ctx* ctx, const TileParams& TP, int64_t total, cudaStre
     return 0;
 }
 
-extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
-                          int64_t n_stream, int64_t stream_size, int is_int64, int64_t first_sample, int64_t last_sample,
-                          void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes,
-                          int blocksize_hint, void* stream) {
+// fab_decode, fab_decode_isolated and fab_verify.  d_status null (fab_decode): a stream-fatal error goes to the call's
+// error mask.
+// d_status set: every stream reports its own (k_dec_meta, walker), and the rows of failed streams are filled once the
+// walker and the restore are done.  store = false (fab_verify): d_out, d_offsets and d_gains are null and the tile
+// decoder runs its no-store instantiation.
+static int dec_uniform(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                       int64_t n_stream, int64_t stream_size, int is_int64, int64_t first_sample, int64_t last_sample,
+                       void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes, int blocksize_hint,
+                       int32_t* d_status, bool store, void* stream) {
     if (!ctx) return FAB_ERROR_CUDA;
     if (n_stream <= 0) return ERROR_ZERO_NSTREAM;
     if (stream_size <= 0) return ERROR_ZERO_STREAMSIZE;
@@ -1131,6 +1157,7 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
     P.first = first_decode; P.n_decode = n_decode; P.data = (int32_t*)d_out; P.crc = ctx->d_crc;
     P.meta = (StreamMeta*)scr; P.frame_off = (long long*)(scr + meta_b); P.nframes_cap = nframes_cap;
     P.stream_flag = (int*)(scr + meta_b + fo_b); P.err = ctx->d_err; P.verify_crc16 = 1; P.frame_flag = frame_flag;
+    P.status = d_status;
 
     dec_index_streams(ctx, P, max_nbytes, st);
     const bool fuse_restore = d_offsets && d_gains && !is_int64;
@@ -1144,10 +1171,11 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
         TP.D = P; TP.j0 = first_decode / bsh; TP.nwin = nwin; TP.frame_flag = frame_flag;
         TP.restore = fuse_restore ? 1 : 0; TP.offsets = (const float*)d_offsets; TP.gains = (const float*)d_gains;
         TP.W = WinParams{};
-        int rc2 = dec_items<false>(ctx, TP, total, st);
+        int rc2 = store ? dec_items<false>(ctx, TP, total, st) : dec_items<false, false>(ctx, TP, total, st);
         if (rc2) return rc2;
     }
-    k_dec_walker<<<(unsigned)((n_stream + 31) / 32), 32, 0, st>>>(P);
+    if (d_status) k_dec_walker_iso<<<(unsigned)((n_stream + 31) / 32), 32, 0, st>>>(P);
+    else k_dec_walker<<<(unsigned)((n_stream + 31) / 32), 32, 0, st>>>(P);
     ctx->launches++;
 
     if (fuse_restore) {
@@ -1174,8 +1202,53 @@ extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int6
             ctx->launches++;
         }
     }
+    if (d_status && store) {
+        // a few CTAs per stream: those of good streams leave at once, the rare failed row is strided over
+        const bool flt = d_offsets && d_gains;
+        const int64_t gx = std::min<int64_t>((n_decode + 2047) / 2048, 16);
+        for (int64_t s0 = 0; s0 < n_stream; s0 += 65535) {
+            int64_t ns = std::min<int64_t>(65535, n_stream - s0);
+            dim3 grid((unsigned)gx, (unsigned)ns);
+            if (is_int64)
+                k_dec_fill_failed<unsigned long long><<<grid, 256, 0, st>>>(
+                    d_status + s0, (unsigned long long*)d_out + s0 * n_decode, n_decode, flt ? 0x7FF8000000000000ull : 0ull);
+            else
+                k_dec_fill_failed<uint32_t><<<grid, 256, 0, st>>>(d_status + s0, (uint32_t*)d_out + s0 * n_decode, n_decode,
+                                                                  flt ? 0x7FC00000u : 0u);
+            ctx->launches++;
+        }
+    }
     FAB_CUDA(ctx, cudaGetLastError());
     return 0;
+}
+
+extern "C" int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                          int64_t n_stream, int64_t stream_size, int is_int64, int64_t first_sample, int64_t last_sample,
+                          void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes,
+                          int blocksize_hint, void* stream) {
+    return dec_uniform(ctx, d_bytes, d_starts, d_nbytes, n_stream, stream_size, is_int64, first_sample, last_sample, d_out,
+                       d_offsets, d_gains, max_nbytes, blocksize_hint, nullptr, true, stream);
+}
+
+extern "C" int fab_decode_isolated(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts,
+                                   const int64_t* d_nbytes, int64_t n_stream, int64_t stream_size, int is_int64,
+                                   int64_t first_sample, int64_t last_sample, void* d_out, const void* d_offsets,
+                                   const void* d_gains, int64_t max_nbytes, int blocksize_hint, int32_t* d_status,
+                                   void* stream) {
+    return dec_uniform(ctx, d_bytes, d_starts, d_nbytes, n_stream, stream_size, is_int64, first_sample, last_sample, d_out,
+                       d_offsets, d_gains, max_nbytes, blocksize_hint, d_status, true, stream);
+}
+
+extern "C" int fab_verify(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                          int64_t n_stream, int64_t stream_size, int is_int64, int64_t max_nbytes, int blocksize_hint,
+                          int32_t* d_status, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    if (!d_status) {            // (the walker's discard mode reports through the status array only)
+        ctx->last_error = "fab_verify: d_status must not be NULL";
+        return ERROR_ALLOC;
+    }
+    return dec_uniform(ctx, d_bytes, d_starts, d_nbytes, n_stream, stream_size, is_int64, -1, -1, nullptr, nullptr, nullptr,
+                       max_nbytes, blocksize_hint, d_status, false, stream);
 }
 
 // Workspace of one fab_decode_windows call: fab_decode's layout for the stream slots | item0 of the windows.  The item

@@ -210,7 +210,9 @@ FA_D uint32_t crc16_bytes(const CrcTables* t, const uint8_t* p, int64_t n) {
 }
 
 // Decode the frame at `p` (window end `end`).  Returns the frame length in bytes, or -1.
-// expect_nch / expect_bps: what the stream must carry (flacarray: 1|2 channels, 32 bps).
+// expect_nch / expect_bps: what the stream must carry (flacarray: 1|2 channels, 32 bps).  Samples [lo, hi) of the frame are
+// stored from out_base on; an empty range (discard mode: out_base may be null) decodes and checks the whole frame all the
+// same.
 FA_D int64_t decode_frame_general(const uint8_t* p, const uint8_t* end, const CrcTables* t, int si_bps, int expect_nch,
                                   FrameHdr& fh, int32_t* out_base, int lo, int hi, bool check_crc16) {
     if (!parse_frame_header(p, end - p, t, fh)) return -1;
@@ -261,7 +263,16 @@ struct DecParams {
     int* err;
     int verify_crc16;
     const unsigned char* frame_flag;  // optional [n_sel][nframes_cap]: when set, frame_body only decodes flagged frames
+    // optional [n_sel] (fab_decode_isolated, fab_verify): when set, a stream that cannot be decoded reports its
+    // ERROR_DECODE_INIT / ERROR_DECODE_PROCESS bit here instead of in *err; meta writes every entry, the walker its failures
+    int* status = nullptr;
 };
+
+// a stream-fatal error of stream k: its own status entry, or the call's error mask
+FA_D void stream_failed(const DecParams& P, int64_t k, int bit) {
+    if (P.status) P.status[k] = bit;
+    else atom_or_global(P.err, bit);
+}
 
 // number of frames / size of frame j for a fixed-blocksize stream
 FA_D int64_t frames_in_stream(int64_t stream_size, int bs) { return (stream_size + bs - 1) / bs; }
@@ -337,8 +348,9 @@ FA_D void meta_body(const DecParams& P, int64_t k) {
     P.meta[k] = m;
     long long* fo = P.frame_off + k * (int64_t)(P.nframes_cap + 1);
     int flag = 0;
+    if (P.status) P.status[k] = 0;
     if (m.first_frame < 0 || m.channels != P.nch || m.bps != 32) {
-        atom_or_global(P.err, kErrDecodeInit);
+        stream_failed(P, k, kErrDecodeInit);
         flag = 4;  // undecodable
     } else if (m.blocksize <= 0) {
         flag = 1;  // variable blocksize: sequential walker
@@ -444,8 +456,9 @@ FA_D void frame_body(const DecParams& P, int64_t k, int64_t j, int64_t first, in
     const uint8_t* buf = P.bytes + P.starts[k];
     const uint8_t* end = buf + P.nbytes[k];
     int64_t s0 = j * (int64_t)m.blocksize;  // first sample of the frame
-    int32_t* base = P.data + (out + (s0 - first)) * P.nch;
+    int32_t* base = P.data + (P.data ? (out + (s0 - first)) * P.nch : 0);
     int64_t lo = first - s0, hi = first + n - s0;
+    if (!P.data) hi = lo;                   // discard mode (fab_verify): decode and check, store nothing
     FrameHdr fh;
     int64_t len = decode_frame_general(buf + off, end, P.crc, m.bps, P.nch, fh, base,
                                        (int)(lo < 0 ? 0 : lo), (int)(hi > m.blocksize ? m.blocksize : hi),
@@ -456,9 +469,19 @@ FA_D void frame_body(const DecParams& P, int64_t k, int64_t j, int64_t first, in
 }
 FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) { frame_body(P, k, j, P.first, P.n_decode, k * P.n_decode); }
 
+// (a template: the stores of fab_decode's walker stay what they were; register allocation there is sensitive to them)
+template <bool ISO>
+FA_D void walker_failed(const DecParams& P, int64_t k) {
+    if constexpr (ISO) P.status[k] = kErrDecodeProcess;
+    else atom_or_global(P.err, kErrDecodeProcess);
+}
+
 // ---- stage 4: sequential walker for streams the parallel path could not index -----------------------
 // (variable blocksize, ambiguous sync candidates, failed chain check).  Always verifies CRC-16.
-// Decodes the window [first, first + n) of stream k to output element `out` on.
+// Decodes the window [first, first + n) of stream k to output element `out` on.  ISO (fab_decode_isolated, fab_verify;
+// P.status set): a failure goes to the stream's status entry instead of the call's error mask, and P.data may be null
+// (discard mode: decode and check, store nothing).  ISO = false is fab_decode's and fab_decode_windows' walker.
+template <bool ISO = false>
 FA_D void walker_body(const DecParams& P, int64_t k, int64_t first, int64_t n, int64_t out) {
     int flag = P.stream_flag[k];
     if (flag == 0 || flag == 4) return;
@@ -468,15 +491,17 @@ FA_D void walker_body(const DecParams& P, int64_t k, int64_t first, int64_t n, i
     int64_t pos = m.first_frame, sample = 0, last = first + n;
     uint64_t expect = 0;
     while (sample < last) {
-        if (pos >= P.nbytes[k]) { atom_or_global(P.err, kErrDecodeProcess); return; }
+        if (pos >= P.nbytes[k]) { walker_failed<ISO>(P, k); return; }
         FrameHdr fh;
-        int32_t* base = P.data + (out + (sample - first)) * P.nch;
+        int32_t* base = nullptr;
         int64_t lo = first - sample, hi = last - sample;
+        if (!ISO || P.data) base = P.data + (out + (sample - first)) * P.nch;
+        else hi = lo;                       // discard mode
         int64_t len = decode_frame_general(buf + pos, end, P.crc, m.bps, P.nch, fh, base, (int)(lo < 0 ? 0 : lo),
                                            (int)(hi > 65536 ? 65536 : hi), true);
-        if (len < 0) { atom_or_global(P.err, kErrDecodeProcess); return; }
+        if (len < 0) { walker_failed<ISO>(P, k); return; }
         if (fh.variable ? ((int64_t)fh.number != sample) : (fh.number != expect)) {
-            atom_or_global(P.err, kErrDecodeProcess);
+            walker_failed<ISO>(P, k);
             return;
         }
         expect++;
@@ -484,6 +509,7 @@ FA_D void walker_body(const DecParams& P, int64_t k, int64_t first, int64_t n, i
         pos += len;
     }
 }
-FA_D void walker_body(const DecParams& P, int64_t k) { walker_body(P, k, P.first, P.n_decode, k * P.n_decode); }
+template <bool ISO = false>
+FA_D void walker_body(const DecParams& P, int64_t k) { walker_body<ISO>(P, k, P.first, P.n_decode, k * P.n_decode); }
 
 }  // namespace fa

@@ -430,7 +430,8 @@ struct TileParams {
 };
 
 // Decode + flush all tiles of one channel pass with a compile-time upper bound on the predictor order.
-template <int ORD>
+// STORE = false (fab_verify): the same decode and checks, without the flush of the tiles to D.data.
+template <int ORD, bool STORE = true>
 FA_D void tile_channel_pass(const TileParams& P, TileShared* ws, BitRdC& br, TileLane& L, bool& run,
                             bool& fail, bool& punt, int bs, uint32_t bsmax, int c, int nch) {
     const int ln = lane();
@@ -468,6 +469,7 @@ FA_D void tile_channel_pass(const TileParams& P, TileShared* ws, BitRdC& br, Til
                 }
             }
         }
+        if constexpr (!STORE) continue;
         syncwarp();
         // transpose.  Common case (one channel, every active row holds all 32 samples of this block inside
         // its window, 16-byte aligned destination): 8 trips, each lane moves 4 consecutive samples of one
@@ -524,8 +526,9 @@ FA_D void tile_channel_pass(const TileParams& P, TileShared* ws, BitRdC& br, Til
 }
 
 // One warp: 32 consecutive work items (resolve_item: WIN = false the (stream, frame) pairs of fab_decode, WIN = true
-// the frames of the windows of P.W).  `ws` = this warp's shared storage.
-template <bool WIN = false>
+// the frames of the windows of P.W).  `ws` = this warp's shared storage.  STORE = false: decode and check every item,
+// write no samples (the row descriptions, which only the flush reads, are not published).
+template <bool WIN = false, bool STORE = true>
 FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
     const DecParams& D = P.D;
     const int ln = lane();
@@ -578,7 +581,7 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
         }
     }
     // publish the row description
-    {
+    if constexpr (STORE) {
         TileRow r;
         r.out = nullptr; r.lo = 0; r.hi = 0; r.off = 0.f; r.coeff = 0.f;
         if (active) {
@@ -590,8 +593,8 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
             if (P.restore) { r.off = P.offsets[k]; r.coeff = restore_coeff_f32(P.gains[k]); }
         }
         ws->row[ln] = r;
+        syncwarp();
     }
-    syncwarp();
     uint32_t bsmax = (uint32_t)(active ? bs : 0);
     for (int m = 16; m >= 1; m >>= 1) { uint32_t o = shfl_xor(bsmax, m); bsmax = o > bsmax ? o : bsmax; }
 
@@ -616,9 +619,9 @@ FA_D void tile_warp_body(const TileParams& P, int64_t item0, TileShared* ws) {
         // warp-uniform bound on the predictor order picks the instantiation of the sample loop
         uint32_t omax = (uint32_t)((run && L.mode == 2) ? L.order : 0);
         for (int m = 16; m >= 1; m >>= 1) { uint32_t o = shfl_xor(omax, m); omax = o > omax ? o : omax; }
-        if (omax <= 4) tile_channel_pass<4>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
-        else if (omax <= 8) tile_channel_pass<8>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
-        else tile_channel_pass<kTileOrd>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
+        if (omax <= 4) tile_channel_pass<4, STORE>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
+        else if (omax <= 8) tile_channel_pass<8, STORE>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
+        else tile_channel_pass<kTileOrd, STORE>(P, ws, br, L, run, fail, punt, bs, bsmax, c, nch);
         if (run && br.err) fail = true;
     }
     if (active) {

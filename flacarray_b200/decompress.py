@@ -1,10 +1,11 @@
 """array_decompress / array_decompress_slice: same contract as
 /root/reference/src/flacarray/decompress.py:18-205 (keep mask, sample window, single-stream
-flattening rules, error messages); array_decompress_windows: many per-stream sample windows in one decode.
-The FLAC decode and the int->float restore run on the device."""
+flattening rules, error messages), plus on_error="fill" (per-stream fault isolation);
+array_decompress_windows: many per-stream sample windows in one decode; array_verify: check streams without
+decoding them out.  The FLAC decode and the int->float restore run on the device."""
 import numpy as np
 
-from .libflacarray import decode_flac, decode_flac_float, decode_windows, is_torch
+from .libflacarray import check_on_error, decode_flac, decode_flac_float, decode_windows, is_torch, verify_flac
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -32,6 +33,7 @@ def array_decompress_slice(
     is_int64=False,
     use_threads=False,
     no_flatten=False,
+    on_error="raise",
 ):
     """Decompress a window of selected streams and restore the original data type.
 
@@ -40,7 +42,13 @@ def array_decompress_slice(
     or neither -- turn the integers back into floats.  A single stream may be described by scalars or 1-element
     arrays and then comes back flattened unless `no_flatten`.  Returns (array, indices): `indices` lists the index
     tuples of the kept streams in storage order, or is None without `keep`.
+
+    on_error: "raise" (default) fails the whole call when any stream cannot be decoded.  "fill" decodes every stream it
+    can and returns (array, indices, status): status is an int32 numpy array of array.shape[:-1] ((1,) for a flattened
+    single stream), in the same row order, holding 0 or the stream's ERROR_DECODE_INIT (1 << 13) / ERROR_DECODE_PROCESS
+    (1 << 14) bit; the rows of failed streams are 0 (integers) or NaN (floats).  Call-level errors still raise.
     """
+    isolate = check_on_error(on_error)
     if (stream_offsets is None) != (stream_gains is None):
         which = "gains" if stream_gains is None else "offsets"
         given = "offsets" if stream_gains is None else "gains"
@@ -67,14 +75,21 @@ def array_decompress_slice(
         # an all-False mask: the reference hands back an empty (0, n) array
         n = last - first if (first >= 0 and last >= 0) else stream_size
         arr = np.zeros(tuple(starts.shape) + (n,), dtype=_result_dtype(is_int64, restored))
+        if isolate:
+            arr = (arr, np.zeros(tuple(starts.shape), np.int32))
     elif restored:
         arr = decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, first_sample=first,
-                                last_sample=last, is_int64=is_int64)
+                                last_sample=last, is_int64=is_int64, on_error=on_error)
     else:
         arr = decode_flac(compressed, starts, nbytes, stream_size, first_sample=first, last_sample=last,
-                          use_threads=use_threads, is_int64=is_int64)
+                          use_threads=use_threads, is_int64=is_int64, on_error=on_error)
+    status = None
+    if isolate:
+        arr, status = arr
     if single and not no_flatten:
         arr = arr.reshape((-1,))
+    if isolate:
+        return arr, indices, status
     return arr, indices
 
 
@@ -91,9 +106,12 @@ def array_decompress(
     is_int64=False,
     use_threads=False,
     no_flatten=False,
+    on_error="raise",
 ):
-    """Decompress a FLAC encoded array and restore the original data type."""
-    arr, _ = array_decompress_slice(
+    """Decompress a FLAC encoded array and restore the original data type.
+
+    on_error="fill" returns (array, status) instead of failing on a damaged stream (see array_decompress_slice)."""
+    res = array_decompress_slice(
         compressed,
         stream_size,
         stream_starts,
@@ -106,8 +124,11 @@ def array_decompress(
         is_int64=is_int64,
         use_threads=use_threads,
         no_flatten=no_flatten,
+        on_error=on_error,
     )
-    return arr
+    if check_on_error(on_error):
+        return res[0], res[2]
+    return res[0]
 
 
 @function_timer
@@ -146,3 +167,18 @@ def array_decompress_windows(
             stream_gains = ensure_one_element(stream_gains, fdt)
     return decode_windows(compressed, stream_starts, stream_nbytes, stream_size, streams, first, last,
                           offsets=stream_offsets, gains=stream_gains, is_int64=is_int64)
+
+
+@function_timer
+def array_verify(compressed, stream_size, stream_starts, stream_nbytes, is_int64=False):
+    """Check every stream without decoding it out: every frame is decoded and checked (CRC-8 / CRC-16, syntax, frame
+    chain, sample count) exactly as a full decode would, and no samples are stored or copied back.
+
+    Returns an int32 numpy array shaped like stream_starts ((1,) for a single stream given as scalars): 0 for a stream a
+    full decode accepts, else its ERROR_DECODE_INIT (1 << 13) / ERROR_DECODE_PROCESS (1 << 14) bit.  Host-resident bytes
+    are copied to the device in groups of streams.
+    """
+    if not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts)):
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+    return verify_flac(compressed, stream_starts, stream_nbytes, stream_size, is_int64=is_int64)

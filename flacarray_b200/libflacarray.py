@@ -606,8 +606,9 @@ def _encode_host(flat, n_stream, stream_size, level, quanta, dt, precision=None)
 
 
 def _decode_host(compressed, h_starts, h_nbytes, n_stream, stream_size, first_sample, last_sample, is_int64,
-                 offsets=None, gains=None):
-    """Host compressed bytes -> host samples (numpy, flat); optional int->float restore on the device."""
+                 offsets=None, gains=None, status=None):
+    """Host compressed bytes -> host samples (numpy, flat); optional int->float restore on the device.  status: int32
+    CUDA tensor [n_stream] for per-stream fault isolation (every chunk of streams fills its slice)."""
     dev = _device()
     n_decode = stream_size
     if first_sample >= 0 and last_sample >= 0:
@@ -650,7 +651,8 @@ def _decode_host(compressed, h_starts, h_nbytes, n_stream, stream_size, first_sa
             for t in (dc, d_st, d_nb):
                 t.record_stream(cur)
             out = decode_device(dc, d_st, d_nb, b - a, int(stream_size), int(first_sample), int(last_sample), is_int64,
-                                max_nb, hint, None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b])
+                                max_nb, hint, None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b],
+                                None if status is None else status[a:b])
             del dc, d_st, d_nb
             e2 = torch.cuda.Event()
             e2.record(cur)
@@ -741,10 +743,12 @@ def blocksize_hint(compressed, starts):
 
 
 def decode_device(comp, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64, max_nbytes,
-                  bs_hint, offsets=None, gains=None):
+                  bs_hint, offsets=None, gains=None, status=None):
     """Device-level decode.  All arrays are CUDA tensors; returns a flat CUDA tensor.
 
-    With offsets/gains the int->float restore (utils.c:330-368) is applied on the device.
+    With offsets/gains the int->float restore (utils.c:330-368) is applied on the device.  With `status` (int32 CUDA
+    tensor [n_stream]) the decode isolates failures per stream (fab_decode_isolated): each stream's error bits go to
+    its status entry, failed rows are filled with 0 / NaN, and only call-level errors raise.
     """
     dev = comp.device
     n_decode = stream_size
@@ -754,9 +758,14 @@ def decode_device(comp, starts, nbytes, n_stream, stream_size, first_sample, las
         ctx = _lib.context(dev)
         out = torch.empty(n_stream * max(n_decode, 0), dtype=torch.int64 if is_int64 else torch.int32, device=dev)
         st = _stream(dev)
-        rc = _lib.lib().fab_decode(ctx.handle, _ptr(comp), _ptr(starts), _ptr(nbytes), n_stream, stream_size,
-                                   1 if is_int64 else 0, first_sample, last_sample, _ptr(out), _ptr(offsets),
-                                   _ptr(gains), int(max_nbytes), int(bs_hint), st)
+        if status is None:
+            rc = _lib.lib().fab_decode(ctx.handle, _ptr(comp), _ptr(starts), _ptr(nbytes), n_stream, stream_size,
+                                       1 if is_int64 else 0, first_sample, last_sample, _ptr(out), _ptr(offsets),
+                                       _ptr(gains), int(max_nbytes), int(bs_hint), st)
+        else:
+            rc = _lib.lib().fab_decode_isolated(ctx.handle, _ptr(comp), _ptr(starts), _ptr(nbytes), n_stream, stream_size,
+                                                1 if is_int64 else 0, first_sample, last_sample, _ptr(out), _ptr(offsets),
+                                                _ptr(gains), int(max_nbytes), int(bs_hint), _ptr(status), st)
         _check(rc, ctx, st, "Decoding")
     if offsets is not None and gains is not None:
         out = out.view(torch.float64 if is_int64 else torch.float32)
@@ -785,7 +794,7 @@ def _check_byte_windows(h_starts, h_nbytes, n_compressed):
         raise RuntimeError("stream starts / nbytes point outside the compressed buffer")
 
 
-def _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64):
+def _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64, status=None):
     on_dev = is_torch(compressed) and compressed.is_cuda
     h_starts = starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)
     h_nbytes = nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)
@@ -794,13 +803,13 @@ def _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample
         if is_torch(compressed):
             compressed = compressed.numpy()
         return _decode_host(compressed, h_starts, h_nbytes, int(n_stream), int(stream_size), int(first_sample),
-                            int(last_sample), is_int64)
+                            int(last_sample), is_int64, status=status)
     max_nb = int(h_nbytes.max()) if h_nbytes.size else 0
     hint = blocksize_hint(compressed, h_starts)
     d_starts = to_device(h_starts, compressed.device, torch.int64)
     d_nbytes = to_device(h_nbytes, compressed.device, torch.int64)
     return decode_device(compressed, d_starts, d_nbytes, int(n_stream), int(stream_size), int(first_sample),
-                         int(last_sample), is_int64, max_nb, hint)
+                         int(last_sample), is_int64, max_nb, hint, status=status)
 
 
 def wrap_decode_i32(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, use_threads):
@@ -813,9 +822,28 @@ def wrap_decode_i64(compressed, starts, nbytes, n_stream, stream_size, first_sam
     return _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, True)
 
 
+def check_on_error(on_error):
+    """True for on_error="fill" (per-stream fault isolation), False for "raise"; anything else is a ValueError."""
+    if isinstance(on_error, str) and on_error in ("raise", "fill"):
+        return on_error == "fill"
+    raise ValueError(f"on_error must be 'raise' or 'fill', not {on_error!r}")
+
+
+def _status_tensor(compressed, n_stream):
+    """Device int32 [n_stream] for the per-stream status of an isolated decode or a verify."""
+    dev = compressed.device if (is_torch(compressed) and compressed.is_cuda) else _device()
+    return torch.empty(max(n_stream, 1), dtype=torch.int32, device=dev)[:n_stream]
+
+
 def decode_flac(compressed, starts, nbytes, stream_size, first_sample=-1, last_sample=-1, use_threads=False,
-                is_int64=False):
-    """Decompress a FLAC compressed bytestream (pyx:713-823)."""
+                is_int64=False, on_error="raise"):
+    """Decompress a FLAC compressed bytestream (pyx:713-823).
+
+    on_error="fill": a stream that cannot be decoded does not fail the call; returns (array, status) where status
+    (int32 numpy, shaped like starts) holds 0 or the stream's ERROR_DECODE_INIT / ERROR_DECODE_PROCESS bit and the rows
+    of failed streams are 0.
+    """
+    isolate = check_on_error(on_error)
     if np_dtype(compressed) != compressed_dtype:
         raise RuntimeError("Compressed data should be of type uint8")
     if not _is_contiguous(compressed):
@@ -842,6 +870,11 @@ def decode_flac(compressed, starts, nbytes, stream_size, first_sample=-1, last_s
     n_stream = int(np.prod(starts.shape))
     flat_starts = starts.reshape((-1,))
     flat_nbytes = nbytes.reshape((-1,))
+    if isolate:
+        status = _status_tensor(compressed, n_stream)
+        flat_output = _wrap_decode(compressed, flat_starts, flat_nbytes, n_stream, stream_size, first_sample, last_sample,
+                                   is_int64, status=status)
+        return flat_output.reshape(output_shape), to_host(status).reshape(tuple(starts.shape))
     if is_int64:
         flat_output = wrap_decode_i64(compressed, flat_starts, flat_nbytes, n_stream, stream_size, first_sample,
                                       last_sample, use_threads)
@@ -890,8 +923,10 @@ def encode_flac_float(data, level, quanta, precision=None):
 
 
 def decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, first_sample=-1, last_sample=-1,
-                      is_int64=False):
-    """decode_flac followed by utils.int_to_float (utils.c:330-368) without leaving the device."""
+                      is_int64=False, on_error="raise"):
+    """decode_flac followed by utils.int_to_float (utils.c:330-368) without leaving the device.  on_error="fill" as in
+    decode_flac, with the rows of failed streams set to NaN."""
+    isolate = check_on_error(on_error)
     n_decode = stream_size
     _check_sample_range(stream_size, first_sample, last_sample)
     if first_sample >= 0 and last_sample >= 0:
@@ -902,12 +937,18 @@ def decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, f
     h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1)
     h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1)
     _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
+    status = _status_tensor(compressed, n_stream) if isolate else None
+
+    def result(out):
+        out = out.reshape(output_shape)
+        return (out, to_host(status).reshape(tuple(starts.shape))) if isolate else out
+
     if not on_dev:
         if is_torch(compressed):
             compressed = compressed.numpy()
         out = _decode_host(compressed, h_starts, h_nbytes, n_stream, int(stream_size), int(first_sample), int(last_sample),
-                           is_int64, offsets, gains)
-        return out.reshape(output_shape)
+                           is_int64, offsets, gains, status=status)
+        return result(out)
     max_nb = int(h_nbytes.max()) if h_nbytes.size else 0
     hint = blocksize_hint(compressed, h_starts)
     comp = compressed
@@ -917,8 +958,78 @@ def decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, f
     off = to_device(offsets.reshape((-1,)), comp.device, fdt)
     gain = to_device(gains.reshape((-1,)), comp.device, fdt)
     out = decode_device(comp, d_starts, d_nbytes, n_stream, int(stream_size), int(first_sample), int(last_sample),
-                        is_int64, max_nb, hint, off, gain)
-    return out.reshape(output_shape)
+                        is_int64, max_nb, hint, off, gain, status=status)
+    return result(out)
+
+
+# -------------------------------------------------------------------------------------------------
+# Verify: decode and check every frame, store no samples (fab_verify; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+
+def verify_device(comp, starts, nbytes, n_stream, stream_size, is_int64, max_nbytes, bs_hint, status):
+    """Device-level fab_verify: CUDA tensors in, `status` (int32 CUDA tensor [n_stream]) filled."""
+    dev = comp.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_verify(ctx.handle, _ptr(comp), _ptr(starts), _ptr(nbytes), n_stream, stream_size,
+                                   1 if is_int64 else 0, int(max_nbytes), int(bs_hint), _ptr(status), st)
+        _check(rc, ctx, st, "Verifying")
+    return status
+
+
+def verify_flac(compressed, starts, nbytes, stream_size, is_int64=False):
+    """Decode and check every frame of every stream without storing samples.  Returns an int32 numpy array shaped like
+    `starts`: 0, or the ERROR_DECODE_INIT / ERROR_DECODE_PROCESS bit of a stream that decoding would reject.  Host bytes
+    go to the device in groups of streams; no samples come back."""
+    if np_dtype(compressed) != compressed_dtype:
+        raise RuntimeError("Compressed data should be of type uint8")
+    if len(compressed.shape) != 1 or not _is_contiguous(compressed):
+        raise RuntimeError("Compressed byte array should be one dimensional and C-contiguous")
+    if stream_size <= 0:
+        raise RuntimeError("You must specify the non-zero output stream size")
+    shape = tuple(starts.shape)
+    h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1).astype(np.int64)
+    h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1).astype(np.int64)
+    n_stream = h_starts.size
+    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
+    if n_stream == 0:
+        return np.zeros(shape, np.int32)
+    status = _status_tensor(compressed, n_stream)
+    hint = blocksize_hint(compressed, h_starts)
+    if is_torch(compressed) and compressed.is_cuda:
+        dev = compressed.device
+        verify_device(compressed, to_device(h_starts, dev, torch.int64), to_device(h_nbytes, dev, torch.int64), n_stream,
+                      int(stream_size), is_int64, int(h_nbytes.max()), hint, status)
+        return to_host(status).reshape(shape)
+    if is_torch(compressed):
+        compressed = compressed.numpy()
+    dev = status.device
+    src = _as_host_tensor(compressed)
+    ranges = _chunk_ranges(n_stream, max(1, int(h_nbytes.sum()) // n_stream))
+    h_ends = h_starts + h_nbytes
+    with torch.cuda.device(dev):
+        cur = torch.cuda.current_stream(dev)
+        s_in, _ = _side_streams(dev)
+
+        def prep(feed, i):
+            a, b = ranges[i]
+            lo, hi = int(h_starts[a:b].min()), int(h_ends[a:b].max())
+            dc = torch.empty(max(hi - lo, 1), dtype=torch.uint8, device=dev)
+            feed.copy(dc[:hi - lo], src[lo:hi])
+            d_st = torch.from_numpy(h_starts[a:b] - lo).to(dev, non_blocking=True)
+            d_nb = torch.from_numpy(np.ascontiguousarray(h_nbytes[a:b])).to(dev, non_blocking=True)
+            e = torch.cuda.Event()
+            e.record(s_in)
+            return dc, d_st, d_nb, e, int(h_nbytes[a:b].max())
+
+        for (a, b), (dc, d_st, d_nb, e, max_nb) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
+            cur.wait_event(e)
+            for t in (dc, d_st, d_nb):
+                t.record_stream(cur)
+            verify_device(dc, d_st, d_nb, b - a, int(stream_size), is_int64, max_nb, hint, status[a:b])
+            del dc, d_st, d_nb
+    return to_host(status).reshape(shape)
 
 
 # -------------------------------------------------------------------------------------------------

@@ -157,6 +157,28 @@ int fab_decode(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_star
                void* stream);
 
 /*
+ * fab_decode with per-stream fault isolation (no reference equivalent: the reference fails the whole call).
+ * d_status[n_stream] (int32, device) receives 0 or the ERROR_DECODE_INIT / ERROR_DECODE_PROCESS bit of each
+ * stream; the output rows of failed streams are filled (0 for integer output, quiet NaN for float output);
+ * the mask fab_finish returns carries only call-level errors (CUDA, ALLOC, SAMPLE_RANGE, ...).  Only frames
+ * overlapping [first, last) are examined.  Same launches as fab_decode plus one fill kernel per 65535 streams.
+ * A NULL d_status makes the call a plain fab_decode.  Workspace: fab_decode_workspace_bytes.
+ */
+int fab_decode_isolated(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes,
+                        int64_t n_stream, int64_t stream_size, int is_int64, int64_t first_sample, int64_t last_sample,
+                        void* d_out, const void* d_offsets, const void* d_gains, int64_t max_nbytes, int blocksize_hint,
+                        int32_t* d_status, void* stream);
+/*
+ * Decode every frame of every stream and check it (CRC-8/16, syntax, frame chain, sample count) without writing
+ * samples; d_status as above.  A stream is accepted exactly when a full fab_decode of it succeeds (the same
+ * decoder stages, with the tile decoder's stores and the restore left out), so an archive can be checked after a
+ * transfer without room for its samples.  d_status must not be NULL (ERROR_ALLOC otherwise).
+ * Workspace: fab_decode_workspace_bytes.
+ */
+int fab_verify(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t* d_starts, const int64_t* d_nbytes, int64_t n_stream,
+               int64_t stream_size, int is_int64, int64_t max_nbytes, int blocksize_hint, int32_t* d_status, void* stream);
+
+/*
  * Decode many sample windows, each of its own stream and range, in one call (no reference equivalent).
  * Window w = (d_win_stream[w], d_win_first[w], d_win_last[w], d_win_out[w]) decodes samples [first, last)
  * of stream slot d_win_stream[w] in [0, n_stream) to d_out[d_win_out[w] ...] (counted in samples of the
