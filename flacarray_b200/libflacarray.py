@@ -10,6 +10,7 @@ torch tensors (device-resident; results stay on the device as torch tensors).  `
 `*_threaded` variants are accepted and ignored: the work is always parallel on the GPU.
 There is no CPU path: without the built library or without a CUDA device these functions raise.
 """
+import collections
 import ctypes as C
 import os
 import threading
@@ -172,21 +173,8 @@ def stream_std(data):
         d = src.to(dev, non_blocking=True)
         return to_host(stream_std_device(d.view(-1), n_stream, stream_size)).reshape(lead)
     with torch.cuda.device(dev):
-        cur = torch.cuda.current_stream(dev)
-        s_in, _ = _side_streams(dev)
-
-        def prep(feed, i):
-            a, b = ranges[i]
-            dc = torch.empty((b - a, stream_size), dtype=tdt, device=dev)
-            feed.copy(dc, src[a:b])
-            e = torch.cuda.Event()
-            e.record(s_in)
-            return dc, e
-
         parts = []
-        for (a, b), (dc, ev) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
-            cur.wait_event(ev)
-            dc.record_stream(cur)
+        for a, b, dc in _staged(dev, ranges, _rows_prep(src, dev)):
             parts.append(stream_std_device(dc.view(-1), b - a, stream_size))
             del dc
         return to_host(torch.cat(parts)).reshape(lead)
@@ -454,13 +442,13 @@ def _host_copy(dst, src):
 
 class _Feeder:
     """Host -> device copies on the input side stream, issued by one helper thread a few chunks ahead of
-    the kernels.  Pinned sources are copied in place.  Pageable sources (the usual numpy array) are
+    the kernels (_staged).  Pinned sources are copied in place.  Pageable sources (the usual numpy array) are
     first copied into one of two pinned staging buffers with torch's multi-threaded CPU copy -- a plain
     cudaMemcpy from pageable memory runs at a fraction of the PCIe rate and blocks the caller -- so
     staging chunk i+1 overlaps the transfer and the kernels of chunk i."""
 
-    def __init__(self, dev, s_in, prep, n_items, depth=2):
-        self.dev, self.s_in, self.prep, self.n, self.depth = dev, s_in, prep, n_items, depth
+    def __init__(self, s_in):
+        self.s_in = s_in
         self.stage = [None, None]
         self.stage_ev = [None, None]
         self.k = 0
@@ -484,28 +472,49 @@ class _Feeder:
         e.record(self.s_in)
         self.stage_ev[k] = e
 
-    def _run(self, i):
-        with torch.cuda.device(self.dev), torch.cuda.stream(self.s_in):
-            return self.prep(self, i)
 
-    def __iter__(self):
-        pool = _feeder_pool()
-        futs = []
-        nxt = 0
-        try:
-            for i in range(self.n):
-                while nxt < self.n and nxt <= i + self.depth:
-                    futs.append(pool.submit(self._run, nxt))
-                    nxt += 1
-                yield futs[i].result()
-                futs[i] = None
-        finally:
-            for f in futs:
-                if f is not None and not f.cancel():
-                    try:
-                        f.result()
-                    except Exception:  # noqa: BLE001 - the first error is already on its way up
-                        pass
+def _staged(dev, ranges, prep):
+    """The host -> device side of every host-buffer pipeline.  For each group of streams [a, b) in `ranges`, the helper
+    thread runs prep(feed, a, b) on the input side stream, up to two groups ahead of the caller: prep issues the group's
+    copies through feed.copy and returns what the group's kernels read.  Yields (a, b, *what prep returned) once the
+    current stream is ordered after those copies.  No reference to a yielded group is kept here, so its device buffers
+    go back to the caching allocator as soon as the caller drops them after queuing its kernels (record_stream keeps
+    them valid until those kernels have run)."""
+    cur = torch.cuda.current_stream(dev)
+    s_in = _side_streams(dev)[0]
+    feed = _Feeder(s_in)
+
+    def run(a, b):
+        with torch.cuda.device(dev), torch.cuda.stream(s_in):
+            bufs = prep(feed, a, b)
+            e = torch.cuda.Event()
+            e.record(s_in)
+        return e, bufs
+
+    def take(fut):
+        e, bufs = fut.result()
+        cur.wait_event(e)
+        for t in bufs:
+            if is_torch(t):
+                t.record_stream(cur)
+        return bufs
+
+    pool = _feeder_pool()
+    futs = collections.deque()
+    nxt = 0
+    try:
+        for i, (a, b) in enumerate(ranges):
+            while nxt < len(ranges) and nxt <= i + 2:
+                futs.append(pool.submit(run, *ranges[nxt]))
+                nxt += 1
+            yield (a, b, *take(futs.popleft()))
+    finally:
+        for f in futs:
+            if not f.cancel():
+                try:
+                    f.result()
+                except Exception:  # noqa: BLE001 - the first error is already on its way up
+                    pass
 
 
 def _as_host_tensor(a):
@@ -513,6 +522,42 @@ def _as_host_tensor(a):
     if not a.flags.writeable:
         a = a.copy()
     return torch.from_numpy(a)
+
+
+def _rows_prep(src, dev):
+    """_staged prep: rows [a, b) of a host tensor."""
+    def prep(feed, a, b):
+        dc = torch.empty((b - a,) + tuple(src.shape[1:]), dtype=src.dtype, device=dev)   # owned by s_in's pool
+        feed.copy(dc, src[a:b])
+        return (dc,)
+    return prep
+
+
+def _group_bytes(comp, starts, nbytes):
+    """The host bytes that stage one group of streams, and the streams' starts rebased into them.  The covering range
+    [min start, max end) is one plain copy; when it is more than twice the streams' own bytes (a sparse keep mask,
+    windows over scattered streams) only the streams' bytes are gathered."""
+    lo, hi = int(starts.min()), int((starts + nbytes).max())
+    if hi - lo <= 2 * int(nbytes.sum()):
+        return comp[lo:hi], starts - lo
+    rel = np.zeros(starts.size, np.int64)
+    np.cumsum(nbytes[:-1], out=rel[1:])
+    return np.concatenate([comp[int(s):int(s) + int(n)] for s, n in zip(starts, nbytes)]), rel
+
+
+def _bytes_prep(compressed, h_starts, h_nbytes, dev):
+    """_staged prep: the bytes of streams [a, b) of a host compressed buffer -> (device bytes, the streams' starts in
+    them, their nbytes, the largest of those nbytes)."""
+    comp = _as_host_tensor(compressed.numpy() if is_torch(compressed) else compressed).numpy()
+
+    def prep(feed, a, b):
+        part, rel = _group_bytes(comp, h_starts[a:b], h_nbytes[a:b])
+        dc = torch.empty(max(part.size, 1), dtype=torch.uint8, device=dev)
+        feed.copy(dc[:part.size], torch.from_numpy(part))
+        d_st = torch.from_numpy(rel).to(dev, non_blocking=True)
+        d_nb = torch.from_numpy(np.ascontiguousarray(h_nbytes[a:b])).to(dev, non_blocking=True)
+        return dc, d_st, d_nb, int(h_nbytes[a:b].max())
+    return prep
 
 
 def _encode_host(flat, n_stream, stream_size, level, quanta, dt, precision=None):
@@ -550,25 +595,14 @@ def _encode_host(flat, n_stream, stream_size, level, quanta, dt, precision=None)
                 None if gain is None else to_host(gain))
     with torch.cuda.device(dev):
         cur = torch.cuda.current_stream(dev)
-        s_in, s_out = _side_streams(dev)
-
-        def prep(feed, i):
-            a, b = ranges[i]
-            dc = torch.empty((b - a, stream_size), dtype=tdt, device=dev)   # owned by s_in's pool
-            feed.copy(dc, src[a:b])
-            e = torch.cuda.Event()
-            e.record(s_in)
-            return dc, e
-
+        s_out = _side_streams(dev)[1]
         raw_total = n_stream * stream_size * isz
         bound = int(_lib.lib().fab_encode_bound(n_stream, stream_size, _FAB[dt], level))
         host = None
         cap = 0
         pos = 0
         parts = []
-        for (a, b), (dc, ev) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
-            cur.wait_event(ev)
-            dc.record_stream(cur)
+        for a, b, dc in _staged(dev, ranges, _rows_prep(src, dev)):
             out, starts, nbytes, tot, off, gain = _encode_device_raw(dc.view(-1), b - a, stream_size, level,
                                                                      chunk_quanta(dc, a, b))
             del dc                # input chunk can go back to the pool
@@ -603,65 +637,6 @@ def _encode_host(flat, n_stream, stream_size, level, quanta, dt, precision=None)
             gain = to_host(torch.cat([p[3] for p in parts]))
         s_out.synchronize()
     return host[:pos].numpy(), starts, nbytes, off, gain
-
-
-def _decode_host(compressed, h_starts, h_nbytes, n_stream, stream_size, first_sample, last_sample, is_int64,
-                 offsets=None, gains=None, status=None):
-    """Host compressed bytes -> host samples (numpy, flat); optional int->float restore on the device.  status: int32
-    CUDA tensor [n_stream] for per-stream fault isolation (every chunk of streams fills its slice)."""
-    dev = _device()
-    n_decode = stream_size
-    if first_sample >= 0 and last_sample >= 0:
-        n_decode = last_sample - first_sample
-    h_starts = np.asarray(h_starts, dtype=np.int64).reshape(-1)
-    h_nbytes = np.asarray(h_nbytes, dtype=np.int64).reshape(-1)
-    restore = offsets is not None and gains is not None
-    if is_int64:
-        odt = torch.float64 if restore else torch.int64
-    else:
-        odt = torch.float32 if restore else torch.int32
-    isz = 8 if is_int64 else 4
-    hint = blocksize_hint(compressed, h_starts)
-    src = _as_host_tensor(compressed)
-    ranges = _chunk_ranges(n_stream, max(n_decode, 1) * isz)
-    h_ends = h_starts + h_nbytes
-    with torch.cuda.device(dev):
-        cur = torch.cuda.current_stream(dev)
-        s_in, s_out = _side_streams(dev)
-        fdt = torch.float64 if is_int64 else torch.float32
-        d_off = to_device(np.asarray(offsets).reshape(-1), dev, fdt) if restore else None
-        d_gain = to_device(np.asarray(gains).reshape(-1), dev, fdt) if restore else None
-        out_host = torch.empty((n_stream, max(n_decode, 0)), dtype=odt, pin_memory=True)
-
-        def prep(feed, i):
-            a, b = ranges[i]
-            # the byte range covering this chunk's streams (keep masks select sparse subsets)
-            lo = int(h_starts[a:b].min())
-            hi = int(h_ends[a:b].max())
-            dc = torch.empty(max(hi - lo, 1), dtype=torch.uint8, device=dev)
-            feed.copy(dc[:hi - lo], src[lo:hi])
-            d_st = torch.from_numpy(h_starts[a:b] - lo).to(dev, non_blocking=True)
-            d_nb = torch.from_numpy(np.ascontiguousarray(h_nbytes[a:b])).to(dev, non_blocking=True)
-            e = torch.cuda.Event()
-            e.record(s_in)
-            return dc, d_st, d_nb, e, int(h_nbytes[a:b].max())
-
-        for (a, b), (dc, d_st, d_nb, e, max_nb) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
-            cur.wait_event(e)
-            for t in (dc, d_st, d_nb):
-                t.record_stream(cur)
-            out = decode_device(dc, d_st, d_nb, b - a, int(stream_size), int(first_sample), int(last_sample), is_int64,
-                                max_nb, hint, None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b],
-                                None if status is None else status[a:b])
-            del dc, d_st, d_nb
-            e2 = torch.cuda.Event()
-            e2.record(cur)
-            out.record_stream(s_out)
-            s_out.wait_event(e2)
-            with torch.cuda.stream(s_out):
-                out_host[a:b].view(-1).copy_(out.view(odt), non_blocking=True)
-        s_out.synchronize()
-    return out_host.view(-1).numpy()
 
 
 def _wrap_encode(flatdata, n_stream, stream_size, level, dt):
@@ -794,32 +769,65 @@ def _check_byte_windows(h_starts, h_nbytes, n_compressed):
         raise RuntimeError("stream starts / nbytes point outside the compressed buffer")
 
 
-def _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64, status=None):
-    on_dev = is_torch(compressed) and compressed.is_cuda
-    h_starts = starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)
-    h_nbytes = nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)
-    _check_byte_windows(h_starts.reshape(-1), h_nbytes.reshape(-1), compressed.numel() if is_torch(compressed) else compressed.size)
-    if not on_dev:
-        if is_torch(compressed):
-            compressed = compressed.numpy()
-        return _decode_host(compressed, h_starts, h_nbytes, int(n_stream), int(stream_size), int(first_sample),
-                            int(last_sample), is_int64, status=status)
-    max_nb = int(h_nbytes.max()) if h_nbytes.size else 0
-    hint = blocksize_hint(compressed, h_starts)
-    d_starts = to_device(h_starts, compressed.device, torch.int64)
-    d_nbytes = to_device(h_nbytes, compressed.device, torch.int64)
-    return decode_device(compressed, d_starts, d_nbytes, int(n_stream), int(stream_size), int(first_sample),
-                         int(last_sample), is_int64, max_nb, hint, status=status)
+def _stream_index(compressed, starts, nbytes):
+    """The front door of every decode and verify: flat int64 host copies of starts and nbytes, checked against the
+    compressed buffer, whether that buffer is on the device, and the blocksize hint of the call."""
+    h_starts = np.asarray(starts.cpu().numpy() if is_torch(starts) else starts, dtype=np.int64).reshape(-1)
+    h_nbytes = np.asarray(nbytes.cpu().numpy() if is_torch(nbytes) else nbytes, dtype=np.int64).reshape(-1)
+    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
+    return h_starts, h_nbytes, is_torch(compressed) and compressed.is_cuda, blocksize_hint(compressed, h_starts)
+
+
+def _decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64, offsets=None,
+            gains=None, isolate=False):
+    """Decode streams [0, n_stream) into one flat array: a CUDA tensor for device bytes; numpy for host bytes, which go
+    to the device in groups of streams while the previous group's samples come back.  With offsets and gains the
+    samples are restored to floats on the device.  Returns (flat, status): with `isolate` status is the int32 numpy
+    per-stream status (each group fills its slice), else None."""
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
+    dev = compressed.device if on_dev else _device()
+    n_decode = last_sample - first_sample if (first_sample >= 0 and last_sample >= 0) else stream_size
+    fdt = torch.float64 if is_int64 else torch.float32
+    with torch.cuda.device(dev):
+        status = _status_tensor(dev, n_stream) if isolate else None
+        d_off = None if offsets is None else to_device(offsets, dev, fdt).reshape(-1)
+        d_gain = None if gains is None else to_device(gains, dev, fdt).reshape(-1)
+        if on_dev:
+            out = decode_device(compressed, to_device(h_starts, dev, torch.int64), to_device(h_nbytes, dev, torch.int64),
+                                n_stream, stream_size, first_sample, last_sample, is_int64,
+                                int(h_nbytes.max()) if h_nbytes.size else 0, hint, d_off, d_gain, status)
+        else:
+            odt = fdt if d_off is not None else (torch.int64 if is_int64 else torch.int32)
+            out_host = torch.empty((n_stream, max(n_decode, 0)), dtype=odt, pin_memory=True)
+            cur = torch.cuda.current_stream(dev)
+            s_out = _side_streams(dev)[1]
+            ranges = _chunk_ranges(n_stream, max(n_decode, 1) * (8 if is_int64 else 4))
+            for a, b, dc, d_st, d_nb, max_nb in _staged(dev, ranges, _bytes_prep(compressed, h_starts, h_nbytes, dev)):
+                out = decode_device(dc, d_st, d_nb, b - a, stream_size, first_sample, last_sample, is_int64, max_nb, hint,
+                                    None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b],
+                                    None if status is None else status[a:b])
+                del dc, d_st, d_nb
+                e = torch.cuda.Event()
+                e.record(cur)
+                out.record_stream(s_out)
+                s_out.wait_event(e)
+                with torch.cuda.stream(s_out):
+                    out_host[a:b].view(-1).copy_(out.view(odt), non_blocking=True)
+            s_out.synchronize()
+            out = out_host.view(-1).numpy()
+    return out, None if status is None else to_host(status)
 
 
 def wrap_decode_i32(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, use_threads):
     """pyx:597-653.  Returns the flat int32 array."""
-    return _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, False)
+    return _decode(compressed, starts, nbytes, int(n_stream), int(stream_size), int(first_sample), int(last_sample),
+                   False)[0]
 
 
 def wrap_decode_i64(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, use_threads):
     """pyx:655-711."""
-    return _wrap_decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, True)
+    return _decode(compressed, starts, nbytes, int(n_stream), int(stream_size), int(first_sample), int(last_sample),
+                   True)[0]
 
 
 def check_on_error(on_error):
@@ -829,9 +837,8 @@ def check_on_error(on_error):
     raise ValueError(f"on_error must be 'raise' or 'fill', not {on_error!r}")
 
 
-def _status_tensor(compressed, n_stream):
+def _status_tensor(dev, n_stream):
     """Device int32 [n_stream] for the per-stream status of an isolated decode or a verify."""
-    dev = compressed.device if (is_torch(compressed) and compressed.is_cuda) else _device()
     return torch.empty(max(n_stream, 1), dtype=torch.int32, device=dev)[:n_stream]
 
 
@@ -866,22 +873,11 @@ def decode_flac(compressed, starts, nbytes, stream_size, first_sample=-1, last_s
     if first_sample >= 0 and last_sample >= 0:
         n_decode = last_sample - first_sample
 
-    output_shape = tuple(starts.shape) + (n_decode,)
-    n_stream = int(np.prod(starts.shape))
-    flat_starts = starts.reshape((-1,))
-    flat_nbytes = nbytes.reshape((-1,))
-    if isolate:
-        status = _status_tensor(compressed, n_stream)
-        flat_output = _wrap_decode(compressed, flat_starts, flat_nbytes, n_stream, stream_size, first_sample, last_sample,
-                                   is_int64, status=status)
-        return flat_output.reshape(output_shape), to_host(status).reshape(tuple(starts.shape))
-    if is_int64:
-        flat_output = wrap_decode_i64(compressed, flat_starts, flat_nbytes, n_stream, stream_size, first_sample,
-                                      last_sample, use_threads)
-    else:
-        flat_output = wrap_decode_i32(compressed, flat_starts, flat_nbytes, n_stream, stream_size, first_sample,
-                                      last_sample, use_threads)
-    return flat_output.reshape(output_shape)
+    lead = tuple(starts.shape)
+    out, status = _decode(compressed, starts.reshape((-1,)), nbytes.reshape((-1,)), int(np.prod(lead)), int(stream_size),
+                          int(first_sample), int(last_sample), is_int64, isolate=isolate)
+    out = out.reshape(lead + (n_decode,))
+    return (out, status.reshape(lead)) if isolate else out
 
 
 # -------------------------------------------------------------------------------------------------
@@ -931,35 +927,11 @@ def decode_flac_float(compressed, starts, nbytes, stream_size, offsets, gains, f
     _check_sample_range(stream_size, first_sample, last_sample)
     if first_sample >= 0 and last_sample >= 0:
         n_decode = last_sample - first_sample
-    output_shape = tuple(starts.shape) + (n_decode,)
-    n_stream = int(np.prod(starts.shape))
-    on_dev = is_torch(compressed) and compressed.is_cuda
-    h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1)
-    h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1)
-    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
-    status = _status_tensor(compressed, n_stream) if isolate else None
-
-    def result(out):
-        out = out.reshape(output_shape)
-        return (out, to_host(status).reshape(tuple(starts.shape))) if isolate else out
-
-    if not on_dev:
-        if is_torch(compressed):
-            compressed = compressed.numpy()
-        out = _decode_host(compressed, h_starts, h_nbytes, n_stream, int(stream_size), int(first_sample), int(last_sample),
-                           is_int64, offsets, gains, status=status)
-        return result(out)
-    max_nb = int(h_nbytes.max()) if h_nbytes.size else 0
-    hint = blocksize_hint(compressed, h_starts)
-    comp = compressed
-    d_starts = to_device(h_starts, comp.device, torch.int64)
-    d_nbytes = to_device(h_nbytes, comp.device, torch.int64)
-    fdt = torch.float64 if is_int64 else torch.float32
-    off = to_device(offsets.reshape((-1,)), comp.device, fdt)
-    gain = to_device(gains.reshape((-1,)), comp.device, fdt)
-    out = decode_device(comp, d_starts, d_nbytes, n_stream, int(stream_size), int(first_sample), int(last_sample),
-                        is_int64, max_nb, hint, off, gain, status=status)
-    return result(out)
+    lead = tuple(starts.shape)
+    out, status = _decode(compressed, starts, nbytes, int(np.prod(lead)), int(stream_size), int(first_sample),
+                          int(last_sample), is_int64, offsets, gains, isolate)
+    out = out.reshape(lead + (n_decode,))
+    return (out, status.reshape(lead)) if isolate else out
 
 
 # -------------------------------------------------------------------------------------------------
@@ -989,44 +961,19 @@ def verify_flac(compressed, starts, nbytes, stream_size, is_int64=False):
     if stream_size <= 0:
         raise RuntimeError("You must specify the non-zero output stream size")
     shape = tuple(starts.shape)
-    h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1).astype(np.int64)
-    h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1).astype(np.int64)
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
     n_stream = h_starts.size
-    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
     if n_stream == 0:
         return np.zeros(shape, np.int32)
-    status = _status_tensor(compressed, n_stream)
-    hint = blocksize_hint(compressed, h_starts)
-    if is_torch(compressed) and compressed.is_cuda:
-        dev = compressed.device
+    dev = compressed.device if on_dev else _device()
+    status = _status_tensor(dev, n_stream)
+    if on_dev:
         verify_device(compressed, to_device(h_starts, dev, torch.int64), to_device(h_nbytes, dev, torch.int64), n_stream,
                       int(stream_size), is_int64, int(h_nbytes.max()), hint, status)
         return to_host(status).reshape(shape)
-    if is_torch(compressed):
-        compressed = compressed.numpy()
-    dev = status.device
-    src = _as_host_tensor(compressed)
     ranges = _chunk_ranges(n_stream, max(1, int(h_nbytes.sum()) // n_stream))
-    h_ends = h_starts + h_nbytes
     with torch.cuda.device(dev):
-        cur = torch.cuda.current_stream(dev)
-        s_in, _ = _side_streams(dev)
-
-        def prep(feed, i):
-            a, b = ranges[i]
-            lo, hi = int(h_starts[a:b].min()), int(h_ends[a:b].max())
-            dc = torch.empty(max(hi - lo, 1), dtype=torch.uint8, device=dev)
-            feed.copy(dc[:hi - lo], src[lo:hi])
-            d_st = torch.from_numpy(h_starts[a:b] - lo).to(dev, non_blocking=True)
-            d_nb = torch.from_numpy(np.ascontiguousarray(h_nbytes[a:b])).to(dev, non_blocking=True)
-            e = torch.cuda.Event()
-            e.record(s_in)
-            return dc, d_st, d_nb, e, int(h_nbytes[a:b].max())
-
-        for (a, b), (dc, d_st, d_nb, e, max_nb) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
-            cur.wait_event(e)
-            for t in (dc, d_st, d_nb):
-                t.record_stream(cur)
+        for a, b, dc, d_st, d_nb, max_nb in _staged(dev, ranges, _bytes_prep(compressed, h_starts, h_nbytes, dev)):
             verify_device(dc, d_st, d_nb, b - a, int(stream_size), is_int64, max_nb, hint, status[a:b])
             del dc, d_st, d_nb
     return to_host(status).reshape(shape)
@@ -1096,10 +1043,8 @@ def decode_windows(compressed, starts, nbytes, stream_size, streams, first, last
         raise RuntimeError("You must specify the non-zero output stream size")
     if (offsets is None) != (gains is None):
         raise RuntimeError("Offsets and gains must be given together")
-    h_starts = (starts.cpu().numpy() if is_torch(starts) else np.asarray(starts)).reshape(-1).astype(np.int64)
-    h_nbytes = (nbytes.cpu().numpy() if is_torch(nbytes) else np.asarray(nbytes)).reshape(-1).astype(np.int64)
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
     n_stream = h_starts.size
-    _check_byte_windows(h_starts, h_nbytes, compressed.numel() if is_torch(compressed) else compressed.size)
     s, f, l_ = _window_records(n_stream, int(stream_size), streams, first, last)
     restore = offsets is not None
     woff = np.zeros(s.size + 1, np.int64)
@@ -1110,7 +1055,6 @@ def decode_windows(compressed, starts, nbytes, stream_size, streams, first, last
     else:
         odt = torch.float32 if restore else torch.int32
     idt = torch.int64 if is_int64 else torch.int32
-    on_dev = is_torch(compressed) and compressed.is_cuda
     if s.size == 0:
         if on_dev:
             return torch.empty(0, dtype=odt, device=compressed.device), woff
@@ -1124,7 +1068,6 @@ def decode_windows(compressed, starts, nbytes, stream_size, streams, first, last
     if restore:
         h_off = np.asarray(offsets.cpu() if is_torch(offsets) else offsets).reshape(-1)[uniq]
         h_gain = np.asarray(gains.cpu() if is_torch(gains) else gains).reshape(-1)[uniq]
-    hint = blocksize_hint(compressed, u_starts)
     if on_dev:
         dev = compressed.device
         out = torch.empty(max(total, 1), dtype=idt, device=dev)
@@ -1143,8 +1086,6 @@ def _decode_windows_host(compressed, u_starts, u_nbytes, stream_size, inv, f, l_
                          h_gain):
     """Host compressed bytes: the referenced streams' bytes go to the device in staged copies, in groups of streams
     (_chunk_ranges) when they exceed one chunk; every group decodes its windows into one packed device output."""
-    if is_torch(compressed):
-        compressed = compressed.numpy()
     dev = _device()
     total = int(woff[-1])
     n_u = u_starts.size
@@ -1152,43 +1093,23 @@ def _decode_windows_host(compressed, u_starts, u_nbytes, stream_size, inv, f, l_
     order = np.argsort(inv, kind="stable")          # windows grouped by stream slot
     bounds = np.searchsorted(inv[order], np.arange(n_u + 1))
     ranges = _chunk_ranges(n_u, max(1, int(u_nbytes.sum()) // n_u))
-    src = _as_host_tensor(compressed)
+    stream_bytes = _bytes_prep(compressed, u_starts, u_nbytes, dev)
+
+    def prep(feed, a, b):
+        sel = order[bounds[a]:bounds[b]]
+        return stream_bytes(feed, a, b) + tuple(torch.from_numpy(np.ascontiguousarray(x)).to(dev, non_blocking=True)
+                                                for x in (inv[sel] - a, f[sel], l_[sel], sel.astype(np.int64)))
+
     with torch.cuda.device(dev):
-        cur = torch.cuda.current_stream(dev)
-        s_in, _ = _side_streams(dev)
         fdt = torch.float64 if is_int64 else torch.float32
         out = torch.empty(max(total, 1), dtype=idt, device=dev)
         d_wout = to_device(woff[:-1], dev, torch.int64)
-
-        def prep(feed, i):
-            a, b = ranges[i]
-            st, nb = u_starts[a:b], u_nbytes[a:b]
-            lo, hi = int(st.min()), int((st + nb).max())
-            if hi - lo == int(nb.sum()):                 # back to back (any order): one contiguous range
-                part, rel = src[lo:hi], st - lo
-            else:                                        # gather the streams' bytes into one buffer first
-                rel = np.zeros(b - a, np.int64)
-                np.cumsum(nb[:-1], out=rel[1:])
-                part = torch.from_numpy(np.concatenate([compressed[int(x):int(x) + int(n)] for x, n in zip(st, nb)]))
-            dc = torch.empty(max(part.numel(), 1), dtype=torch.uint8, device=dev)
-            feed.copy(dc[:part.numel()], part)
-            sel = order[bounds[a]:bounds[b]]
-            dw = [torch.from_numpy(np.ascontiguousarray(x)).to(dev, non_blocking=True)
-                  for x in (rel, nb, inv[sel] - a, f[sel], l_[sel], sel.astype(np.int64))]
-            e = torch.cuda.Event()
-            e.record(s_in)
-            return dc, dw, e, int(nb.max())
-
         d_off = to_device(h_off, dev, fdt) if restore else None
         d_gain = to_device(h_gain, dev, fdt) if restore else None
-        for (a, b), (dc, dw, e, max_nb) in zip(ranges, _Feeder(dev, s_in, prep, len(ranges))):
-            cur.wait_event(e)
-            for t in [dc] + dw:
-                t.record_stream(cur)
-            d_st, d_nb, d_ws, d_wf, d_wl, d_sel = dw
-            d_wo = d_wout[d_sel]
-            decode_windows_device(dc, d_st, d_nb, b - a, stream_size, is_int64, d_ws, d_wf, d_wl, d_wo, out, max_nb, hint,
-                                  None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b])
-            del dc, dw, d_st, d_nb, d_ws, d_wf, d_wl, d_sel, d_wo
+        for a, b, dc, d_st, d_nb, max_nb, d_ws, d_wf, d_wl, d_sel in _staged(dev, ranges, prep):
+            decode_windows_device(dc, d_st, d_nb, b - a, stream_size, is_int64, d_ws, d_wf, d_wl, d_wout[d_sel], out,
+                                  max_nb, hint, None if d_off is None else d_off[a:b],
+                                  None if d_gain is None else d_gain[a:b])
+            del dc, d_st, d_nb, d_ws, d_wf, d_wl, d_sel
         host = to_host(out[:total].view(odt))
     return host
