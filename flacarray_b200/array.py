@@ -15,7 +15,7 @@ import copy
 import numpy as np
 
 from .compress import array_compress
-from .decompress import array_decompress_slice, array_decompress_windows, array_verify
+from .decompress import array_decompress_slice, array_decompress_windows, array_verify, stats_slice
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -344,6 +344,38 @@ class FlacArray:
         status = array_verify(self._compressed, self._stream_size, self._stream_starts, self._stream_nbytes,
                               is_int64=self._is_int64)
         return status.reshape(self._leading_shape)
+
+    def stats(self, keep=None, stream_slice=None, bin=None, keep_indices=False, on_error="raise"):
+        """Per-stream and per-bin count, min, max, mean and std of the local data without decompressing it into memory
+        (array_stats).  `keep` and `stream_slice` select as to_array does, except that the slice is normalised like an
+        index (None and negative bounds allowed; its step must be 1).  `bin`: None (one bin) or a bin length >= 1.
+        Returns a StreamStats whose arrays have to_array's shape with the sample axis replaced by the bin axis (dropped
+        for bin=None), or (stats, indices) with `keep` and `keep_indices`.  on_error="fill" adds the int32 status last,
+        as to_array does."""
+        first, last = 0, self._stream_size
+        if stream_slice is not None:
+            first, last, step = stream_slice.indices(self._stream_size)
+            if step != 1:
+                raise ValueError("Only stream slices with a step size of 1 are supported")
+        stats, indices, status = stats_slice(
+            self._compressed,
+            self._stream_size,
+            self._stream_starts,
+            self._stream_nbytes,
+            stream_offsets=self._stream_offsets,
+            stream_gains=self._stream_gains,
+            keep=keep,
+            first_stream_sample=first,
+            last_stream_sample=last,
+            bin=bin,
+            is_int64=self._is_int64,
+            no_flatten=(not self._flatten_single),
+            on_error=on_error,
+        )
+        res = (stats, indices) if (keep is not None and keep_indices) else (stats,)
+        if status is not None:
+            res = res + (status,)
+        return res[0] if len(res) == 1 else res
 
     def to_windows(self, streams, first, last):
         """Decompress many sample windows of local streams in one call.

@@ -24,6 +24,7 @@
 #include "fa_encode.h"
 #include "fa_encode_fixed.h"
 #include "fa_quant.h"
+#include "fa_stats.h"
 
 using namespace fa;
 
@@ -448,6 +449,18 @@ __global__ void __launch_bounds__(256) k_dec_fill_failed(const int* __restrict__
     if (status[s] == 0) return;
     W* o = out + s * n_per_stream;
     for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n_per_stream; i += (int64_t)gridDim.x * 256) o[i] = fill;
+}
+
+// ---- fab_row_stats (fa_stats.h): grid = (pieces / kStatsWarps, rows of one slab); one warp per piece / per bin -------
+template <bool I64>
+__global__ void __launch_bounds__(kStatsWarps * 32) k_row_stats(const StatsParams P, int64_t row0) {
+    const int64_t idx = (int64_t)blockIdx.x * kStatsWarps + (threadIdx.x >> 5);
+    if (idx < P.nbins * P.ppb) stats_piece_warp<I64>(P, row0 + blockIdx.y, idx);
+}
+
+__global__ void __launch_bounds__(kStatsWarps * 32) k_row_stats_merge(const StatsParams P, int64_t row0) {
+    const int64_t b = (int64_t)blockIdx.x * kStatsWarps + (threadIdx.x >> 5);
+    if (b < P.nbins) stats_merge_warp(P, row0 + blockIdx.y, b);
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
@@ -1328,6 +1341,76 @@ extern "C" int fab_decode_windows(fab_ctx* ctx, const unsigned char* d_bytes, co
         if (fuse_restore) k_restore_win<false><<<(unsigned)((total + 3) / 4), 128, 0, st>>>(TP, total);
         else k_restore_win<true><<<(unsigned)((total + 3) / 4), 128, 0, st>>>(TP, total);
         ctx->launches++;
+    }
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+// =================================================================================================
+// Per-row, per-bin statistics of decoded integer rows
+// =================================================================================================
+// bin == 0: one bin per row.  Returns 0 and fills *P's geometry, or the error bits of bad arguments.
+static int stats_geometry(int64_t n_rows, int64_t n, int64_t bin, int is_int64, StatsParams* P) {
+    if (n_rows <= 0) return ERROR_ZERO_NSTREAM;
+    if (n <= 0) return ERROR_ZERO_STREAMSIZE;
+    if (bin < 0) return ERROR_DECODE_SAMPLE_RANGE;
+    const int64_t len = bin == 0 ? n : std::min(bin, n);
+    if (len > kStatsMaxBin) return ERROR_DECODE_SAMPLE_RANGE;
+    P->is_int64 = is_int64 ? 1 : 0;
+    P->n_rows = n_rows; P->n = n; P->bin = len;
+    P->nbins = (n + len - 1) / len;
+    P->piece = kStatsPieceBytes / (is_int64 ? 8 : 4);
+    P->ppb = (len + P->piece - 1) / P->piece;
+    if ((P->nbins * P->ppb + kStatsWarps - 1) / kStatsWarps > 0x7FFFFFFFll) return ERROR_ALLOC;
+    return 0;
+}
+
+static size_t stats_workspace(const StatsParams& P) {
+    return P.ppb > 1 ? align256((size_t)P.n_rows * (size_t)P.nbins * (size_t)P.ppb * sizeof(StatPart)) : 0;
+}
+
+extern "C" int64_t fab_row_stats_workspace_bytes(int64_t n_rows, int64_t n, int64_t bin, int is_int64) {
+    StatsParams P{};
+    if (stats_geometry(n_rows, n, bin, is_int64, &P)) return -1;
+    return (int64_t)stats_workspace(P);
+}
+
+extern "C" int fab_row_stats(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, int64_t bin,
+                             const void* d_offsets, const void* d_gains, const int32_t* d_status, int64_t* d_count,
+                             void* d_min, void* d_max, double* d_mean, double* d_std, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    StatsParams P{};
+    int rc = stats_geometry(n_rows, n, bin, is_int64, &P);
+    if (rc) return rc;
+    if ((d_offsets == nullptr) != (d_gains == nullptr) || ((uintptr_t)d_rows & (is_int64 ? 7 : 3)) != 0) {
+        ctx->last_error = "fab_row_stats: offsets and gains go together, and d_rows must be aligned to its element size";
+        return ERROR_CONVERT_TYPE;
+    }
+    if (!d_rows || !d_count || !d_min || !d_max || !d_mean || !d_std) {
+        ctx->last_error = "fab_row_stats: d_rows and the five result arrays must not be NULL";
+        return ERROR_ALLOC;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t ws = stats_workspace(P);
+    if (ws) {
+        unsigned char* scr;
+        rc = ctx_scratch(ctx, ws, &scr, st);
+        if (rc) return rc;
+        P.part = (StatPart*)scr;
+    }
+    P.rows = d_rows; P.offsets = d_offsets; P.gains = d_gains; P.status = d_status;
+    P.count = (long long*)d_count; P.mn = d_min; P.mx = d_max; P.mean = d_mean; P.std = d_std;
+    const unsigned gx = (unsigned)((P.nbins * P.ppb + kStatsWarps - 1) / kStatsWarps);
+    const unsigned gm = (unsigned)((P.nbins + kStatsWarps - 1) / kStatsWarps);
+    for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {
+        const dim3 grid(gx, (unsigned)std::min<int64_t>(65535, n_rows - r0));
+        if (is_int64) k_row_stats<true><<<grid, kStatsWarps * 32, 0, st>>>(P, r0);
+        else k_row_stats<false><<<grid, kStatsWarps * 32, 0, st>>>(P, r0);
+        ctx->launches++;
+        if (P.ppb > 1) {
+            k_row_stats_merge<<<dim3(gm, grid.y), kStatsWarps * 32, 0, st>>>(P, r0);
+            ctx->launches++;
+        }
     }
     FAB_CUDA(ctx, cudaGetLastError());
     return 0;

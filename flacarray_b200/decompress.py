@@ -2,10 +2,12 @@
 /root/reference/src/flacarray/decompress.py:18-205 (keep mask, sample window, single-stream
 flattening rules, error messages), plus on_error="fill" (per-stream fault isolation);
 array_decompress_windows: many per-stream sample windows in one decode; array_verify: check streams without
-decoding them out.  The FLAC decode and the int->float restore run on the device."""
+decoding them out; array_stats: per-stream and per-bin statistics without decoding the array out.  The FLAC decode, the
+int->float restore and the statistics run on the device."""
 import numpy as np
 
-from .libflacarray import check_on_error, decode_flac, decode_flac_float, decode_windows, is_torch, verify_flac
+from .libflacarray import (StreamStats, check_bin, check_on_error, decode_flac, decode_flac_float, decode_windows,
+                           is_torch, stats_flac, verify_flac)
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -182,3 +184,85 @@ def array_verify(compressed, stream_size, stream_starts, stream_nbytes, is_int64
         stream_starts = ensure_one_element(stream_starts, np.int64)
         stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
     return verify_flac(compressed, stream_starts, stream_nbytes, stream_size, is_int64=is_int64)
+
+
+def stats_slice(compressed, stream_size, stream_starts, stream_nbytes, stream_offsets=None, stream_gains=None, keep=None,
+                first_stream_sample=None, last_stream_sample=None, bin=None, is_int64=False, no_flatten=False,
+                on_error="raise"):
+    """array_stats with the index tuples of the kept streams and FlacArray's flattening rule: returns (StreamStats,
+    indices, status), status None unless on_error="fill"."""
+    isolate = check_on_error(on_error)
+    if (stream_offsets is None) != (stream_gains is None):
+        raise RuntimeError("Offsets and gains must be given together")
+    restored = stream_offsets is not None
+    first = 0 if first_stream_sample is None else int(first_stream_sample)
+    last = int(stream_size) if last_stream_sample is None else int(last_stream_sample)
+    if first < 0 or last > stream_size:
+        raise ValueError(f"sample range [{first}, {last}) lies outside the stream of {stream_size} samples")
+    if last <= first:
+        raise ValueError(f"sample range [{first}, {last}) is empty")
+    length = check_bin(bin, last - first)
+    nbins = -(-(last - first) // length)
+
+    single = not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts)) or tuple(stream_starts.shape) == (1,)
+    if single:
+        fdt = np.float64 if is_int64 else np.float32
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+        if restored:
+            stream_offsets = ensure_one_element(stream_offsets, fdt)
+            stream_gains = ensure_one_element(stream_gains, fdt)
+    starts, nbytes, indices = keep_select(keep, _host(stream_starts), _host(stream_nbytes))
+    offsets = select_keep_indices(None if not restored else _host(stream_offsets), indices)
+    gains = select_keep_indices(None if not restored else _host(stream_gains), indices)
+    lead = tuple(starts.shape)
+    tail = () if bin is None else (nbins,)
+    if starts.size == 0:
+        vdt = _result_dtype(is_int64, restored)
+        z = lead + tail
+        stats = StreamStats(np.zeros(z, np.int64), np.zeros(z, vdt), np.zeros(z, vdt), np.zeros(z), np.zeros(z))
+        status = np.zeros(lead, np.int32)
+    else:
+        stats, status = stats_flac(compressed, starts, nbytes, stream_size, first, last, bin, offsets, gains, is_int64,
+                                   isolate)
+        stats = StreamStats(*(v.reshape(lead + tail) for v in stats))
+        status = None if status is None else status.reshape(lead)
+    if single and not no_flatten:
+        stats = StreamStats(*(v.reshape(tail) for v in stats))
+    return stats, indices, (status if isolate else None)
+
+
+@function_timer
+def array_stats(
+    compressed,
+    stream_size,
+    stream_starts,
+    stream_nbytes,
+    stream_offsets=None,
+    stream_gains=None,
+    keep=None,
+    first_stream_sample=None,
+    last_stream_sample=None,
+    bin=None,
+    is_int64=False,
+    on_error="raise",
+):
+    """Per-stream and per-bin statistics of the decompressed samples without materialising them.
+
+    Streams and samples are selected as in array_decompress_slice (`keep`, [first_stream_sample, last_stream_sample),
+    offsets and gains both or neither).  `bin`: None for one bin over the whole sample range, or an integer B >= 1 that
+    cuts the range into ceil(n / B) bins of B samples (the last one may be shorter); a bin may hold at most 2^32 - 1
+    samples.  Returns StreamStats(count, min, max, mean, std): each array has the shape array_decompress_slice's result
+    would have with the sample axis replaced by the bin axis (dropped when bin is None).  count is int64, min / max are
+    in the array's dtype and equal to the decoded samples' min / max, mean and std (population, ddof = 0) are float64:
+    the sums are exact integers, then mean = S / n and std = sqrt(n*Q - S^2) / n are each rounded once, and floats go
+    through the restore's offset and coefficient.
+
+    Compressed bytes on the device are decoded there in groups of streams; host bytes are copied to the device in
+    groups.  Only the statistics come back.  on_error="fill" returns (stats, status) as array_decompress does: a stream
+    that cannot be decoded gets count 0, NaN mean / std and NaN (floats) or 0 (integers) min / max.
+    """
+    stats, _, status = stats_slice(compressed, stream_size, stream_starts, stream_nbytes, stream_offsets=stream_offsets,
+                                   stream_gains=stream_gains, keep=keep, first_stream_sample=first_stream_sample,
+                                   last_stream_sample=last_stream_sample, bin=bin, is_int64=is_int64, on_error=on_error)
+    return (stats, status) if status is not None else stats

@@ -778,6 +778,29 @@ def _stream_index(compressed, starts, nbytes):
     return h_starts, h_nbytes, is_torch(compressed) and compressed.is_cuda, blocksize_hint(compressed, h_starts)
 
 
+def _decode_groups(compressed, h_starts, h_nbytes, on_dev, hint, dev, ranges, stream_size, first_sample, last_sample,
+                   is_int64, d_off=None, d_gain=None, status=None):
+    """The per-group decode shared by every whole-stream decode: for each group of streams [a, b) in `ranges` yields
+    (a, b, the group's flat CUDA output).  Device bytes are decoded in place; host bytes reach the device through
+    _staged.  d_off / d_gain (restore) and status (per-stream isolation) are CUDA tensors over all n streams, and each
+    group gets its slice.  A group's output goes back to the caching allocator when the caller drops it."""
+    def part(t, a, b):
+        return None if t is None else t[a:b]
+
+    if on_dev:
+        d_st, d_nb = to_device(h_starts, dev, torch.int64), to_device(h_nbytes, dev, torch.int64)
+        for a, b in ranges:
+            yield a, b, decode_device(compressed, d_st[a:b], d_nb[a:b], b - a, stream_size, first_sample, last_sample,
+                                      is_int64, int(h_nbytes[a:b].max()) if b > a else 0, hint, part(d_off, a, b),
+                                      part(d_gain, a, b), part(status, a, b))
+        return
+    for a, b, dc, d_st, d_nb, max_nb in _staged(dev, ranges, _bytes_prep(compressed, h_starts, h_nbytes, dev)):
+        out = decode_device(dc, d_st, d_nb, b - a, stream_size, first_sample, last_sample, is_int64, max_nb, hint,
+                            part(d_off, a, b), part(d_gain, a, b), part(status, a, b))
+        del dc, d_st, d_nb
+        yield a, b, out
+
+
 def _decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, last_sample, is_int64, offsets=None,
             gains=None, isolate=False):
     """Decode streams [0, n_stream) into one flat array: a CUDA tensor for device bytes; numpy for host bytes, which go
@@ -793,20 +816,17 @@ def _decode(compressed, starts, nbytes, n_stream, stream_size, first_sample, las
         d_off = None if offsets is None else to_device(offsets, dev, fdt).reshape(-1)
         d_gain = None if gains is None else to_device(gains, dev, fdt).reshape(-1)
         if on_dev:
-            out = decode_device(compressed, to_device(h_starts, dev, torch.int64), to_device(h_nbytes, dev, torch.int64),
-                                n_stream, stream_size, first_sample, last_sample, is_int64,
-                                int(h_nbytes.max()) if h_nbytes.size else 0, hint, d_off, d_gain, status)
+            # one group: the whole decode is one call and its output is the result
+            (_, _, out), = _decode_groups(compressed, h_starts, h_nbytes, True, hint, dev, [(0, n_stream)], stream_size,
+                                          first_sample, last_sample, is_int64, d_off, d_gain, status)
         else:
             odt = fdt if d_off is not None else (torch.int64 if is_int64 else torch.int32)
             out_host = torch.empty((n_stream, max(n_decode, 0)), dtype=odt, pin_memory=True)
             cur = torch.cuda.current_stream(dev)
             s_out = _side_streams(dev)[1]
             ranges = _chunk_ranges(n_stream, max(n_decode, 1) * (8 if is_int64 else 4))
-            for a, b, dc, d_st, d_nb, max_nb in _staged(dev, ranges, _bytes_prep(compressed, h_starts, h_nbytes, dev)):
-                out = decode_device(dc, d_st, d_nb, b - a, stream_size, first_sample, last_sample, is_int64, max_nb, hint,
-                                    None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b],
-                                    None if status is None else status[a:b])
-                del dc, d_st, d_nb
+            for a, b, out in _decode_groups(compressed, h_starts, h_nbytes, False, hint, dev, ranges, stream_size,
+                                            first_sample, last_sample, is_int64, d_off, d_gain, status):
                 e = torch.cuda.Event()
                 e.record(cur)
                 out.record_stream(s_out)
@@ -977,6 +997,99 @@ def verify_flac(compressed, starts, nbytes, stream_size, is_int64=False):
             verify_device(dc, d_st, d_nb, b - a, int(stream_size), is_int64, max_nb, hint, status[a:b])
             del dc, d_st, d_nb
     return to_host(status).reshape(shape)
+
+
+# -------------------------------------------------------------------------------------------------
+# Statistics: count, min, max, mean and std per stream and bin, reduced from the decoded integers on the device
+# (fab_row_stats; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+_STATS_GROUP_BYTES = 4 << 30      # decoded integers of one group of device-resident streams (see DESIGN.md section 6)
+_MAX_BIN = (1 << 32) - 1          # a bin's exact sums are sized for at most this many samples
+
+StreamStats = collections.namedtuple("StreamStats", ["count", "min", "max", "mean", "std"])
+
+
+def check_bin(bin, n_decode):
+    """The bin length of a stats call over n_decode samples: None is one bin of all of them, else an integer >= 1 (a bin
+    longer than the range is one bin).  Raises ValueError for anything else and for bins of more than 2^32 - 1."""
+    if bin is not None and (isinstance(bin, bool) or not isinstance(bin, (int, np.integer)) or int(bin) < 1):
+        raise ValueError(f"bin must be None or an integer >= 1, not {bin!r}")
+    length = n_decode if bin is None else min(int(bin), n_decode)
+    if length > _MAX_BIN:
+        raise ValueError(f"a bin of {length} samples is longer than the 2^32 - 1 samples a bin may hold")
+    return length
+
+
+def _stats_ranges(n_stream, row_bytes, cap):
+    """Whole-stream groups of device-resident streams whose decoded rows take at most `cap` bytes (one stream at least)."""
+    per = max(1, cap // max(row_bytes, 1))
+    return [(a, min(a + per, n_stream)) for a in range(0, n_stream, per)]
+
+
+def row_stats_device(rows, is_int64, n_rows, n, bin, offsets, gains, status, count, mn, mx, mean, std):
+    """Device-level fab_row_stats over CUDA tensors; bin = 0 is one bin per row."""
+    dev = rows.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_row_stats(ctx.handle, _ptr(rows), 1 if is_int64 else 0, n_rows, n, bin, _ptr(offsets),
+                                      _ptr(gains), _ptr(status), _ptr(count), _ptr(mn), _ptr(mx), _ptr(mean), _ptr(std), st)
+        if rc != 0:
+            _check(rc, ctx, st, "Statistics")
+
+
+def stats_flac(compressed, starts, nbytes, stream_size, first_sample, last_sample, bin, offsets=None, gains=None,
+               is_int64=False, isolate=False):
+    """count, min, max, mean and std of samples [first_sample, last_sample) of every stream, per bin of `bin` samples
+    (None: one bin), without storing the decoded array: groups of streams are decoded to integers on the device and
+    reduced there by fab_row_stats; only the statistics come back.  Offsets and gains (both or neither) give the float
+    statistics of the restored samples.  Returns (StreamStats of numpy arrays [n_stream, nbins], status): status is the
+    int32 per-stream status with `isolate` (failed streams are filled), else None and a failed decode raises."""
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
+    n_stream = h_starts.size
+    n_decode = last_sample - first_sample
+    length = check_bin(bin, n_decode)
+    nbins = -(-n_decode // length)
+    dev = compressed.device if on_dev else _device()
+    fdt = torch.float64 if is_int64 else torch.float32
+    restore = offsets is not None
+    vdt = fdt if restore else (torch.int64 if is_int64 else torch.int32)
+    vsz = 8 if is_int64 else 4
+    m = n_stream * nbins
+    with torch.cuda.device(dev):
+        # every result in one device buffer, so that they come back in one copy
+        res = torch.empty(24 * m + 2 * vsz * m + 4 * n_stream + 8, dtype=torch.uint8, device=dev)
+        count = res[:8 * m].view(torch.int64)
+        mean = res[8 * m:16 * m].view(torch.float64)
+        std = res[16 * m:24 * m].view(torch.float64)
+        mn = res[24 * m:24 * m + vsz * m].view(vdt)
+        mx = res[24 * m + vsz * m:24 * m + 2 * vsz * m].view(vdt)
+        status = res[24 * m + 2 * vsz * m:24 * m + 2 * vsz * m + 4 * n_stream].view(torch.int32) if isolate else None
+        d_off = to_device(offsets, dev, fdt).reshape(-1) if restore else None
+        d_gain = to_device(gains, dev, fdt).reshape(-1) if restore else None
+        row_bytes = n_decode * vsz
+        if on_dev:
+            ranges = _stats_ranges(n_stream, row_bytes, _STATS_GROUP_BYTES)
+        else:
+            ranges = _chunk_ranges(n_stream, row_bytes)
+        full = first_sample == 0 and last_sample == stream_size
+        for a, b, rows in _decode_groups(compressed, h_starts, h_nbytes, on_dev, hint, dev, ranges, stream_size,
+                                         -1 if full else first_sample, -1 if full else last_sample, is_int64,
+                                         status=status):
+            o0, o1 = a * nbins, b * nbins
+            row_stats_device(rows, is_int64, b - a, n_decode, 0 if bin is None else length,
+                             None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b],
+                             None if status is None else status[a:b], count[o0:o1], mn[o0:o1], mx[o0:o1], mean[o0:o1],
+                             std[o0:o1])
+            del rows
+        h = to_host(res)
+    vnp = _TORCH2NP[vdt]
+    out = StreamStats(h[:8 * m].view(np.int64), h[24 * m:24 * m + vsz * m].view(vnp),
+                      h[24 * m + vsz * m:24 * m + 2 * vsz * m].view(vnp), h[8 * m:16 * m].view(np.float64),
+                      h[16 * m:24 * m].view(np.float64))
+    out = StreamStats(*(v.reshape(n_stream, nbins) for v in out))
+    st = h[24 * m + 2 * vsz * m:24 * m + 2 * vsz * m + 4 * n_stream].view(np.int32) if isolate else None
+    return out, st
 
 
 # -------------------------------------------------------------------------------------------------

@@ -200,6 +200,33 @@ int64_t fab_decode_windows_workspace_bytes(int64_t n_stream, int64_t stream_size
                                            int blocksize_hint);
 
 /*
+ * Per-row, per-bin statistics of decoded integer rows (no reference equivalent): the reduction behind
+ * FlacArray.stats().  d_rows: [n_rows][n] int32 (is_int64 = 0) or int64, e.g. the output of fab_decode without
+ * offsets / gains, aligned to its element size.  Each row is cut into bins of `bin` samples (bin = 0: one bin of n
+ * samples; a bin longer than n is one bin; the last bin may be shorter), nbins = ceil(n / bin); a bin longer than
+ * 2^32 - 1 samples is rejected.  Per (row, bin), row-major [n_rows][nbins]:
+ *   d_count  int64   the number of samples;
+ *   d_min    / d_max  the extreme values, in the array's type: int32 / int64, or float32 / float64 when d_offsets and
+ *            d_gains ([n_rows] float32 / float64, as fab_decode takes them; both NULL for integer output) are given --
+ *            then they are the restored extremes, bit-equal to the min / max of the restored samples;
+ *   d_mean / d_std    double: the mean and population standard deviation (ddof = 0).  The sums S = sum x and
+ *            Q = sum x^2 are exact integers; mean = dbl(S) / n and std = sqrt(dbl(n*Q - S^2)) / n with dbl() the
+ *            round-to-nearest-even conversion and plain IEEE double operations after it, so results do not depend on how
+ *            the rows were grouped into calls.  With offsets / gains: mean = off + coeff * mean, std = |coeff| * std, with
+ *            the restore's coeff = 1 / gain in the storage type, widened to double.
+ * d_status ([n_rows] int32, may be NULL): rows with a non-zero status get count 0, NaN mean / std and min / max NaN
+ * (float output) or 0 (integer output).  Bad arguments return error bits (ERROR_ZERO_NSTREAM, ERROR_ZERO_STREAMSIZE,
+ * ERROR_DECODE_SAMPLE_RANGE for a negative or too long bin, ERROR_CONVERT_TYPE for offsets without gains or a
+ * misaligned d_rows, ERROR_ALLOC for NULL arrays) and launch nothing.  Workspace: fab_row_stats_workspace_bytes
+ * (0 when none is needed, -1 for invalid arguments); a caller-supplied workspace that is too small fails with
+ * ERROR_ALLOC.  One or two launches per 65535 rows.
+ */
+int fab_row_stats(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, int64_t bin,
+                  const void* d_offsets, const void* d_gains, const int32_t* d_status, int64_t* d_count, void* d_min,
+                  void* d_max, double* d_mean, double* d_std, void* stream);
+int64_t fab_row_stats_workspace_bytes(int64_t n_rows, int64_t n, int64_t bin, int is_int64);
+
+/*
  * Per-stream population standard deviation of float32 / float64 streams, in the input's type: the device side of
  * `precision` -> quanta (replaces np.std(data, axis=-1) in utils.py:282-296).  One read of the input, moments
  * accumulated in double precision; differs from numpy's pairwise single-precision sum by rounding only.
