@@ -15,7 +15,7 @@ import copy
 import numpy as np
 
 from .compress import array_compress
-from .decompress import array_decompress_slice, array_decompress_windows, array_verify, stats_slice
+from .decompress import array_combine, array_decompress_slice, array_decompress_windows, array_verify, stats_slice
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -376,6 +376,28 @@ class FlacArray:
         if status is not None:
             res = res + (status,)
         return res[0] if len(res) == 1 else res
+
+    def combine(self, weights=None, groups=None, n_groups=None, stream_slice=None, on_error="raise"):
+        """Per-sample weighted sums across the local streams without decompressing them into memory (array_combine):
+        the common mode (groups=None), the common mode of each wafer or band (groups = a label per stream), A - B pair
+        differences (a group per pair, weights +1 / -1) or group averages (weights 1 / size).  `groups` and `weights`
+        have one entry per stream, in the leading shape or flat; -1 leaves a stream out.  `stream_slice` selects samples
+        as stats() does.  Returns float64 (n,) for groups=None, else (n_groups, n): a CUDA tensor when the compressed
+        bytes are on the device, else numpy; each row is the fold acc = +0.0, acc = acc + w_k * float64(x_k) over the
+        group's streams in storage order, with x_k the row to_array returns.  on_error="fill" returns (combined, status)
+        with the int32 status in the leading shape; failed streams add nothing, and streams left out are not examined and
+        report 0 (see verify())."""
+        first, last = 0, self._stream_size
+        if stream_slice is not None:
+            first, last, step = stream_slice.indices(self._stream_size)
+            if step != 1:
+                raise ValueError("Only stream slices with a step size of 1 are supported")
+        starts = np.asarray(self._stream_starts).reshape(self._leading_shape)
+        nbytes = np.asarray(self._stream_nbytes).reshape(self._leading_shape)
+        return array_combine(self._compressed, self._stream_size, starts, nbytes, stream_offsets=self._stream_offsets,
+                             stream_gains=self._stream_gains, weights=weights, groups=groups, n_groups=n_groups,
+                             first_stream_sample=first, last_stream_sample=last, is_int64=self._is_int64,
+                             on_error=on_error)
 
     def to_windows(self, streams, first, last):
         """Decompress many sample windows of local streams in one call.

@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "../../include/flacarray_b200.h"
+#include "fa_combine.h"
 #include "fa_decode.h"
 #include "fa_decode_tile.h"
 #include "fa_encode.h"
@@ -461,6 +462,14 @@ __global__ void __launch_bounds__(kStatsWarps * 32) k_row_stats(const StatsParam
 __global__ void __launch_bounds__(kStatsWarps * 32) k_row_stats_merge(const StatsParams P, int64_t row0) {
     const int64_t b = (int64_t)blockIdx.x * kStatsWarps + (threadIdx.x >> 5);
     if (b < P.nbins) stats_merge_warp(P, row0 + blockIdx.y, b);
+}
+
+// ---- fab_combine_rows (fa_combine.h): grid = (column chunks, segments of one slab); one CTA per (segment, chunk) ----
+template <bool I64, bool FLT>
+__global__ void __launch_bounds__(kCombineThreads) k_combine_rows(const CombineParams P, int64_t s0) {
+    __shared__ CombineRow sh[kCombineThreads];
+    combine_segment_cta<I64, FLT, kCombineThreads>(P, s0 + blockIdx.y,
+                                                   (int64_t)blockIdx.x * (kCombineThreads * kCombineCols), sh);
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
@@ -1411,6 +1420,50 @@ extern "C" int fab_row_stats(fab_ctx* ctx, const void* d_rows, int is_int64, int
             k_row_stats_merge<<<dim3(gm, grid.y), kStatsWarps * 32, 0, st>>>(P, r0);
             ctx->launches++;
         }
+    }
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+// =================================================================================================
+// Per-sample weighted sums across decoded integer rows
+// =================================================================================================
+extern "C" int fab_combine_rows(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n,
+                                const void* d_offsets, const void* d_gains, const int32_t* d_status,
+                                const double* d_weights, const int64_t* d_seg, const int64_t* d_seg_out, int64_t n_seg,
+                                double* d_out, int64_t n_out, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    if (n_rows <= 0 || n_seg <= 0 || n_out <= 0) return ERROR_ZERO_NSTREAM;
+    if (n <= 0) return ERROR_ZERO_STREAMSIZE;
+    if (!d_rows || !d_weights || !d_seg || !d_seg_out || !d_out) {
+        ctx->last_error = "fab_combine_rows: d_rows, d_weights, d_seg, d_seg_out and d_out must not be NULL";
+        return ERROR_ALLOC;
+    }
+    if ((d_offsets == nullptr) != (d_gains == nullptr) || ((uintptr_t)d_rows & (is_int64 ? 7 : 3)) != 0 ||
+        (((uintptr_t)d_weights | (uintptr_t)d_seg | (uintptr_t)d_seg_out | (uintptr_t)d_out) & 7) != 0) {
+        ctx->last_error = "fab_combine_rows: offsets and gains go together, and every array must be aligned to its "
+                          "element size";
+        return ERROR_CONVERT_TYPE;
+    }
+    const int64_t gx = (n + kCombineThreads * kCombineCols - 1) / (kCombineThreads * kCombineCols);
+    if (gx > 0x7FFFFFFFll) return ERROR_ALLOC;
+    CombineParams P{};
+    P.rows = d_rows; P.n_rows = n_rows; P.n = n;
+    P.offsets = d_offsets; P.gains = d_gains; P.status = d_status; P.weights = d_weights;
+    P.seg = (const int64_t*)d_seg; P.seg_out = (const int64_t*)d_seg_out; P.n_seg = n_seg;
+    P.out = d_out; P.n_out = n_out; P.err = ctx->d_err;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool flt = d_offsets != nullptr;
+    for (int64_t s0 = 0; s0 < n_seg; s0 += 65535) {
+        const dim3 grid((unsigned)gx, (unsigned)std::min<int64_t>(65535, n_seg - s0));
+        if (is_int64) {
+            if (flt) k_combine_rows<true, true><<<grid, kCombineThreads, 0, st>>>(P, s0);
+            else k_combine_rows<true, false><<<grid, kCombineThreads, 0, st>>>(P, s0);
+        } else {
+            if (flt) k_combine_rows<false, true><<<grid, kCombineThreads, 0, st>>>(P, s0);
+            else k_combine_rows<false, false><<<grid, kCombineThreads, 0, st>>>(P, s0);
+        }
+        ctx->launches++;
     }
     FAB_CUDA(ctx, cudaGetLastError());
     return 0;

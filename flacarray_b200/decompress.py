@@ -2,12 +2,13 @@
 /root/reference/src/flacarray/decompress.py:18-205 (keep mask, sample window, single-stream
 flattening rules, error messages), plus on_error="fill" (per-stream fault isolation);
 array_decompress_windows: many per-stream sample windows in one decode; array_verify: check streams without
-decoding them out; array_stats: per-stream and per-bin statistics without decoding the array out.  The FLAC decode, the
-int->float restore and the statistics run on the device."""
+decoding them out; array_stats: per-stream and per-bin statistics without decoding the array out; array_combine:
+per-sample weighted sums across streams without decoding the array out.  The FLAC decode, the int->float restore, the
+statistics and the sums run on the device."""
 import numpy as np
 
-from .libflacarray import (StreamStats, check_bin, check_on_error, decode_flac, decode_flac_float, decode_windows,
-                           is_torch, stats_flac, verify_flac)
+from .libflacarray import (StreamStats, check_bin, check_combine_args, check_on_error, combine_flac, decode_flac,
+                           decode_flac_float, decode_windows, is_torch, stats_flac, verify_flac)
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -266,3 +267,70 @@ def array_stats(
                                    stream_gains=stream_gains, keep=keep, first_stream_sample=first_stream_sample,
                                    last_stream_sample=last_stream_sample, bin=bin, is_int64=is_int64, on_error=on_error)
     return (stats, status) if status is not None else stats
+
+
+@function_timer
+def array_combine(
+    compressed,
+    stream_size,
+    stream_starts,
+    stream_nbytes,
+    stream_offsets=None,
+    stream_gains=None,
+    weights=None,
+    groups=None,
+    n_groups=None,
+    first_stream_sample=None,
+    last_stream_sample=None,
+    is_int64=False,
+    on_error="raise",
+):
+    """Per-sample weighted sums across streams (common modes, pair differences, group averages) without materialising
+    the decoded array.
+
+    `groups` gives every stream the output row it adds into: an integer array with one entry per stream, shaped like
+    stream_starts or flat in C order; -1 leaves a stream out (it is neither copied nor decoded).  None puts every stream
+    in one group and the result is 1-D, (n,); otherwise it is (n_groups, n), n_groups defaulting to groups.max() + 1 (give
+    it so that callers without streams in some group get results of the same shape).  `weights`: one float64 per stream
+    (default 1.0), used as given.  Samples [first_stream_sample, last_stream_sample) of every stream are combined, and
+    offsets and gains (both or neither) restore floats as array_decompress does.
+
+    With x_k the row array_decompress returns for stream k, each output row g is the fold over the streams k of group g
+    in storage order, in plain IEEE double (multiply and add each rounded, no FMA):
+        acc = +0.0;  acc = acc + w_k * float64(x_k)
+    float32 widens exactly and int64 converts with round to nearest even, so
+    `for k: acc += w[k] * x[k].astype(np.float64)` in numpy gives the same bits, whatever the residency or the grouping
+    of streams into device calls.
+
+    The result is float64: a CUDA tensor when the compressed bytes are on the device, else numpy.  on_error="fill"
+    returns (combined, status) with the int32 status shaped like stream_starts: a stream that cannot be decoded adds
+    nothing and reports its ERROR_DECODE_* bit.  Streams with group -1 are not examined and report 0 (array_verify checks
+    every stream).  A weights or groups size that is not the stream count, non-integer or boolean groups, a group below -1
+    or at least n_groups, n_groups < 0, an empty sample range and an unknown on_error raise ValueError before any device
+    is used.
+    """
+    isolate = check_on_error(on_error)
+    if (stream_offsets is None) != (stream_gains is None):
+        raise RuntimeError("Offsets and gains must be given together")
+    first = 0 if first_stream_sample is None else int(first_stream_sample)
+    last = int(stream_size) if last_stream_sample is None else int(last_stream_sample)
+    if first < 0 or last > stream_size:
+        raise ValueError(f"sample range [{first}, {last}) lies outside the stream of {stream_size} samples")
+    if last <= first:
+        raise ValueError(f"sample range [{first}, {last}) is empty")
+    single = not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts))
+    if single:
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+    lead = tuple(stream_starts.shape)
+    n_stream = int(np.prod(lead))
+    w, g, n_out = check_combine_args(n_stream, weights, groups, n_groups)
+    offsets = None if stream_offsets is None else _host(stream_offsets)
+    gains = None if stream_gains is None else _host(stream_gains)
+    out, status = combine_flac(compressed, _host(stream_starts), _host(stream_nbytes), stream_size, first, last, w, g,
+                               n_out, offsets, gains, is_int64, isolate)
+    if groups is None:
+        out = out.reshape(last - first)
+    if isolate:
+        return out, status.reshape(lead)
+    return out

@@ -1093,6 +1093,130 @@ def stats_flac(compressed, starts, nbytes, stream_size, first_sample, last_sampl
 
 
 # -------------------------------------------------------------------------------------------------
+# Weighted sums across streams: per-sample sums of weighted streams per group, folded from the decoded integers on the
+# device (fab_combine_rows; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+
+def check_combine_args(n_stream, weights, groups, n_groups):
+    """The weights (float64, default 1), output row of every stream (int64, -1 = left out; None = all in row 0) and the
+    number of output rows of a combine over n_stream streams, flat.  Raises ValueError for a size that is not n_stream,
+    non-integer or boolean groups, a group below -1 or at least n_groups, and n_groups < 0."""
+    def host(a):
+        return a.cpu().numpy() if is_torch(a) else np.asarray(a)
+
+    if weights is None:
+        w = np.ones(n_stream)
+    else:
+        w = host(weights)
+        if w.dtype == np.bool_ or w.dtype.kind not in "iuf":
+            raise ValueError(f"weights must be real numbers, not {w.dtype}")
+        w = w.astype(np.float64).reshape(-1)
+        if w.size != n_stream:
+            raise ValueError(f"weights has {w.size} entries for {n_stream} streams")
+    if groups is None:
+        if n_groups is not None:
+            raise ValueError("n_groups needs groups")
+        return w, np.zeros(n_stream, np.int64), 1
+    g = host(groups)
+    if g.dtype.kind not in "iu":
+        raise ValueError(f"groups must be integers, not {g.dtype}")
+    g = g.astype(np.int64).reshape(-1)
+    if g.size != n_stream:
+        raise ValueError(f"groups has {g.size} entries for {n_stream} streams")
+    if n_groups is None:
+        n_groups = int(g.max()) + 1 if g.size else 0
+    elif isinstance(n_groups, bool) or not isinstance(n_groups, (int, np.integer)) or int(n_groups) < 0:
+        raise ValueError(f"n_groups must be an integer >= 0, not {n_groups!r}")
+    n_groups = int(n_groups)
+    if g.size and (int(g.min()) < -1 or int(g.max()) >= n_groups):
+        raise ValueError(f"groups must lie in [-1, {n_groups}), found [{int(g.min())}, {int(g.max())}]")
+    return w, g, n_groups
+
+
+def combine_device(rows, is_int64, n_rows, n, offsets, gains, status, weights, seg, seg_out, n_seg, out, n_out):
+    """Device-level fab_combine_rows over CUDA tensors."""
+    dev = rows.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_combine_rows(ctx.handle, _ptr(rows), 1 if is_int64 else 0, n_rows, n, _ptr(offsets),
+                                         _ptr(gains), _ptr(status), _ptr(weights), _ptr(seg), _ptr(seg_out), n_seg,
+                                         _ptr(out), n_out, st)
+        if rc != 0:
+            _check(rc, ctx, st, "Combining")
+
+
+def _segments(labels, ranges):
+    """Segments of every decode group: consecutive rows of `labels` (sorted) with the same label.  Returns the
+    concatenated row bounds (rebased to each group, n_seg + 1 per group), output rows, and each group's offsets into
+    them."""
+    bounds, outs, where = [], [], []
+    nb = no = 0
+    for a, b in ranges:
+        lab = labels[a:b]
+        cut = np.flatnonzero(lab[1:] != lab[:-1]) + 1
+        bd = np.concatenate([[0], cut, [b - a]]).astype(np.int64)
+        bounds.append(bd)
+        outs.append(lab[bd[:-1]])
+        where.append((nb, no, bd.size - 1))
+        nb += bd.size
+        no += bd.size - 1
+    return np.concatenate(bounds), np.concatenate(outs).astype(np.int64), where
+
+
+def combine_flac(compressed, starts, nbytes, stream_size, first_sample, last_sample, weights, groups, n_groups,
+                 offsets=None, gains=None, is_int64=False, isolate=False):
+    """Per-sample weighted sums of samples [first_sample, last_sample) over the streams of each group, without storing
+    the decoded array: the streams with groups >= 0 are decoded to integers on the device in (group, storage index)
+    order, group by group of streams, and fab_combine_rows folds each group's rows into its output row.  `weights`,
+    `groups` and `n_groups` as check_combine_args returns them.  Returns (out [n_groups, n] float64: a CUDA tensor for
+    device bytes, else numpy; status): status is the int32 numpy per-stream status with `isolate` (0 for streams left
+    out), else None and a failed decode raises."""
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
+    n_stream = h_starts.size
+    n_decode = last_sample - first_sample
+    sel = np.flatnonzero(groups >= 0)
+    order = sel[np.argsort(groups[sel], kind="stable")]      # by group, storage order within a group
+    m = order.size
+    dev = compressed.device if on_dev else _device()
+    fdt = torch.float64 if is_int64 else torch.float32
+    restore = offsets is not None
+    st_all = np.zeros(n_stream, np.int32) if isolate else None
+    with torch.cuda.device(dev):
+        out = torch.zeros((n_groups, n_decode), dtype=torch.float64, device=dev)
+        if m and n_groups:
+            row_bytes = n_decode * (8 if is_int64 else 4)
+            if on_dev:
+                ranges = _stats_ranges(m, row_bytes, _STATS_GROUP_BYTES)
+            else:
+                ranges = _chunk_ranges(m, row_bytes)
+            labels = groups[order]
+            bounds, outs, where = _segments(labels, ranges)
+            d_w = to_device(weights[order], dev, torch.float64)
+            d_bounds = to_device(bounds, dev, torch.int64)
+            d_outs = to_device(outs, dev, torch.int64)
+            d_off = to_device(np.asarray(offsets).reshape(-1)[order], dev, fdt) if restore else None
+            d_gain = to_device(np.asarray(gains).reshape(-1)[order], dev, fdt) if restore else None
+            status = _status_tensor(dev, m) if isolate else None
+            full = first_sample == 0 and last_sample == stream_size
+            for (a, b, rows), (nb, no, n_seg) in zip(
+                    _decode_groups(compressed, h_starts[order], h_nbytes[order], on_dev, hint, dev, ranges, stream_size,
+                                   -1 if full else first_sample, -1 if full else last_sample, is_int64, status=status),
+                    where):
+                combine_device(rows, is_int64, b - a, n_decode, None if d_off is None else d_off[a:b],
+                               None if d_gain is None else d_gain[a:b], None if status is None else status[a:b],
+                               d_w[a:b], d_bounds[nb:nb + n_seg + 1], d_outs[no:no + n_seg], n_seg, out, n_groups)
+                del rows
+            ctx = _lib.context(dev)
+            _check(0, ctx, _stream(dev), "Combining")
+            if isolate:
+                st_all[order] = to_host(status)
+        if not on_dev:
+            out = to_host(out)
+    return out, st_all
+
+
+# -------------------------------------------------------------------------------------------------
 # Per-stream sample windows (fab_decode_windows; no reference equivalent)
 # -------------------------------------------------------------------------------------------------
 

@@ -227,6 +227,32 @@ int fab_row_stats(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows
 int64_t fab_row_stats_workspace_bytes(int64_t n_rows, int64_t n, int64_t bin, int is_int64);
 
 /*
+ * Per-sample weighted sums across decoded integer rows (no reference equivalent): the reduction behind
+ * FlacArray.combine() (common modes, pair differences, group averages).  d_rows: [n_rows][n] int32 (is_int64 = 0) or
+ * int64, e.g. the output of fab_decode without offsets / gains, aligned to its element size.  Rows come as n_seg
+ * segments: segment s is rows [d_seg[s], d_seg[s + 1]) and adds into row d_seg_out[s] of d_out ([n_out][n] double).
+ * For every sample i of segment s, in plain IEEE double (multiply and add each rounded, never an FMA):
+ *     acc = d_out[d_seg_out[s]][i]
+ *     for k = d_seg[s] .. d_seg[s + 1] - 1 with d_status[k] == 0:   acc = acc + d_weights[k] * x_k[i]
+ *     d_out[d_seg_out[s]][i] = acc
+ * x_k[i] is the integer (int64 converts with round to nearest even) or, when d_offsets and d_gains ([n_rows] float32 /
+ * float64, as fab_decode takes them; both NULL for integer rows) are given, the value fab_decode's restore produces in
+ * the array's type, widened to double.  So a zero-filled d_out gives the fold +0.0 + w x + ... in row order, and a
+ * segment continues from what an earlier call stored in its output row: a group of rows split over several calls gives
+ * the same bits as one call.  d_weights: [n_rows] double.  d_status ([n_rows] int32, may be NULL): rows with a non-zero
+ * status are skipped.  d_seg ([n_seg + 1]) and d_seg_out ([n_seg]) are device int64 and must satisfy
+ * 0 <= d_seg[s] <= d_seg[s + 1] <= n_rows, 0 <= d_seg_out[s] < n_out and d_seg_out strictly increasing, so that no two
+ * segments write the same output row; they are checked on the device, and a record that breaks a rule sets
+ * ERROR_DECODE_SAMPLE_RANGE in the mask fab_finish returns and its segment writes nothing (the output of such a call
+ * is not meaningful).  Bad arguments return error bits (ERROR_ZERO_NSTREAM for n_rows, n_seg or n_out <= 0,
+ * ERROR_ZERO_STREAMSIZE for n <= 0, ERROR_ALLOC for NULL arrays, ERROR_CONVERT_TYPE for offsets without gains or a
+ * misaligned array) and launch nothing.  No workspace.  One launch per 65535 segments.
+ */
+int fab_combine_rows(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, const void* d_offsets,
+                     const void* d_gains, const int32_t* d_status, const double* d_weights, const int64_t* d_seg,
+                     const int64_t* d_seg_out, int64_t n_seg, double* d_out, int64_t n_out, void* stream);
+
+/*
  * Per-stream population standard deviation of float32 / float64 streams, in the input's type: the device side of
  * `precision` -> quanta (replaces np.std(data, axis=-1) in utils.py:282-296).  One read of the input, moments
  * accumulated in double precision; differs from numpy's pairwise single-precision sum by rounding only.
