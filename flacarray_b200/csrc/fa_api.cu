@@ -272,64 +272,11 @@ __global__ void __launch_bounds__(256) k_restore(const I* in, int64_t n_per_stre
 }
 
 // ---- decode stages ---------------------------------------------------------------------------------
-// One warp per stream.  Lane 0 walks the (short) metadata chain; the frame-size table of streams written
-// by this library is then turned into frame offsets by the whole warp (coalesced 3-byte reads, warp scan)
-// instead of a serial loop per stream -- same results as meta_body (fa_decode.h), which remains the
-// reference for the rules.
+// one warp per stream: metadata + frame offsets (meta_warp)
 __global__ void __launch_bounds__(128) k_dec_meta(const DecParams P) {
     const int64_t k = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
     if (k >= P.n_sel) return;
-    const int ln = threadIdx.x & 31;
-    const uint8_t* buf = P.bytes + P.starts[k];
-    const long long nb = P.nbytes[k];
-    StreamMeta m;
-    if (ln == 0) {
-        parse_stream_meta(buf, nb, m);
-        P.meta[k] = m;
-    }
-    m.first_frame = __shfl_sync(0xffffffffu, m.first_frame, 0);
-    m.table_off = __shfl_sync(0xffffffffu, m.table_off, 0);
-    m.blocksize = __shfl_sync(0xffffffffu, m.blocksize, 0);
-    m.channels = __shfl_sync(0xffffffffu, m.channels, 0);
-    m.bps = __shfl_sync(0xffffffffu, m.bps, 0);
-    m.table_entries = __shfl_sync(0xffffffffu, m.table_entries, 0);
-    long long* fo = P.frame_off + k * (int64_t)(P.nframes_cap + 1);
-    int flag = 0;
-    if (m.first_frame < 0 || m.channels != P.nch || m.bps != 32) {
-        if (ln == 0) stream_failed(P, k, kErrDecodeInit);
-        flag = 4;  // undecodable
-    } else if (m.blocksize <= 0) {
-        flag = 1;  // variable blocksize: sequential walker
-    } else {
-        const int64_t nf = frames_in_stream(P.stream_size, m.blocksize);
-        if (nf > P.nframes_cap) {
-            flag = 1;
-        } else if (m.table_off >= 0 && m.table_entries == nf) {
-            const uint8_t* tb = buf + m.table_off;
-            long long pos = m.first_frame;      // offset of frame j0 (warp-uniform carry)
-            for (int64_t j0 = 0; j0 < nf; j0 += 32) {
-                const int64_t j = j0 + ln;
-                long long len = 0;
-                if (j < nf) len = ((long long)tb[3 * j] << 16) | ((long long)tb[3 * j + 1] << 8) | tb[3 * j + 2];
-                long long inc = len;
-                for (int d = 1; d < 32; d <<= 1) {
-                    long long v = __shfl_up_sync(0xffffffffu, inc, d);
-                    if (ln >= d) inc += v;
-                }
-                if (j < nf) fo[j] = pos + inc - len;
-                pos += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (ln == 0) fo[nf] = pos;
-            if (pos != nb) flag = 1;
-        } else {
-            for (int64_t j = ln; j < nf; j += 32) fo[j] = -1;
-            if (ln == 0) fo[nf] = nb;
-        }
-    }
-    if (ln == 0) {
-        P.stream_flag[k] = flag;
-        if (P.status && flag != 4) P.status[k] = 0;
-    }
+    meta_warp(P, k);
 }
 
 constexpr int kSyncThreads = 256;
@@ -347,20 +294,7 @@ constexpr int kDecThreads = 128;
 template <bool WIN>
 __global__ void __launch_bounds__(kDecThreads) k_dec_frames(const DecParams P, const WinParams W, int64_t nwin) {
     // one thread per work item (stream, frame index inside the sample window), see resolve_item
-    int64_t idx = (int64_t)blockIdx.x * kDecThreads + threadIdx.x;
-    const WorkItem it = resolve_item<WIN>(P, W, nwin, idx);
-    const int64_t k = it.k;
-    if (k < 0) return;
-    if (P.stream_flag[k] != 0) return;
-    int bs = P.meta[k].blocksize;
-    int64_t j0 = it.first / bs, j1 = (it.first + it.n - 1) / bs;
-    if (j1 - j0 + 1 > it.nwin) {  // blocksize differs from the host's hint: leave the stream to the walker
-        if (it.jrel == 0) atomicOr(&P.stream_flag[k], 1);
-        return;
-    }
-    int64_t j = j0 + it.jrel;
-    if (j > j1) return;
-    frame_body(P, k, j, it.first, it.n, it.out);
+    frames_item<WIN>(P, W, nwin, (int64_t)blockIdx.x * kDecThreads + threadIdx.x);
 }
 
 // throughput path: one warp = 32 (stream, frame) items, see fa_decode_tile.h.
@@ -442,14 +376,10 @@ __global__ void k_dec_walker_iso(const DecParams P) {
 }
 
 // fab_decode_isolated: overwrite the whole output row of every stream whose status is not 0 with `fill` (0 for integer
-// output, a quiet NaN for float output), after the walker and the restore.  grid = (x, streams of one slab); W is the
-// output element (uint32_t for int32 / float32, unsigned long long for int64 / float64).
+// output, a quiet NaN for float output), after the walker and the restore.  grid = (x, streams of one slab).
 template <typename W>
 __global__ void __launch_bounds__(256) k_dec_fill_failed(const int* __restrict__ status, W* out, int64_t n_per_stream, W fill) {
-    const int64_t s = blockIdx.y;
-    if (status[s] == 0) return;
-    W* o = out + s * n_per_stream;
-    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n_per_stream; i += (int64_t)gridDim.x * 256) o[i] = fill;
+    fill_failed<W>(status, out, n_per_stream, fill, blockIdx.y, (int64_t)blockIdx.x * 256 + threadIdx.x, (int64_t)gridDim.x * 256);
 }
 
 // ---- fab_row_stats (fa_stats.h): grid = (pieces / kStatsWarps, rows of one slab); one warp per piece / per bin -------
@@ -473,54 +403,18 @@ __global__ void __launch_bounds__(kCombineThreads) k_combine_rows(const CombineP
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
-// Window records -> item space: a record that names a stream slot outside [0, n_sel) or a range outside the stream
-// sets ERROR_DECODE_SAMPLE_RANGE and gets no items; W.item0 = exclusive prefix of the frame counts (hinted blocksize),
-// W.item0[n_win] = the number of items.  One CTA, chunks of 1024 windows with a running carry.
+// window records -> item space (win_prep_cta), one CTA
 constexpr int kWinScanThreads = 1024;
 __global__ void __launch_bounds__(kWinScanThreads) k_win_prep(const WinParams W, int64_t n_sel, int64_t stream_size, int* err) {
     __shared__ long long wpre[kWinScanThreads / 32];
     __shared__ long long ctot;
-    long long* item0 = const_cast<long long*>(W.item0);
-    const int ln = threadIdx.x & 31, wp = threadIdx.x >> 5;
-    long long carry = 0;
-    for (int64_t w0 = 0; w0 < W.n_win; w0 += kWinScanThreads) {
-        const int64_t w = w0 + threadIdx.x;
-        long long cnt = 0;
-        if (w < W.n_win) {
-            if (win_valid(W, w, n_sel, stream_size)) cnt = frames_in_window(W.first[w], W.last[w] - W.first[w], W.bsh);
-            else atom_or_global(err, kErrDecodeSampleRange);
-        }
-        long long inc = cnt;       // inclusive scan inside the warp, then over the warps' totals
-        for (int d = 1; d < 32; d <<= 1) {
-            long long v = __shfl_up_sync(0xffffffffu, inc, d);
-            if (ln >= d) inc += v;
-        }
-        if (ln == 31) wpre[wp] = inc;
-        __syncthreads();
-        if (wp == 0) {
-            const long long t = wpre[ln];
-            long long ti = t;
-            for (int d = 1; d < 32; d <<= 1) {
-                long long v = __shfl_up_sync(0xffffffffu, ti, d);
-                if (ln >= d) ti += v;
-            }
-            wpre[ln] = ti - t;
-            if (ln == 31) ctot = ti;
-        }
-        __syncthreads();
-        if (w < W.n_win) item0[w] = carry + wpre[wp] + inc - cnt;
-        carry += ctot;
-        __syncthreads();           // (wpre / ctot are rewritten by the next chunk)
-    }
-    if (threadIdx.x == 0) item0[W.n_win] = carry;
+    win_prep_cta<kWinScanThreads>(W, n_sel, stream_size, err, wpre, &ctot);
 }
 
-// fab_decode_windows: the frames of the windows, one thread per work item (walker-decoded streams: per window)
+// fab_decode_windows: the walker, one thread per window (walker_win)
 __global__ void k_dec_walker_win(const DecParams P, const WinParams W) {
     const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (w >= W.n_win || !win_valid(W, w, P.n_sel, P.stream_size)) return;
-    const long long first = W.first[w], n = W.last[w] - first;
-    if (n > 0) walker_body(P, W.stream[w], first, n, W.out[w]);
+    if (w < W.n_win) walker_win(P, W, w);
 }
 
 // Windowed int -> float, one warp per work item over the item's samples.  F64: every sample (the decoders wrote int64
@@ -1068,17 +962,9 @@ static DecWorkspace dec_workspace(int64_t n_stream, int nframes_cap) {
     W.total = W.meta_b + W.fo_b + W.flag_b + W.fflag_b + 256;
     return W;
 }
-static int dec_frames_cap(int64_t stream_size, int blocksize_hint, int* cap) {
-    int bsh = blocksize_hint > 0 ? blocksize_hint : 4096;
-    if (bsh < 16) bsh = 16;
-    int64_t cap64 = (stream_size + bsh - 1) / bsh;
-    if (cap64 > (1 << 26)) return ERROR_ALLOC;
-    *cap = (int)cap64;
-    return 0;
-}
 extern "C" int64_t fab_decode_workspace_bytes(int64_t n_stream, int64_t stream_size, int blocksize_hint) {
-    int cap = 0;
-    if (n_stream <= 0 || stream_size <= 0 || dec_frames_cap(stream_size, blocksize_hint, &cap)) return 0;
+    int bsh = 0, cap = 0;
+    if (n_stream <= 0 || stream_size <= 0 || dec_frames_cap(stream_size, blocksize_hint, &bsh, &cap)) return 0;
     return (int64_t)dec_workspace(n_stream, cap).total;
 }
 
@@ -1152,9 +1038,8 @@ static int dec_uniform(fab_ctx* ctx, const unsigned char* d_bytes, const int64_t
     }
     cudaStream_t st = (cudaStream_t)stream;
     const int nch = is_int64 ? 2 : 1;
-    int nframes_cap = 0;
-    if (dec_frames_cap(stream_size, blocksize_hint, &nframes_cap)) return ERROR_ALLOC;
-    const int bsh = std::max(16, blocksize_hint > 0 ? blocksize_hint : 4096);
+    int bsh = 0, nframes_cap = 0;
+    if (dec_frames_cap(stream_size, blocksize_hint, &bsh, &nframes_cap)) return ERROR_ALLOC;
 
     const DecWorkspace W = dec_workspace(n_stream, nframes_cap);
     const size_t meta_b = W.meta_b, fo_b = W.fo_b, flag_b = W.flag_b, fflag_b = W.fflag_b;
@@ -1278,8 +1163,9 @@ extern "C" int fab_verify(fab_ctx* ctx, const unsigned char* d_bytes, const int6
 static size_t win_item0_bytes(int64_t n_win) { return align256((size_t)(n_win + 1) * 8); }
 extern "C" int64_t fab_decode_windows_workspace_bytes(int64_t n_stream, int64_t stream_size, int64_t n_win,
                                                       int64_t total_items, int blocksize_hint) {
-    int cap = 0;
-    if (n_stream <= 0 || stream_size <= 0 || n_win < 0 || total_items < 0 || dec_frames_cap(stream_size, blocksize_hint, &cap))
+    int bsh = 0, cap = 0;
+    if (n_stream <= 0 || stream_size <= 0 || n_win < 0 || total_items < 0 ||
+        dec_frames_cap(stream_size, blocksize_hint, &bsh, &cap))
         return 0;
     return (int64_t)(dec_workspace(n_stream, cap).total + win_item0_bytes(n_win));
 }
@@ -1296,9 +1182,8 @@ extern "C" int fab_decode_windows(fab_ctx* ctx, const unsigned char* d_bytes, co
     if (stream_size <= 0) return ERROR_ZERO_STREAMSIZE;
     cudaStream_t st = (cudaStream_t)stream;
     const int nch = is_int64 ? 2 : 1;
-    int nframes_cap = 0;
-    if (dec_frames_cap(stream_size, blocksize_hint, &nframes_cap)) return ERROR_ALLOC;
-    const int bsh = std::max(16, blocksize_hint > 0 ? blocksize_hint : 4096);
+    int bsh = 0, nframes_cap = 0;
+    if (dec_frames_cap(stream_size, blocksize_hint, &bsh, &nframes_cap)) return ERROR_ALLOC;
 
     const DecWorkspace DW = dec_workspace(n_stream, nframes_cap);
     unsigned char* scr;
@@ -1358,22 +1243,6 @@ extern "C" int fab_decode_windows(fab_ctx* ctx, const unsigned char* d_bytes, co
 // =================================================================================================
 // Per-row, per-bin statistics of decoded integer rows
 // =================================================================================================
-// bin == 0: one bin per row.  Returns 0 and fills *P's geometry, or the error bits of bad arguments.
-static int stats_geometry(int64_t n_rows, int64_t n, int64_t bin, int is_int64, StatsParams* P) {
-    if (n_rows <= 0) return ERROR_ZERO_NSTREAM;
-    if (n <= 0) return ERROR_ZERO_STREAMSIZE;
-    if (bin < 0) return ERROR_DECODE_SAMPLE_RANGE;
-    const int64_t len = bin == 0 ? n : std::min(bin, n);
-    if (len > kStatsMaxBin) return ERROR_DECODE_SAMPLE_RANGE;
-    P->is_int64 = is_int64 ? 1 : 0;
-    P->n_rows = n_rows; P->n = n; P->bin = len;
-    P->nbins = (n + len - 1) / len;
-    P->piece = kStatsPieceBytes / (is_int64 ? 8 : 4);
-    P->ppb = (len + P->piece - 1) / P->piece;
-    if ((P->nbins * P->ppb + kStatsWarps - 1) / kStatsWarps > 0x7FFFFFFFll) return ERROR_ALLOC;
-    return 0;
-}
-
 static size_t stats_workspace(const StatsParams& P) {
     return P.ppb > 1 ? align256((size_t)P.n_rows * (size_t)P.nbins * (size_t)P.ppb * sizeof(StatPart)) : 0;
 }
@@ -1858,8 +1727,7 @@ int host_decode_pipelined(fab_ctx* ctx, HostPipe& hp, const unsigned char* bytes
                         d_aux[2] = {{hp.dev_aux[0]}, {hp.dev_aux[1]}};
     std::thread drainer;                 // copies chunk c-2 out of pinned memory while chunk c is staged
     std::atomic<int> drain_err{0};
-    int bs_hint = 0;
-    if (nbytes[0] >= 12 && memcmp(bytes + starts[0], "fLaC", 4) == 0) bs_hint = (bytes[starts[0] + 8] << 8) | bytes[starts[0] + 9];
+    const int bs_hint = stream_blocksize_hint(bytes + starts[0], nbytes[0]);
     std::vector<int64_t> rel[2];
     int rc = 0;
     for (int64_t c = 0; c < nchunk + 2; ++c) {
@@ -1995,8 +1863,7 @@ int host_decode(const unsigned char* bytes, const int64_t* starts, const int64_t
         cudaMemcpy(d_starts, rel.data(), (size_t)n_stream * 8, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(d_nb, nbytes, (size_t)n_stream * 8, cudaMemcpyHostToDevice) != cudaSuccess)
         return FAB_ERROR_CUDA;
-    int bs_hint = 0;
-    if (nbytes[0] >= 12 && memcmp(bytes + starts[0], "fLaC", 4) == 0) bs_hint = (bytes[starts[0] + 8] << 8) | bytes[starts[0] + 9];
+    const int bs_hint = stream_blocksize_hint(bytes + starts[0], nbytes[0]);
     int rc = fab_decode(ctx, (const unsigned char*)d_b.p, d_starts, d_nb, n_stream, stream_size, is_int64, first, last,
                         d_o.p, nullptr, nullptr, mx, bs_hint, nullptr);
     if (rc) return rc;

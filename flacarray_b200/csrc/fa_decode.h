@@ -243,7 +243,7 @@ FA_D int64_t decode_frame_general(const uint8_t* p, const uint8_t* end, const Cr
 }  // namespace fa
 
 // =================================================================================================
-// Kernel bodies (thin __global__ wrappers in fa_kernels.cu map thread indices onto these).
+// Kernel bodies (thin __global__ wrappers in fa_api.cu map thread indices onto these).
 // =================================================================================================
 namespace fa {
 
@@ -277,6 +277,25 @@ FA_D void stream_failed(const DecParams& P, int64_t k, int bit) {
 // number of frames / size of frame j for a fixed-blocksize stream
 FA_D int64_t frames_in_stream(int64_t stream_size, int bs) { return (stream_size + bs - 1) / bs; }
 
+// ---- host-side sizing of a decode call ------------------------------------------------------------------------------
+// The blocksize hint: STREAMINFO's min blocksize of the call's first stream, 0 when its bytes do not start with one.
+inline int stream_blocksize_hint(const uint8_t* s, int64_t nbytes) {
+    return nbytes >= 12 && memcmp(s, "fLaC", 4) == 0 ? (s[8] << 8) | s[9] : 0;
+}
+
+// The hinted blocksize *bsh (4096 without a hint, at least 16: the smallest legal blocksize) and the frame-table rows of a
+// stream slot *cap.  The item space of a call has the frames of the hinted blocksize; a stream whose blocksize needs more
+// frames than that goes to the walker.  Returns kErrAlloc for a table of more than 2^26 frames per stream.
+inline int dec_frames_cap(int64_t stream_size, int blocksize_hint, int* bsh, int* cap) {
+    int b = blocksize_hint > 0 ? blocksize_hint : 4096;
+    if (b < 16) b = 16;
+    const int64_t c = (stream_size + b - 1) / b;
+    if (c > (1 << 26)) return kErrAlloc;
+    *bsh = b;
+    *cap = (int)c;
+    return 0;
+}
+
 // Per-window sample ranges (fab_decode_windows).  Window w reads samples [first[w], last[w]) of stream slot stream[w] and
 // writes them from output element out[w] on.  Its work items are the frames the window overlaps for the hinted
 // blocksize `bsh`; item0 is the exclusive prefix of those counts, so an item finds its window by a binary search and
@@ -299,6 +318,47 @@ FA_D bool win_valid(const WinParams& W, int64_t w, int64_t n_sel, int64_t stream
 // frames of [first, first + n) for blocksize bs (0 for an empty window)
 FA_D int64_t frames_in_window(int64_t first, int64_t n, int64_t bs) {
     return n > 0 ? (first + n - 1) / bs - first / bs + 1 : 0;
+}
+
+// Window records -> item space (k_win_prep), one CTA of NT threads: a record that names a stream slot outside [0, n_sel)
+// or a range outside the stream sets ERROR_DECODE_SAMPLE_RANGE and gets no items; W.item0 = exclusive prefix of the frame
+// counts (hinted blocksize), W.item0[n_win] = the number of items.  Chunks of NT windows with a running carry.
+// wpre[NT / 32], ctot: shared.
+template <int NT>
+FA_D void win_prep_cta(const WinParams& W, int64_t n_sel, int64_t stream_size, int* err, long long* wpre, long long* ctot) {
+    long long* item0 = const_cast<long long*>(W.item0);
+    const int ln = lane(), wp = warp();
+    long long carry = 0;
+    for (int64_t w0 = 0; w0 < W.n_win; w0 += NT) {
+        const int64_t w = w0 + tid();
+        long long cnt = 0;
+        if (w < W.n_win) {
+            if (win_valid(W, w, n_sel, stream_size)) cnt = frames_in_window(W.first[w], W.last[w] - W.first[w], W.bsh);
+            else atom_or_global(err, kErrDecodeSampleRange);
+        }
+        long long inc = cnt;       // inclusive scan inside the warp, then over the warps' totals
+        for (int d = 1; d < 32; d <<= 1) {
+            long long v = (long long)shfl_up64((unsigned long long)inc, d);
+            if (ln >= d) inc += v;
+        }
+        if (ln == 31) wpre[wp] = inc;
+        sync();
+        if (wp == 0) {
+            const long long t = ln < NT / 32 ? wpre[ln] : 0;
+            long long ti = t;
+            for (int d = 1; d < 32; d <<= 1) {
+                long long v = (long long)shfl_up64((unsigned long long)ti, d);
+                if (ln >= d) ti += v;
+            }
+            if (ln < NT / 32) wpre[ln] = ti - t;
+            if (ln == 31) *ctot = ti;
+        }
+        sync();
+        if (w < W.n_win) item0[w] = carry + wpre[wp] + inc - cnt;
+        carry += *ctot;
+        sync();                    // (wpre / ctot are rewritten by the next chunk)
+    }
+    if (tid() == 0) item0[W.n_win] = carry;
 }
 
 // One work item of the decoder's index space: frame `jrel` (counted from the window's first frame) of the window
@@ -374,6 +434,63 @@ FA_D void meta_body(const DecParams& P, int64_t k) {
         }
     }
     P.stream_flag[k] = flag;
+}
+
+// ---- stage 1 as the product runs it (k_dec_meta): one warp per stream.  Lane 0 walks the (short) metadata chain; the
+// frame-size table of streams written by this library is then turned into frame offsets by the whole warp (coalesced
+// 3-byte reads, warp scan) instead of a serial loop per stream.  Same results as meta_body, the reference for the rules.
+FA_D void meta_warp(const DecParams& P, int64_t k) {
+    const int ln = lane();
+    const uint8_t* buf = P.bytes + P.starts[k];
+    const long long nb = P.nbytes[k];
+    StreamMeta m;
+    if (ln == 0) {
+        parse_stream_meta(buf, nb, m);
+        P.meta[k] = m;
+    }
+    m.first_frame = (int64_t)shfl64((unsigned long long)m.first_frame, 0);
+    m.table_off = (int64_t)shfl64((unsigned long long)m.table_off, 0);
+    m.blocksize = (int32_t)shfl((uint32_t)m.blocksize, 0);
+    m.channels = (int32_t)shfl((uint32_t)m.channels, 0);
+    m.bps = (int32_t)shfl((uint32_t)m.bps, 0);
+    m.table_entries = (int32_t)shfl((uint32_t)m.table_entries, 0);
+    long long* fo = P.frame_off + k * (int64_t)(P.nframes_cap + 1);
+    int flag = 0;
+    if (m.first_frame < 0 || m.channels != P.nch || m.bps != 32) {
+        if (ln == 0) stream_failed(P, k, kErrDecodeInit);
+        flag = 4;  // undecodable
+    } else if (m.blocksize <= 0) {
+        flag = 1;  // variable blocksize: sequential walker
+    } else {
+        const int64_t nf = frames_in_stream(P.stream_size, m.blocksize);
+        if (nf > P.nframes_cap) {
+            flag = 1;
+        } else if (m.table_off >= 0 && m.table_entries == nf) {
+            const uint8_t* tb = buf + m.table_off;
+            long long pos = m.first_frame;      // offset of frame j0 (warp-uniform carry)
+            for (int64_t j0 = 0; j0 < nf; j0 += 32) {
+                const int64_t j = j0 + ln;
+                long long len = 0;
+                if (j < nf) len = ((long long)tb[3 * j] << 16) | ((long long)tb[3 * j + 1] << 8) | tb[3 * j + 2];
+                long long inc = len;
+                for (int d = 1; d < 32; d <<= 1) {
+                    long long v = (long long)shfl_up64((unsigned long long)inc, d);
+                    if (ln >= d) inc += v;
+                }
+                if (j < nf) fo[j] = pos + inc - len;
+                pos += (long long)shfl64((unsigned long long)inc, 31);
+            }
+            if (ln == 0) fo[nf] = pos;
+            if (pos != nb) flag = 1;
+        } else {
+            for (int64_t j = ln; j < nf; j += 32) fo[j] = -1;
+            if (ln == 0) fo[nf] = nb;
+        }
+    }
+    if (ln == 0) {
+        P.stream_flag[k] = flag;
+        if (P.status && flag != 4) P.status[k] = 0;
+    }
 }
 
 // ---- stage 2 (foreign streams only): test byte position p of stream k for a frame header -----------
@@ -469,6 +586,25 @@ FA_D void frame_body(const DecParams& P, int64_t k, int64_t j, int64_t first, in
 }
 FA_D void frame_body(const DecParams& P, int64_t k, int64_t j) { frame_body(P, k, j, P.first, P.n_decode, k * P.n_decode); }
 
+// Work item idx of the call's index space (resolve_item) through the general decoder (k_dec_frames, after the tile path:
+// P.frame_flag set, so only the frames it flagged are decoded).
+template <bool WIN>
+FA_D void frames_item(const DecParams& P, const WinParams& W, int64_t nwin, int64_t idx) {
+    const WorkItem it = resolve_item<WIN>(P, W, nwin, idx);
+    const int64_t k = it.k;
+    if (k < 0) return;
+    if (P.stream_flag[k] != 0) return;
+    int bs = P.meta[k].blocksize;
+    int64_t j0 = it.first / bs, j1 = (it.first + it.n - 1) / bs;
+    if (j1 - j0 + 1 > it.nwin) {  // blocksize differs from the host's hint: leave the stream to the walker
+        if (it.jrel == 0) atom_or_global(&P.stream_flag[k], 1);
+        return;
+    }
+    int64_t j = j0 + it.jrel;
+    if (j > j1) return;
+    frame_body(P, k, j, it.first, it.n, it.out);
+}
+
 // (a template: the stores of fab_decode's walker stay what they were; register allocation there is sensitive to them)
 template <bool ISO>
 FA_D void walker_failed(const DecParams& P, int64_t k) {
@@ -511,5 +647,23 @@ FA_D void walker_body(const DecParams& P, int64_t k, int64_t first, int64_t n, i
 }
 template <bool ISO = false>
 FA_D void walker_body(const DecParams& P, int64_t k) { walker_body<ISO>(P, k, P.first, P.n_decode, k * P.n_decode); }
+
+// fab_decode_windows' walker (k_dec_walker_win): window w of a stream the parallel path left to it
+FA_D void walker_win(const DecParams& P, const WinParams& W, int64_t w) {
+    if (!win_valid(W, w, P.n_sel, P.stream_size)) return;
+    const long long first = W.first[w], n = W.last[w] - first;
+    if (n > 0) walker_body(P, W.stream[w], first, n, W.out[w]);
+}
+
+// fab_decode_isolated, after the walker and the restore (k_dec_fill_failed): elements i0, i0 + stride, ... of the output row
+// of stream s are overwritten with `fill` when its status is not 0.  W is the output element (uint32_t for int32 / float32,
+// unsigned long long for int64 / float64).
+template <typename W>
+FA_D void fill_failed(const int* FA_RESTRICT status, W* out, int64_t n_per_stream, W fill, int64_t s, int64_t i0,
+                      int64_t stride) {
+    if (status[s] == 0) return;
+    W* o = out + s * n_per_stream;
+    for (int64_t i = i0; i < n_per_stream; i += stride) o[i] = fill;
+}
 
 }  // namespace fa

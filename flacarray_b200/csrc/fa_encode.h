@@ -276,12 +276,8 @@ FA_D double shfl_down_d(double v, int d) {
     memcpy(&v, &u, 8);
     return v;
 }
-FA_D unsigned long long shfl_xor_u64(unsigned long long u, int m) {
-    uint32_t lo = shfl_xor((uint32_t)u, m), hi = shfl_xor((uint32_t)(u >> 32), m);
-    return ((unsigned long long)hi << 32) | lo;
-}
 FA_D unsigned long long warp_sum_u64(unsigned long long v) {
-    for (int m = 16; m >= 1; m >>= 1) v += shfl_xor_u64(v, m);
+    for (int m = 16; m >= 1; m >>= 1) v += shfl_xor64(v, m);
     return v;
 }
 // exact warp sum of 32-bit partials as a 64-bit value: two REDUX over the 16-bit halves
@@ -2399,7 +2395,7 @@ FA_D bool enc_channel_full(const EncParams& P, EncCtx& X, const int32_t* park, i
         // finest partitions: 2^gsh consecutive threads each; parameters and estimated bits computed redundantly by
         // every thread of the group
         unsigned long long gs = s;
-        for (int m = 1; m < (1 << gsh); m <<= 1) gs += shfl_xor_u64(gs, m);
+        for (int m = 1; m < (1 << gsh); m <<= 1) gs += shfl_xor64(gs, m);
         const uint32_t npart = (uint32_t)(bs >> maxp) - (part == 0 ? (uint32_t)order : 0u);
         int kf = 0;
         const uint32_t e = rice_estimate(gs, npart, kf);

@@ -181,13 +181,13 @@ FA_D bool fixed_frame_warp(const EncParams& P, uint32_t g, FxShared* ws) {
         unsigned long long seg[4];      // seg[p] = sum over this lane's partition at order p
         {
             unsigned long long v = lsum;
-            v += shfl_xor_u64(v, 1); v += shfl_xor_u64(v, 2);
+            v += shfl_xor64(v, 1); v += shfl_xor64(v, 2);
             seg[3] = v;
-            v += shfl_xor_u64(v, 4);
+            v += shfl_xor64(v, 4);
             seg[2] = v;
-            v += shfl_xor_u64(v, 8);
+            v += shfl_xor64(v, 8);
             seg[1] = v;
-            v += shfl_xor_u64(v, 16);
+            v += shfl_xor64(v, 16);
             seg[0] = v;
         }
         uint32_t best_bits = 0xFFFFFFFFu;

@@ -33,6 +33,12 @@ FA_D uint32_t shfl(uint32_t v, int src) { return __shfl_sync(0xffffffffu, v, src
 FA_D uint32_t shfl_xor(uint32_t v, int m) { return __shfl_xor_sync(0xffffffffu, v, m); }
 FA_D uint32_t shfl_up(uint32_t v, int d) { return __shfl_up_sync(0xffffffffu, v, d); }
 FA_D uint32_t shfl_down(uint32_t v, int d) { return __shfl_down_sync(0xffffffffu, v, d); }
+FA_D unsigned long long shfl64(unsigned long long v, int src) { return __shfl_sync(0xffffffffu, v, src); }
+FA_D unsigned long long shfl_up64(unsigned long long v, int d) { return __shfl_up_sync(0xffffffffu, v, d); }
+FA_D unsigned long long shfl_xor64(unsigned long long v, int m) {
+    const uint32_t lo = shfl_xor((uint32_t)v, m), hi = shfl_xor((uint32_t)(v >> 32), m);
+    return ((unsigned long long)hi << 32) | lo;
+}
 FA_D uint32_t ballot(bool p) { return __ballot_sync(0xffffffffu, p); }
 FA_D int clz32(uint32_t v) { return __clz((int)v); }
 FA_D int clz64(uint64_t v) { return __clzll((long long)v); }
@@ -226,6 +232,9 @@ inline uint32_t shfl(uint32_t v, int src) { return (uint32_t)xchg_(v, src); }
 inline uint32_t shfl_xor(uint32_t v, int m) { return (uint32_t)xchg_(v, lane() ^ m); }
 inline uint32_t shfl_up(uint32_t v, int d) { return lane() - d >= 0 ? (uint32_t)xchg_(v, lane() - d) : ((void)xchg_(v, lane()), v); }
 inline uint32_t shfl_down(uint32_t v, int d) { return lane() + d < 32 ? (uint32_t)xchg_(v, lane() + d) : ((void)xchg_(v, lane()), v); }
+inline unsigned long long shfl64(unsigned long long v, int src) { return xchg_(v, src); }
+inline unsigned long long shfl_up64(unsigned long long v, int d) { return lane() - d >= 0 ? xchg_(v, lane() - d) : ((void)xchg_(v, lane()), v); }
+inline unsigned long long shfl_xor64(unsigned long long v, int m) { return xchg_(v, lane() ^ m); }
 inline uint32_t ballot(bool p) {
     uint32_t r = 0;
     auto* b = fasim::tls.blk;

@@ -16,6 +16,7 @@
 #pragma once
 #include <type_traits>
 
+#include "fa_bits.h"
 #include "fa_quant.h"
 #include "fa_simt.h"
 
@@ -56,6 +57,24 @@ struct StatsParams {
     double* mean;
     double* std;
 };
+
+// Geometry of a call on rows [n_rows][n]: bin == 0 is one bin per row; piece == 0 is kStatsPieceBytes of samples per piece
+// (fab_row_stats), the host emulator passes smaller pieces.  Returns 0 and fills *P's geometry, or the error bits of bad
+// arguments.
+inline int stats_geometry(int64_t n_rows, int64_t n, int64_t bin, int is_int64, StatsParams* P, int64_t piece = 0) {
+    if (n_rows <= 0) return kErrZeroNstream;
+    if (n <= 0) return kErrZeroStreamsize;
+    if (bin < 0) return kErrDecodeSampleRange;
+    const int64_t len = bin == 0 || bin > n ? n : bin;
+    if (len > kStatsMaxBin) return kErrDecodeSampleRange;
+    P->is_int64 = is_int64 ? 1 : 0;
+    P->n_rows = n_rows; P->n = n; P->bin = len;
+    P->nbins = (n + len - 1) / len;
+    P->piece = piece > 0 ? piece : kStatsPieceBytes / (is_int64 ? 8 : 4);
+    P->ppb = (len + P->piece - 1) / P->piece;
+    if ((P->nbins * P->ppb + kStatsWarps - 1) / kStatsWarps > 0x7FFFFFFFll) return kErrAlloc;
+    return 0;
+}
 
 #if defined(__CUDACC__)
 FA_D double bits_to_double(unsigned long long b) { return __longlong_as_double((long long)b); }
@@ -163,11 +182,6 @@ FA_D void stat_add(StatPart& a, const StatPart& b) {
     a.q0 = lo64(q); a.q1 = hi64(q);
     a.mn = b.mn < a.mn ? b.mn : a.mn;
     a.mx = b.mx > a.mx ? b.mx : a.mx;
-}
-
-FA_D unsigned long long shfl_xor64(unsigned long long v, int m) {
-    const uint32_t lo = shfl_xor((uint32_t)v, m), hi = shfl_xor((uint32_t)(v >> 32), m);
-    return ((unsigned long long)hi << 32) | lo;
 }
 
 FA_D void stat_warp_reduce(StatPart& p) {

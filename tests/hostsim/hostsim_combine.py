@@ -1,39 +1,18 @@
-"""ctypes loader of the host emulation of fab_combine_rows (tests/hostsim/hostsim_combine.cpp), and the numpy fold the
-combined rows are compared with bit for bit.
+"""The numpy fold the combined rows of fab_combine_rows are compared with bit for bit, and the wrapper of its host
+emulation (hs_combine_rows in tests/hostsim/hostsim.cpp: 32-thread blocks, so that small arrays span several column
+chunks and long segments several row tiles).
 
 TEST HARNESS ONLY, like hostsim.py: runs the kernel body of flacarray_b200/csrc/fa_combine.h the way fab_combine_rows
 drives it, on the CPU.  Never imported by the product package.
 """
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB = None
+from hostsim import lib
+
 THREADS = 32          # threads per emulated block: a block covers THREADS * kCombineCols columns and tiles of THREADS rows
 COLS = 2
-
-
-def lib():
-    """The emulator library, built next to this file when stale."""
-    global _LIB
-    if _LIB is not None:
-        return _LIB
-    so = os.path.join(_HERE, "libhostsim_combine.so")
-    srcs = [os.path.join(_HERE, "hostsim_combine.cpp")] + [
-        os.path.join(_HERE, "..", "..", "flacarray_b200", "csrc", f) for f in ("fa_simt.h", "fa_quant.h", "fa_combine.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        subprocess.run([cxx, "-O2", "-std=c++20", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", srcs[0], "-o", so],
-                       check=True, capture_output=True)
-    L = C.CDLL(so)
-    L.hs_combine_rows.restype = C.c_int
-    L.hs_combine_rows.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64] + [C.c_void_p] * 6 + [
-        C.c_int64, C.c_void_p, C.c_int64, C.POINTER(C.c_int)]
-    _LIB = L
-    return L
 
 
 def _ptr(a):

@@ -1,40 +1,15 @@
-"""ctypes loader of the host emulation of fab_row_stats (tests/hostsim/hostsim_stats.cpp), and the pure-Python reference
-the statistics are compared with bit for bit.
+"""The pure-Python reference the statistics of fab_row_stats are compared with bit for bit, and the wrappers of its host
+emulation (hs_row_stats, hs_dbl_u256 in tests/hostsim/hostsim.cpp).
 
 TEST HARNESS ONLY, like hostsim.py: runs the kernel bodies of flacarray_b200/csrc/fa_stats.h the way fab_row_stats drives
 them, on the CPU.  Never imported by the product package.
 """
 import ctypes as C
 import math
-import os
-import subprocess
 
 import numpy as np
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB = None
-
-
-def lib():
-    """The emulator library, built next to this file when stale."""
-    global _LIB
-    if _LIB is not None:
-        return _LIB
-    so = os.path.join(_HERE, "libhostsim_stats.so")
-    srcs = [os.path.join(_HERE, "hostsim_stats.cpp")] + [
-        os.path.join(_HERE, "..", "..", "flacarray_b200", "csrc", f) for f in ("fa_simt.h", "fa_quant.h", "fa_stats.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        subprocess.run([cxx, "-O2", "-std=c++20", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", srcs[0], "-o", so],
-                       check=True, capture_output=True)
-    L = C.CDLL(so)
-    L.hs_row_stats.restype = C.c_int
-    L.hs_row_stats.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_int64] + [C.c_void_p] * 8 + [
-        C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
-    L.hs_dbl_u256.restype = C.c_double
-    L.hs_dbl_u256.argtypes = [C.c_void_p]
-    _LIB = L
-    return L
+from hostsim import lib
 
 
 def _ptr(a):
@@ -66,7 +41,7 @@ def row_stats(rows, bin=None, offsets=None, gains=None, status=None, piece=0):
                             _ptr(offsets), _ptr(gains), _ptr(status), count.ctypes.data, mn.ctypes.data, mx.ctypes.data,
                             mean.ctypes.data, std.ctypes.data, C.byref(npc), C.byref(ppb))
     if rc:
-        raise ValueError("fab_row_stats rejects these arguments")
+        raise ValueError(f"fab_row_stats rejects these arguments (error {rc})")
     return (count, mn, mx, mean, std), ppb.value
 
 

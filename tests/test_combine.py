@@ -1,4 +1,4 @@
-"""Weighted sums across streams on the CPU: the host emulation of fab_combine_rows (tests/hostsim/hostsim_combine.cpp)
+"""Weighted sums across streams on the CPU: the host emulation of fab_combine_rows (tests/hostsim/hostsim.cpp)
 against the numpy fold acc = acc + w_k * float64(x_k), bit for bit.
 
 * int32 and int64 rows of random data and of INT32 / INT64 extremes, int64 values above 2^53 (round to nearest even),

@@ -40,14 +40,6 @@ def H():
     return hostsim
 
 
-@pytest.fixture(scope="module")
-def HW():
-    import hostsim_windows
-
-    hostsim_windows.lib()
-    return hostsim_windows
-
-
 def _frames(case):
     return sum(len(f) for f in case.frames) if case.frames else 0
 
@@ -139,19 +131,48 @@ def test_valid_case_hostsim(H, case):
 
 
 @pytest.mark.parametrize("case", FC.valid_cases(), ids=_ids(FC.valid_cases()))
-def test_valid_case_hostsim_windows(HW, case):
+def test_valid_case_hostsim_windows(H, case):
     comp, st, nb = case.buffer()
     ws = np.array([w[0] for w in case.windows], np.int64)
     wf = np.array([w[1] for w in case.windows], np.int64)
     wl = np.array([w[2] for w in case.windows], np.int64)
-    data, offs, _ = HW.decode_windows(comp, st, nb, case.stream_size, ws, wf, wl, is_int64=case.is_int64, bsh=case.hint())
+    data, offs, _ = H.decode_windows(comp, st, nb, case.stream_size, ws, wf, wl, is_int64=case.is_int64, bsh=case.hint())
     for i in range(ws.size):
         assert np.array_equal(data[offs[i]:offs[i + 1]], case.window_expect(i)), (case.name, case.windows[i])
     if case.full and _frames(case) <= _MODE2_MAX_FRAMES:
         k = len(case.streams)
-        data, offs, _ = HW.decode_windows(comp, st, nb, case.stream_size, np.arange(k), np.zeros(k, np.int64),
-                                          np.full(k, case.stream_size), is_int64=case.is_int64, bsh=case.hint())
+        data, offs, _ = H.decode_windows(comp, st, nb, case.stream_size, np.arange(k), np.zeros(k, np.int64),
+                                         np.full(k, case.stream_size), is_int64=case.is_int64, bsh=case.hint())
         assert np.array_equal(data.reshape(k, -1), case.expect), case.name
+
+
+# ---- stage 1: the product's warp body against the serial reference -------------------------------------------------
+
+_ALL = FC.valid_cases() + FC.invalid_cases() + FC.damage_cases()
+
+
+def _library_case(H):
+    """Three streams of the library's own encoder (emulated): frame-size tables of 81 frames, so that the warp scan
+    carries its offset across three 32-frame chunks."""
+    rng = np.random.default_rng(5)
+    x = np.cumsum(rng.integers(-500, 501, (3, 80 * 1152 + 5)), axis=1).astype(np.int32)
+    comp, st, nb, _, _ = H.encode(x, level=0)
+    return FC.Case("library_encoded_81_frames", [bytes(comp[s:s + n]) for s, n in zip(st, nb)], x.shape[1], 1)
+
+
+@pytest.mark.parametrize("case", _ALL + (None,), ids=_ids(_ALL) + ["library_encoded_81_frames"])
+def test_meta_warp_body_matches_meta_body(H, case):
+    """k_dec_meta's warp body (lane 0 parses, the warp scans the frame-size table) and meta_body agree on the metadata,
+    the frame offsets, the stream flags and the status, with the call's channel count and with the other one (which
+    makes every stream undecodable)."""
+    case = case or _library_case(H)
+    comp, st, nb = case.buffer()
+    for nch in (case.nch, 3 - case.nch):
+        want = H.meta(comp, st, nb, case.stream_size, nch, warp=False)
+        got = H.meta(comp, st, nb, case.stream_size, nch, warp=True)
+        for name, g, w in zip(("meta", "frame offsets", "stream flags", "status"), got, want):
+            assert np.array_equal(g, w), (case.name, nch, name)
+        assert ((want[2] == 4) == (want[3] != 0)).all() and (nch == case.nch or (want[2] == 4).all()), case.name
 
 
 # ---- bad input -----------------------------------------------------------------------------------------------------
@@ -160,36 +181,24 @@ _BAD = FC.invalid_cases() + FC.damage_cases()
 
 
 @pytest.mark.parametrize("case", _BAD, ids=_ids(_BAD))
-def test_bad_case_raises(H, HW, case):
+def test_bad_case_raises(H, case):
     comp, st, nb = case.buffer()
     for mode in (0, 1, 2):
         with pytest.raises(RuntimeError, match="Decoding failed"):
             H.decode(comp, st, nb, case.stream_size, is_int64=case.is_int64, mode=mode)
     with pytest.raises(RuntimeError, match="Decoding failed"):
-        HW.decode_windows(comp, st, nb, case.stream_size, [0], [0], [case.stream_size], is_int64=case.is_int64,
-                          bsh=case.hint())
+        H.decode_windows(comp, st, nb, case.stream_size, [0], [0], [case.stream_size], is_int64=case.is_int64,
+                         bsh=case.hint())
 
 
-def _sanitizer_runtime(name):
-    cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-    try:
-        p = subprocess.run([cxx, f"-print-file-name={name}"], capture_output=True, text=True, check=True).stdout.strip()
-    except (OSError, subprocess.CalledProcessError):
-        return None
-    return p if os.path.isabs(p) and os.path.exists(p) else None
-
-
-def test_bad_cases_under_address_and_ub_sanitizers(tmp_path):
+def test_bad_cases_under_address_and_ub_sanitizers(H, tmp_path):
     """The invalid and damaged streams once more, against an ASan + UBSan build of the emulator in a child process:
     every read the kernel bodies make of bad input must stay inside the buffers (the decode must still fail)."""
-    asan, ubsan = _sanitizer_runtime("libasan.so"), _sanitizer_runtime("libubsan.so")
-    if asan is None or ubsan is None:
+    env = H.sanitizer_env()
+    if env is None:
         pytest.skip("libasan / libubsan not available")
     so = str(tmp_path / "libhostsim_asan.so")
-    cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-    subprocess.run([cxx, "-O1", "-g", "-std=c++20", "-ffp-contract=off", "-fPIC", "-shared", "-pthread",
-                    "-fsanitize=address,undefined", "-fno-sanitize-recover=undefined", "-fno-omit-frame-pointer",
-                    os.path.join(HERE, "hostsim", "hostsim.cpp"), "-o", so], check=True, capture_output=True)
+    H.build(so, H.SANITIZE)
     script = textwrap.dedent(f"""
         import sys
         sys.path[:0] = [{os.path.join(HERE, "hostsim")!r}, {HERE!r}, {os.path.dirname(HERE)!r}]
@@ -208,8 +217,6 @@ def test_bad_cases_under_address_and_ub_sanitizers(tmp_path):
                     print("no error:", case.name, mode)
         print("raised", n)
     """)
-    env = dict(os.environ, LD_PRELOAD=f"{asan} {ubsan}", ASAN_OPTIONS="detect_leaks=0:abort_on_error=0",
-               UBSAN_OPTIONS="halt_on_error=1:print_stacktrace=1", PYTHONDONTWRITEBYTECODE="1")
     r = subprocess.run([sys.executable, "-c", script], env=env, capture_output=True, text=True, timeout=900)
     out = r.stdout + r.stderr
     assert r.returncode == 0, out[-4000:]

@@ -1,5 +1,5 @@
 """Per-stream fault isolation and verify on the CPU: the host emulation of fab_decode_isolated / fab_verify
-(tests/hostsim/hostsim_isolated.cpp) on the streams of tests/flac_corpus.py.
+(tests/hostsim/hostsim.cpp) on the streams of tests/flac_corpus.py.
 
 * every bad corpus case, placed between two good streams of the same stream_size and channel count in one buffer,
   reports [0, !=0, 0]; the good rows are bit-exact and the bad row is zero -- once more under AddressSanitizer + UBSan;
@@ -34,10 +34,10 @@ def _ids(cases):
 
 @pytest.fixture(scope="module")
 def HI():
-    import hostsim_isolated
+    import hostsim
 
-    hostsim_isolated.lib()
-    return hostsim_isolated
+    hostsim.lib()
+    return hostsim
 
 
 @functools.lru_cache(maxsize=None)
@@ -80,26 +80,14 @@ def test_bad_case_isolated(HI, case):
     assert np.array_equal(vs, status), (case.name, vs, status)
 
 
-def _sanitizer_runtime(name):
-    cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-    try:
-        p = subprocess.run([cxx, f"-print-file-name={name}"], capture_output=True, text=True, check=True).stdout.strip()
-    except (OSError, subprocess.CalledProcessError):
-        return None
-    return p if os.path.isabs(p) and os.path.exists(p) else None
-
-
-def test_bad_cases_isolated_under_address_and_ub_sanitizers(tmp_path):
+def test_bad_cases_isolated_under_address_and_ub_sanitizers(HI, tmp_path):
     """The [good, bad, good] calls once more, storing and not storing, against an ASan + UBSan build of the emulator in a
     child process: every read of bad input stays inside the buffers, and every status comes out the same."""
-    asan, ubsan = _sanitizer_runtime("libasan.so"), _sanitizer_runtime("libubsan.so")
-    if asan is None or ubsan is None:
+    env = HI.sanitizer_env()
+    if env is None:
         pytest.skip("libasan / libubsan not available")
-    so = str(tmp_path / "libhostsim_isolated_asan.so")
-    cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-    subprocess.run([cxx, "-O1", "-g", "-std=c++20", "-ffp-contract=off", "-fPIC", "-shared", "-pthread",
-                    "-fsanitize=address,undefined", "-fno-sanitize-recover=undefined", "-fno-omit-frame-pointer",
-                    os.path.join(HERE, "hostsim", "hostsim_isolated.cpp"), "-o", so], check=True, capture_output=True)
+    so = str(tmp_path / "libhostsim_asan.so")
+    HI.build(so, HI.SANITIZE)
     # the good streams come from the (unsanitised) encoder emulation in this process
     inputs = tmp_path / "inputs.npz"
     arrs = {}
@@ -113,7 +101,7 @@ def test_bad_cases_isolated_under_address_and_ub_sanitizers(tmp_path):
         import sys
         import numpy as np
         sys.path[:0] = [{os.path.join(HERE, "hostsim")!r}]
-        import hostsim_isolated as HI
+        import hostsim as HI
         HI.lib({so!r})
         d = np.load({str(inputs)!r})
         ok = 0
@@ -130,8 +118,6 @@ def test_bad_cases_isolated_under_address_and_ub_sanitizers(tmp_path):
                 print("wrong:", i, s, vs)
         print("isolated", ok)
     """)
-    env = dict(os.environ, LD_PRELOAD=f"{asan} {ubsan}", ASAN_OPTIONS="detect_leaks=0:abort_on_error=0",
-               UBSAN_OPTIONS="halt_on_error=1:print_stacktrace=1", PYTHONDONTWRITEBYTECODE="1")
     r = subprocess.run([sys.executable, "-c", script], env=env, capture_output=True, text=True, timeout=900)
     out = r.stdout + r.stderr
     assert r.returncode == 0, out[-4000:]

@@ -1,4 +1,4 @@
-"""Per-stream, per-bin statistics on the CPU: the host emulation of fab_row_stats (tests/hostsim/hostsim_stats.cpp)
+"""Per-stream, per-bin statistics on the CPU: the host emulation of fab_row_stats (tests/hostsim/hostsim.cpp)
 against a pure-Python reference built from Python integers and float(int), bit for bit.
 
 * int32 and int64 rows of random data and rows made of INT32_MIN / INT32_MAX / INT64_MIN / INT64_MAX (Q reaches 2^126

@@ -14,15 +14,10 @@ from test_hostsim import _cases  # noqa: E402
 
 @pytest.fixture(scope="module")
 def H():
-    """The emulator's encoder (hostsim) and window decoder (hostsim_windows) under one name."""
-    from types import SimpleNamespace
-
     import hostsim
-    import hostsim_windows
 
     hostsim.lib()
-    hostsim_windows.lib()
-    return SimpleNamespace(encode=hostsim.encode, decode_windows=hostsim_windows.decode_windows, lib=hostsim_windows.lib)
+    return hostsim
 
 
 def _tiny():
