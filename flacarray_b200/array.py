@@ -15,7 +15,8 @@ import copy
 import numpy as np
 
 from .compress import array_compress
-from .decompress import array_combine, array_decompress_slice, array_decompress_windows, array_verify, stats_slice
+from .decompress import (array_combine, array_decompress_slice, array_decompress_windows, array_flag_ranges, array_verify,
+                         stats_slice)
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -398,6 +399,28 @@ class FlacArray:
                              stream_gains=self._stream_gains, weights=weights, groups=groups, n_groups=n_groups,
                              first_stream_sample=first, last_stream_sample=last, is_int64=self._is_int64,
                              on_error=on_error)
+
+    def flag_ranges(self, lo=None, hi=None, pad=0, keep=None, stream_slice=None, on_error="raise"):
+        """Per-stream ranges of local samples outside [lo, hi] without decompressing them into memory
+        (array_flag_ranges): glitches, samples at the ADC rails, or excursions beyond mean +- k * std from stats().
+        `lo` / `hi`: None, a scalar or one value per stream (leading shape or flat); v < lo or v > hi flags a sample of
+        value v as to_array returns it.  Each flagged sample is widened by `pad` on both sides, overlapping or touching
+        windows merge, and ranges are clipped to the samples `stream_slice` selects (normalised as stats() does).
+        `keep` selects streams as to_array does.  Returns FlagRanges(stream, first, last, nflagged) on the host: stream
+        is the flat C-order index over the leading shape and first / last are absolute sample indices, so
+        to_windows(r.stream, r.first, r.last) cuts the ranges out; nflagged (leading shape) counts each stream's flagged
+        samples, -1 for streams `keep` leaves out.  on_error="fill" returns (ranges, status) as combine() does."""
+        first, last = 0, self._stream_size
+        if stream_slice is not None:
+            first, last, step = stream_slice.indices(self._stream_size)
+            if step != 1:
+                raise ValueError("Only stream slices with a step size of 1 are supported")
+        starts = np.asarray(self._stream_starts).reshape(self._leading_shape)
+        nbytes = np.asarray(self._stream_nbytes).reshape(self._leading_shape)
+        return array_flag_ranges(self._compressed, self._stream_size, starts, nbytes,
+                                 stream_offsets=self._stream_offsets, stream_gains=self._stream_gains, lo=lo, hi=hi,
+                                 pad=pad, keep=keep, first_stream_sample=first, last_stream_sample=last,
+                                 is_int64=self._is_int64, on_error=on_error)
 
     def to_windows(self, streams, first, last):
         """Decompress many sample windows of local streams in one call.

@@ -24,6 +24,7 @@
 #include "fa_decode_tile.h"
 #include "fa_encode.h"
 #include "fa_encode_fixed.h"
+#include "fa_flags.h"
 #include "fa_quant.h"
 #include "fa_stats.h"
 
@@ -400,6 +401,24 @@ __global__ void __launch_bounds__(kCombineThreads) k_combine_rows(const CombineP
     __shared__ CombineRow sh[kCombineThreads];
     combine_segment_cta<I64, FLT, kCombineThreads>(P, s0 + blockIdx.y,
                                                    (int64_t)blockIdx.x * (kCombineThreads * kCombineCols), sh);
+}
+
+// ---- fab_flag_count / fab_flag_write (fa_flags.h): scan and write: grid = (pieces / kFlagWarps, rows of one slab), one
+// warp per piece; offsets: one warp per row
+template <bool I64>
+__global__ void __launch_bounds__(kFlagWarps * 32) k_flag_scan(const FlagParams P, int64_t row0) {
+    const int64_t pc = (int64_t)blockIdx.x * kFlagWarps + (threadIdx.x >> 5);
+    if (pc < P.ppr) flag_scan_warp<I64>(P, row0 + blockIdx.y, pc);
+}
+
+__global__ void __launch_bounds__(kFlagWarps * 32) k_flag_offsets(const FlagParams P) {
+    const int64_t row = (int64_t)blockIdx.x * kFlagWarps + (threadIdx.x >> 5);
+    if (row < P.n_rows) flag_offsets_warp(P, row);
+}
+
+__global__ void __launch_bounds__(kFlagWarps * 32) k_flag_write(const FlagParams P, int64_t row0) {
+    const int64_t pc = (int64_t)blockIdx.x * kFlagWarps + (threadIdx.x >> 5);
+    if (pc < P.ppr) flag_write_warp(P, row0 + blockIdx.y, pc);
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
@@ -1332,6 +1351,101 @@ extern "C" int fab_combine_rows(fab_ctx* ctx, const void* d_rows, int is_int64, 
             if (flt) k_combine_rows<false, true><<<grid, kCombineThreads, 0, st>>>(P, s0);
             else k_combine_rows<false, false><<<grid, kCombineThreads, 0, st>>>(P, s0);
         }
+        ctx->launches++;
+    }
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+// =================================================================================================
+// Ranges of out-of-threshold samples of decoded integer rows
+// =================================================================================================
+extern "C" int64_t fab_flag_ranges_workspace_bytes(int64_t n_rows, int64_t n, int is_int64) {
+    FlagParams P{};
+    if (flag_geometry(n_rows, n, is_int64, 0, &P)) return -1;
+    return (int64_t)flag_workspace_bytes(P);
+}
+
+// the checks both calls share: geometry, the rows and the workspace
+static int flag_setup(fab_ctx* ctx, const char* what, const void* d_rows, int is_int64, int64_t n_rows, int64_t n,
+                      const int32_t* d_status, int64_t pad, void* d_work, int64_t work_bytes, FlagParams* P) {
+    int rc = flag_geometry(n_rows, n, is_int64, pad, P);
+    if (rc) return rc;
+    if (!d_rows || !d_work) {
+        ctx->last_error = std::string(what) + ": d_rows and d_work must not be NULL";
+        return ERROR_ALLOC;
+    }
+    if (((uintptr_t)d_rows & (is_int64 ? 7 : 3)) != 0 || ((uintptr_t)d_work & 15) != 0 || ((uintptr_t)d_status & 3) != 0) {
+        ctx->last_error = std::string(what) + ": d_rows, d_status and d_work must be aligned to their element size "
+                          "(d_work to 16 bytes)";
+        return ERROR_CONVERT_TYPE;
+    }
+    if (work_bytes < 0 || (size_t)work_bytes < flag_workspace_bytes(*P)) {
+        ctx->last_error = std::string(what) + ": workspace too small (fab_flag_ranges_workspace_bytes)";
+        return ERROR_ALLOC;
+    }
+    P->rows = d_rows; P->status = d_status;
+    P->mask = (uint32_t*)d_work;
+    P->sum = (FlagPiece*)((unsigned char*)d_work + flag_mask_bytes(*P));
+    return 0;
+}
+
+extern "C" int fab_flag_count(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, const void* d_lo,
+                              const void* d_hi, const void* d_offsets, const void* d_gains, const int32_t* d_status,
+                              int64_t pad, void* d_work, int64_t work_bytes, int64_t* d_nflag, int64_t* d_nrange,
+                              void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    FlagParams P{};
+    int rc = flag_setup(ctx, "fab_flag_count", d_rows, is_int64, n_rows, n, d_status, pad, d_work, work_bytes, &P);
+    if (rc) return rc;
+    if (!d_lo || !d_hi || !d_nflag || !d_nrange) {
+        ctx->last_error = "fab_flag_count: d_lo, d_hi, d_nflag and d_nrange must not be NULL";
+        return ERROR_ALLOC;
+    }
+    if ((d_offsets == nullptr) != (d_gains == nullptr) ||
+        (((uintptr_t)d_lo | (uintptr_t)d_hi | (uintptr_t)d_nflag | (uintptr_t)d_nrange) & 7) != 0) {
+        ctx->last_error = "fab_flag_count: offsets and gains go together, and every array must be aligned to its element "
+                          "size";
+        return ERROR_CONVERT_TYPE;
+    }
+    P.lo = d_lo; P.hi = d_hi; P.offsets = d_offsets; P.gains = d_gains;
+    P.nflag = (long long*)d_nflag; P.nrange = (long long*)d_nrange;
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned gx = (unsigned)((P.ppr + kFlagWarps - 1) / kFlagWarps);
+    for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {
+        const dim3 grid(gx, (unsigned)std::min<int64_t>(65535, n_rows - r0));
+        if (is_int64) k_flag_scan<true><<<grid, kFlagWarps * 32, 0, st>>>(P, r0);
+        else k_flag_scan<false><<<grid, kFlagWarps * 32, 0, st>>>(P, r0);
+        ctx->launches++;
+    }
+    k_flag_offsets<<<(unsigned)((n_rows + kFlagWarps - 1) / kFlagWarps), kFlagWarps * 32, 0, st>>>(P);
+    ctx->launches++;
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+extern "C" int fab_flag_write(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n,
+                              const int32_t* d_status, int64_t pad, void* d_work, int64_t work_bytes, const int64_t* d_base,
+                              int64_t sample0, int64_t* d_first_out, int64_t* d_last_out, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    FlagParams P{};
+    int rc = flag_setup(ctx, "fab_flag_write", d_rows, is_int64, n_rows, n, d_status, pad, d_work, work_bytes, &P);
+    if (rc) return rc;
+    if (!d_base || !d_first_out || !d_last_out) {
+        ctx->last_error = "fab_flag_write: d_base, d_first_out and d_last_out must not be NULL";
+        return ERROR_ALLOC;
+    }
+    if ((((uintptr_t)d_base | (uintptr_t)d_first_out | (uintptr_t)d_last_out) & 7) != 0) {
+        ctx->last_error = "fab_flag_write: d_base, d_first_out and d_last_out must be aligned to 8 bytes";
+        return ERROR_CONVERT_TYPE;
+    }
+    P.base = (const long long*)d_base; P.sample0 = sample0;
+    P.first_out = (long long*)d_first_out; P.last_out = (long long*)d_last_out;
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned gx = (unsigned)((P.ppr + kFlagWarps - 1) / kFlagWarps);
+    for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {
+        const dim3 grid(gx, (unsigned)std::min<int64_t>(65535, n_rows - r0));
+        k_flag_write<<<grid, kFlagWarps * 32, 0, st>>>(P, r0);
         ctx->launches++;
     }
     FAB_CUDA(ctx, cudaGetLastError());

@@ -3,12 +3,14 @@
 flattening rules, error messages), plus on_error="fill" (per-stream fault isolation);
 array_decompress_windows: many per-stream sample windows in one decode; array_verify: check streams without
 decoding them out; array_stats: per-stream and per-bin statistics without decoding the array out; array_combine:
-per-sample weighted sums across streams without decoding the array out.  The FLAC decode, the int->float restore, the
-statistics and the sums run on the device."""
+per-sample weighted sums across streams without decoding the array out; array_flag_ranges: per-stream ranges of samples
+outside thresholds without decoding the array out.  The FLAC decode, the int->float restore, the statistics, the sums and
+the range search run on the device."""
 import numpy as np
 
-from .libflacarray import (StreamStats, check_bin, check_combine_args, check_on_error, combine_flac, decode_flac,
-                           decode_flac_float, decode_windows, is_torch, stats_flac, verify_flac)
+from .libflacarray import (FlagRanges, StreamStats, check_bin, check_combine_args, check_flag_args, check_on_error,
+                           combine_flac, decode_flac, decode_flac_float, decode_windows, flag_ranges_flac, is_torch,
+                           stats_flac, verify_flac)
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -334,3 +336,86 @@ def array_combine(
     if isolate:
         return out, status.reshape(lead)
     return out
+
+
+@function_timer
+def array_flag_ranges(
+    compressed,
+    stream_size,
+    stream_starts,
+    stream_nbytes,
+    stream_offsets=None,
+    stream_gains=None,
+    lo=None,
+    hi=None,
+    pad=0,
+    keep=None,
+    first_stream_sample=None,
+    last_stream_sample=None,
+    is_int64=False,
+    on_error="raise",
+):
+    """Per-stream ranges of samples outside [lo, hi] (glitches, samples at the ADC rails, excursions beyond N sigma)
+    without materialising the decoded array.
+
+    A sample whose value v (the value array_decompress returns) satisfies v < lo or v > hi is flagged; a threshold equal
+    to v does not flag it.  `lo` and `hi` are each None (no bound on that side), a scalar, or one value per stream shaped
+    like stream_starts or flat; at least one must be given, and lo > hi flags every sample.  Float arrays compare the
+    restored value, widened to float64, with the float64 threshold.  Integer arrays compare exactly: integer thresholds
+    are used as they are, a float lo means x < ceil(lo) and a float hi x > floor(hi).
+
+    Within samples [first_stream_sample, last_stream_sample) of each stream selected by `keep` (a boolean mask shaped
+    like stream_starts), every flagged sample j is widened to [j - pad, j + pad + 1); windows that overlap or touch are
+    merged (flagged samples j1 < j2 that follow each other share a range iff j2 - j1 <= 2 * pad + 1) and each range is
+    clipped to the sample range.  Returns FlagRanges(stream, first, last, nflagged) of int64 numpy arrays: one entry of
+    stream / first / last per range, sorted by (stream, first), with stream the flat C-order index into stream_starts
+    and first / last absolute sample indices, so array_decompress_windows(..., stream, first, last) cuts the ranges
+    out; nflagged, shaped like stream_starts, counts each stream's flagged samples before widening (-1 for streams
+    `keep` leaves out).  Compressed bytes on the device are decoded there in groups of streams; host bytes are copied
+    to the device in groups.
+
+    on_error="fill" returns (ranges, status) with the int32 status shaped like stream_starts: a stream that cannot be
+    decoded gives no ranges and nflagged -1; streams left out report 0.  Both thresholds None, NaN, boolean or
+    non-numeric thresholds, a per-stream threshold of the wrong size, a negative, boolean or non-integer pad, an empty
+    sample range and an unknown on_error raise ValueError before any device is used.  A pad longer than the stream is
+    allowed.
+    """
+    isolate = check_on_error(on_error)
+    if (stream_offsets is None) != (stream_gains is None):
+        raise RuntimeError("Offsets and gains must be given together")
+    restored = stream_offsets is not None
+    first = 0 if first_stream_sample is None else int(first_stream_sample)
+    last = int(stream_size) if last_stream_sample is None else int(last_stream_sample)
+    if first < 0 or last > stream_size:
+        raise ValueError(f"sample range [{first}, {last}) lies outside the stream of {stream_size} samples")
+    if last <= first:
+        raise ValueError(f"sample range [{first}, {last}) is empty")
+    if not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts)):
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+    lead = tuple(stream_starts.shape)
+    n_stream = int(np.prod(lead))
+    lo, hi, pad = check_flag_args(n_stream, lo, hi, pad, restored)
+    if keep is None:
+        sel = np.arange(n_stream, dtype=np.int64)
+    else:
+        k = np.asarray(_host(keep))
+        if k.dtype != np.bool_ or k.size != n_stream:
+            raise ValueError(f"keep must be a boolean mask with one entry per stream ({n_stream})")
+        sel = np.flatnonzero(k.reshape(-1))
+    nflagged = np.full(n_stream, -1, np.int64)
+    status = np.zeros(n_stream, np.int32)
+    stream = first_out = last_out = np.zeros(0, np.int64)
+    if sel.size:
+        def pick(a):
+            return None if a is None else np.asarray(_host(a)).reshape(-1)[sel]
+
+        stream, first_out, last_out, nfl, st = flag_ranges_flac(
+            compressed, pick(stream_starts), pick(stream_nbytes), int(stream_size), first, last, lo[sel], hi[sel], pad,
+            pick(stream_offsets), pick(stream_gains), is_int64, isolate)
+        stream = sel[stream]
+        nflagged[sel] = nfl
+        if isolate:
+            status[sel] = st
+    res = FlagRanges(stream, first_out, last_out, nflagged.reshape(lead))
+    return (res, status.reshape(lead)) if isolate else res

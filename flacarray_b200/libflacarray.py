@@ -12,6 +12,7 @@ There is no CPU path: without the built library or without a CUDA device these f
 """
 import collections
 import ctypes as C
+import math
 import os
 import threading
 
@@ -1214,6 +1215,169 @@ def combine_flac(compressed, starts, nbytes, stream_size, first_sample, last_sam
         if not on_dev:
             out = to_host(out)
     return out, st_all
+
+
+# -------------------------------------------------------------------------------------------------
+# Ranges of out-of-threshold samples: glitch and saturation intervals per stream, found in the decoded integers on the
+# device (fab_flag_count / fab_flag_write; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+FlagRanges = collections.namedtuple("FlagRanges", ["stream", "first", "last", "nflagged"])
+
+_I64_MIN, _I64_MAX = -(1 << 63), (1 << 63) - 1
+
+
+def _threshold(t, n_stream, name):
+    """A threshold as given: None, a Python int, or a flat numpy array (integer or float) of 1 or n_stream values.
+    Raises ValueError for booleans, non-numbers, NaN and a size that is neither a scalar nor one per stream."""
+    if t is None:
+        return None
+    if isinstance(t, (bool, np.bool_)):
+        raise ValueError(f"{name} must be a number or one number per stream, not a boolean")
+    if isinstance(t, int):
+        return t                                   # exact, whatever its size
+    a = t.cpu().numpy() if is_torch(t) else np.asarray(t)
+    if a.dtype.kind not in "iuf":
+        raise ValueError(f"{name} must be a number or one number per stream, not {a.dtype}")
+    if a.ndim and a.size != n_stream:
+        raise ValueError(f"{name} has {a.size} entries for {n_stream} streams")
+    if a.dtype.kind == "f" and np.isnan(a).any():
+        raise ValueError(f"{name} must not be NaN")
+    return a.reshape(-1)
+
+
+def _int_bounds(lo, hi, n_stream):
+    """int64 [L, H] per stream for integer streams: x is flagged iff x < L or x > H (L > H: every sample).  Integers are
+    used as they are; a float lo means x < ceil(lo) and a float hi x > floor(hi), in Python integers, so the rule holds
+    at +-2^63."""
+    def each(t, up):
+        if t is None:
+            return [_I64_MAX if up else _I64_MIN] * n_stream
+        out = []
+        for v in ([t] if isinstance(t, int) else t.tolist()):
+            if isinstance(v, float) and math.isinf(v):
+                v = _I64_MAX + 1 if v > 0 else _I64_MIN - 1     # beyond every int64 on that side
+            elif isinstance(v, float):
+                v = math.floor(v) if up else math.ceil(v)
+            out.append(int(v))
+        return out * n_stream if len(out) == 1 else out
+
+    L, H = np.empty(n_stream, np.int64), np.empty(n_stream, np.int64)
+    for k, (lv, hv) in enumerate(zip(each(lo, False), each(hi, True))):
+        if lv > hv or lv > _I64_MAX or hv < _I64_MIN:
+            lv, hv = 1, 0
+        L[k], H[k] = max(lv, _I64_MIN), min(hv, _I64_MAX)
+    return L, H
+
+
+def check_flag_args(n_stream, lo, hi, pad, is_float):
+    """The per-stream thresholds and the pad of a flag_ranges call over n_stream streams: float64 lo / hi (None: -inf /
+    +inf) for float streams, int64 bounds [L, H] for integer streams (see _int_bounds), and pad as an int.  Raises
+    ValueError when both thresholds are None, for NaN, boolean or non-numeric thresholds, a per-stream threshold of the
+    wrong size, and a pad that is negative, boolean or not an integer."""
+    if lo is None and hi is None:
+        raise ValueError("flag_ranges needs lo, hi or both")
+    lo, hi = _threshold(lo, n_stream, "lo"), _threshold(hi, n_stream, "hi")
+    if isinstance(pad, (bool, np.bool_)) or not isinstance(pad, (int, np.integer)) or int(pad) < 0:
+        raise ValueError(f"pad must be an integer >= 0, not {pad!r}")
+    pad = int(pad)
+    if not is_float:
+        L, H = _int_bounds(lo, hi, n_stream)
+        return L, H, pad
+
+    def flt(t, inf):
+        if t is None:
+            return np.full(n_stream, inf)
+        a = np.asarray(float(t) if isinstance(t, int) else t, np.float64).reshape(-1)
+        return np.ascontiguousarray(np.broadcast_to(a, (n_stream,)))
+
+    return flt(lo, -np.inf), flt(hi, np.inf), pad
+
+
+def flag_count_device(rows, is_int64, n_rows, n, lo, hi, offsets, gains, status, pad, work, nflag, nrange):
+    """Device-level fab_flag_count over CUDA tensors (work: the uint8 workspace)."""
+    dev = rows.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_flag_count(ctx.handle, _ptr(rows), 1 if is_int64 else 0, n_rows, n, _ptr(lo), _ptr(hi),
+                                       _ptr(offsets), _ptr(gains), _ptr(status), pad, _ptr(work), work.numel(),
+                                       _ptr(nflag), _ptr(nrange), st)
+        if rc != 0:
+            _check(rc, ctx, st, "Flagging")
+
+
+def flag_write_device(rows, is_int64, n_rows, n, status, pad, work, base, sample0, first, last):
+    """Device-level fab_flag_write over CUDA tensors, after flag_count_device on the same rows and workspace."""
+    dev = rows.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_flag_write(ctx.handle, _ptr(rows), 1 if is_int64 else 0, n_rows, n, _ptr(status), pad,
+                                       _ptr(work), work.numel(), _ptr(base), sample0, _ptr(first), _ptr(last), st)
+        if rc != 0:
+            _check(rc, ctx, st, "Flagging")
+
+
+def flag_ranges_flac(compressed, starts, nbytes, stream_size, first_sample, last_sample, lo, hi, pad, offsets=None,
+                     gains=None, is_int64=False, isolate=False):
+    """Ranges of out-of-threshold samples in [first_sample, last_sample) of every stream, without storing the decoded
+    array: groups of streams are decoded to integers on the device, fab_flag_count counts each group's ranges, one copy
+    of the counts sizes the group's output and fab_flag_write fills it.  The ranges stay on the device until one copy at
+    the end.  lo, hi and pad as check_flag_args returns them (float thresholds with offsets and gains, integer bounds
+    without).  Returns (stream, first, last, nflag, status) as numpy arrays, first / last as sample indices of the
+    stream; status is the int32 per-stream status with `isolate` (failed streams: no ranges, nflag -1), else None and a
+    failed decode raises."""
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
+    n_stream = h_starts.size
+    n_decode = last_sample - first_sample
+    dev = compressed.device if on_dev else _device()
+    fdt = torch.float64 if is_int64 else torch.float32
+    restore = offsets is not None
+    tdt = torch.float64 if restore else torch.int64
+    with torch.cuda.device(dev):
+        counts = torch.empty(2 * n_stream, dtype=torch.int64, device=dev)
+        nflag, nrange = counts[:n_stream], counts[n_stream:]
+        status = _status_tensor(dev, n_stream) if isolate else None
+        d_lo, d_hi = to_device(lo, dev, tdt), to_device(hi, dev, tdt)
+        d_off = to_device(offsets, dev, fdt).reshape(-1) if restore else None
+        d_gain = to_device(gains, dev, fdt).reshape(-1) if restore else None
+        row_bytes = n_decode * (8 if is_int64 else 4)
+        if on_dev:
+            ranges = _stats_ranges(n_stream, row_bytes, _STATS_GROUP_BYTES)
+        else:
+            ranges = _chunk_ranges(n_stream, row_bytes)
+        ws = int(_lib.lib().fab_flag_ranges_workspace_bytes(max(b - a for a, b in ranges), n_decode,
+                                                             1 if is_int64 else 0))
+        work = torch.empty(ws, dtype=torch.uint8, device=dev)
+        full = first_sample == 0 and last_sample == stream_size
+        parts = []
+        for a, b, rows in _decode_groups(compressed, h_starts, h_nbytes, on_dev, hint, dev, ranges, stream_size,
+                                         -1 if full else first_sample, -1 if full else last_sample, is_int64,
+                                         status=status):
+            sa = None if status is None else status[a:b]
+            flag_count_device(rows, is_int64, b - a, n_decode, d_lo[a:b], d_hi[a:b],
+                              None if d_off is None else d_off[a:b], None if d_gain is None else d_gain[a:b], sa, pad,
+                              work, nflag[a:b], nrange[a:b])
+            nr = to_host(nrange[a:b])                  # sizes the group's output
+            m = int(nr.sum())
+            if m:
+                base = to_device(np.concatenate([[0], np.cumsum(nr)[:-1]]).astype(np.int64), dev, torch.int64)
+                out = torch.empty(2 * m, dtype=torch.int64, device=dev)
+                flag_write_device(rows, is_int64, b - a, n_decode, sa, pad, work, base, first_sample, out[:m], out[m:])
+                parts.append(out)
+            del rows
+        h = to_host(torch.cat([*parts, counts]))
+        st_h = to_host(status) if isolate else None
+    firsts, lasts, o = [], [], 0
+    for t in parts:
+        m = t.numel() // 2
+        firsts.append(h[o:o + m])
+        lasts.append(h[o + m:o + 2 * m])
+        o += 2 * m
+    nfl, nrg = h[o:o + n_stream], h[o + n_stream:o + 2 * n_stream]
+    stream = np.repeat(np.arange(n_stream, dtype=np.int64), nrg)
+    cat = (lambda v: np.concatenate(v) if v else np.zeros(0, np.int64))
+    return stream, cat(firsts), cat(lasts), nfl.copy(), st_h
 
 
 # -------------------------------------------------------------------------------------------------

@@ -253,6 +253,43 @@ int fab_combine_rows(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_r
                      const int64_t* d_seg_out, int64_t n_seg, double* d_out, int64_t n_out, void* stream);
 
 /*
+ * Ranges of out-of-threshold samples of decoded integer rows (no reference equivalent): the search behind
+ * FlacArray.flag_ranges() (glitches, samples at the ADC rails, excursions beyond N sigma).  d_rows: [n_rows][n] int32
+ * (is_int64 = 0) or int64, e.g. the output of fab_decode without offsets / gains, aligned to its element size.  Sample i
+ * of row k is flagged iff its value v is below the row's low threshold or above its high one (a value equal to a
+ * threshold is not flagged):
+ *   integer rows (d_offsets = d_gains = NULL): d_lo / d_hi are int64 [n_rows] bounds L / H, and x is flagged iff
+ *            x < L or x > H (L > H flags every sample);
+ *   float rows (d_offsets, d_gains [n_rows] float32 / float64, as fab_decode takes them): d_lo / d_hi are float64
+ *            [n_rows] thresholds (-inf / +inf leave a side open), and v is fab_decode's restore of x, widened to double.
+ *            The restore is monotone in x, so each row's kept samples are one integer interval, found once per row by
+ *            binary search; offsets and coefficients must be finite.
+ * Flagged samples j1 < j2 that follow each other are in one range iff j2 - j1 <= 2 * pad + 1 (pad >= 0; larger than n
+ * is allowed); a range with first and last flagged samples js and je is [max(js - pad, 0), min(je + pad + 1, n)).
+ *
+ * Two calls on the same rows, status, pad and workspace, the second after the caller has read the counts:
+ *   fab_flag_count  writes d_nflag[k] (int64: flagged samples of row k before widening, -1 for a row with a non-zero
+ *                   d_status) and d_nrange[k] (int64: its ranges, 0 for such a row);
+ *   fab_flag_write  writes the ranges of row k, in order, to slots d_base[k] .. d_base[k] + d_nrange[k] - 1 of
+ *                   d_first_out / d_last_out (int64), as sample indices plus sample0 (the index of the rows' sample 0 in
+ *                   their streams).  d_base: int64 [n_rows].
+ * The workspace d_work (work_bytes >= fab_flag_ranges_workspace_bytes(n_rows, n, is_int64), 16-byte aligned) carries a
+ * per-row bitmask of the flagged samples and per-piece summaries from the first call to the second, so it is supplied
+ * by the caller and not taken from the context; fab_flag_ranges_workspace_bytes returns -1 for invalid arguments.
+ * d_status ([n_rows] int32, may be NULL): rows with a non-zero status are skipped.  Bad arguments return error bits
+ * (ERROR_ZERO_NSTREAM, ERROR_ZERO_STREAMSIZE, ERROR_DECODE_SAMPLE_RANGE for a negative pad, ERROR_CONVERT_TYPE for
+ * offsets without gains or a misaligned array, ERROR_ALLOC for NULL arrays or a workspace that is too small) and launch
+ * nothing.  fab_flag_count: one launch per 65535 rows and one more; fab_flag_write: one launch per 65535 rows.
+ */
+int64_t fab_flag_ranges_workspace_bytes(int64_t n_rows, int64_t n, int is_int64);
+int fab_flag_count(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, const void* d_lo,
+                   const void* d_hi, const void* d_offsets, const void* d_gains, const int32_t* d_status, int64_t pad,
+                   void* d_work, int64_t work_bytes, int64_t* d_nflag, int64_t* d_nrange, void* stream);
+int fab_flag_write(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, const int32_t* d_status,
+                   int64_t pad, void* d_work, int64_t work_bytes, const int64_t* d_base, int64_t sample0,
+                   int64_t* d_first_out, int64_t* d_last_out, void* stream);
+
+/*
  * Per-stream population standard deviation of float32 / float64 streams, in the input's type: the device side of
  * `precision` -> quanta (replaces np.std(data, axis=-1) in utils.py:282-296).  One read of the input, moments
  * accumulated in double precision; differs from numpy's pairwise single-precision sum by rounding only.
