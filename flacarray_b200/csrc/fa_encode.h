@@ -1929,9 +1929,11 @@ FA_D bool enc_channel_fast(const EncParams& P, EncCtx& X, const FrameSrc& S, int
         if (retiring) {
             sync();
             retire_copyout(P, X);
-            sync();
             X.retired = true;
         }
+        // (as in enc_channel_full: every thread is done with the copy-out of the previous frame before thread 0 packs
+        // this one into `out` and overwrites prev_g / prev_nbytes)
+        sync();
         bitpos_end = bitpos0 + (c == 0 ? 8 * frame_header_bytes(bs, f) : 0) + subframe_header_bits(0, 0, 0, 32, 0);
         if (t == 0) {
             Pk pk;
@@ -2350,6 +2352,9 @@ FA_D bool enc_channel_full(const EncParams& P, EncCtx& X, const int32_t* park, i
     if (mode == 0) return false;     // (the copy has landed: the general path may reuse the buffer)
 
     if (mode == 1) {
+        // the other paths pass a barrier before they write `out`; this one must too: the previous frame may still be
+        // copied out of `out` (top of the CTA loop), and thread 0 overwrites prev_g / prev_nbytes behind this frame
+        if (c == 0) sync();
         bitpos_end = bitpos0 + (c == 0 ? 8 * frame_header_bytes(bs, f) : 0) + subframe_header_bits(0, 0, 0, 32, 0);
         if (t == 0) {
             Pk pk;

@@ -146,10 +146,15 @@ int64_t hs_encode_bound(int64_t n_stream, int64_t stream_size, int nch, int leve
     return n_stream * (stream_header_bytes((int)nf) + nf * (16 + 2 + (int64_t)nch * (lp.blocksize * 4 + 8)));
 }
 
-// dtype: 0 i32, 1 i64, 2 f32, 3 f64.  quanta may be NULL (auto) for float input.
-int hs_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size, int level, const void* quanta,
-              uint8_t* out, int64_t cap, long long* starts, long long* nbytes, void* offsets, void* gains,
-              long long* total) {
+}  // extern "C"
+
+namespace {
+// The product's encode on the host.  stats_out / plans_out [n_stream * nframes * nch] and fixed_out [n_stream * nframes],
+// when not null, receive the records k_enc_analyze and k_enc_design left for every (frame, channel) and whether
+// k_enc_fixed took the frame (its records are then left zero).
+int run_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size, int level, const void* quanta,
+               uint8_t* out, int64_t cap, long long* starts, long long* nbytes, void* offsets, void* gains,
+               long long* total, FrameStats* stats_out, FramePlan* plans_out, uint8_t* fixed_out) {
     LevelPreset lp = level_preset(level);
     int nch = (dtype == kI64 || dtype == kF64) ? 2 : 1;
     int nf = (int)((stream_size + lp.blocksize - 1) / lp.blocksize);
@@ -214,6 +219,8 @@ int hs_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size
             fixed_frame_warp(P, (uint32_t)b, ws);
         });
     }
+    if (fixed_out)
+        for (int64_t g = 0; g < total_frames; ++g) fixed_out[g] = fsize[(size_t)g] != 0u;
     fasim::launch(1, kEncThreads, sizeof(AnShared) + 16, [&](int) {
         AnShared* ash = (AnShared*)fasim::smem();
         if (lp.blocksize == kMaxBs) analyze_fill_window(P, ash);
@@ -226,6 +233,8 @@ int hs_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size
     fasim::launch(1, 1, 0, [&](int) {
         for (int64_t i = 0; i < total_frames * nch; ++i) design_frame(P, i);
     });
+    if (stats_out) memcpy(stats_out, stats.data(), (size_t)(total_frames * nch) * sizeof(FrameStats));
+    if (plans_out) memcpy(plans_out, plan_base, (size_t)(total_frames * nch) * sizeof(FramePlan));
     // persistent CTAs: the emulator runs blocks one after the other, so one block drains every ticket
     fasim::launch(1, kEncThreads, enc_smem_bytes(nch), [&](int) {
         if (lp.max_lpc_order > 8) encode_frames_cta<12, true>(P, fasim::smem());
@@ -245,6 +254,31 @@ int hs_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size
             for (int f = 0; f < nf; ++f) finalize_entry(P, s, f, nbytes, total);
     });
     return err;
+}
+}  // namespace
+
+extern "C" {
+
+// dtype: 0 i32, 1 i64, 2 f32, 3 f64.  quanta may be NULL (auto) for float input.
+int hs_encode(const void* data, int dtype, int64_t n_stream, int64_t stream_size, int level, const void* quanta,
+              uint8_t* out, int64_t cap, long long* starts, long long* nbytes, void* offsets, void* gains,
+              long long* total) {
+    return run_encode(data, dtype, n_stream, stream_size, level, quanta, out, cap, starts, nbytes, offsets, gains, total,
+                      nullptr, nullptr, nullptr);
+}
+
+// hs_encode that also returns the analysis and design records of every (frame, channel) (see run_encode)
+int hs_encode_records(const void* data, int dtype, int64_t n_stream, int64_t stream_size, int level, const void* quanta,
+                      uint8_t* out, int64_t cap, long long* starts, long long* nbytes, void* offsets, void* gains,
+                      long long* total, FrameStats* stats_out, FramePlan* plans_out, uint8_t* fixed_out) {
+    return run_encode(data, dtype, n_stream, stream_size, level, quanta, out, cap, starts, nbytes, offsets, gains, total,
+                      stats_out, plans_out, fixed_out);
+}
+
+int hs_record_sizes(int* stats_bytes, int* plan_bytes) {
+    *stats_bytes = (int)sizeof(FrameStats);
+    *plan_bytes = (int)sizeof(FramePlan);
+    return 0;
 }
 
 // mode 0: parallel-path emulation (meta -> sync scan -> per-frame decode -> walker for flagged streams)

@@ -58,6 +58,8 @@ def lib(prebuilt=None):
     L.hs_encode_bound.argtypes = [i64, i64, C.c_int, C.c_int]
     L.hs_encode.restype = C.c_int
     L.hs_encode.argtypes = [p, C.c_int, i64, i64, C.c_int, p, p, i64, p, p, p, p, C.POINTER(C.c_longlong)]
+    L.hs_encode_records.restype = C.c_int
+    L.hs_encode_records.argtypes = L.hs_encode.argtypes + [p, p, p]
     L.hs_decode.restype = C.c_int
     L.hs_decode.argtypes = [p, p, p, i64, i64, C.c_int, i64, i64, p, C.c_int, C.POINTER(C.c_int)]
     L.hs_decode_isolated.restype = C.c_int
@@ -82,7 +84,18 @@ def lib(prebuilt=None):
 _DT = {np.dtype(np.int32): 0, np.dtype(np.int64): 1, np.dtype(np.float32): 2, np.dtype(np.float64): 3}
 
 
-def encode(arr, level=5, quanta=None):
+# csrc/fa_encode.h FrameStats and FramePlan, one record per (frame, channel)
+FRAME_STATS = np.dtype([("mode", "<i4"), ("wasted", "<i4"), ("mn", "<i4"), ("mx", "<i4"), ("bad", "<u4"), ("pad", "<u4"),
+                        ("fe", "<u8", 5), ("ac", "<f8", 13)])
+FRAME_PLAN = np.dtype([(k, "u1") for k in ("mode", "wasted", "ok0", "ok1", "ord0", "ord1", "shift1", "prec1", "wide1",
+                                           "maxp0", "maxp1")] + [("pad", "u1", 5), ("qlp", "<i2", 12),
+                                                                 ("fixed_bits", "<u4"), ("pad2", "<u4")])
+
+
+def encode(arr, level=5, quanta=None, records=False):
+    """Emulated fab_encode: (bytes, starts, nbytes, offsets, gains).  records=True appends (stats, plans, fixed):
+    FRAME_STATS and FRAME_PLAN arrays [n_stream, nframes, nch] as k_enc_analyze and k_enc_design left them, and a bool
+    array [n_stream, nframes] of the frames k_enc_fixed took (their records stay zero)."""
     L = lib()
     a = np.ascontiguousarray(arr)
     a2 = a.reshape(1, -1) if a.ndim == 1 else a.reshape(-1, a.shape[-1])
@@ -98,12 +111,23 @@ def encode(arr, level=5, quanta=None):
     gains = np.zeros(n_stream, fdt)
     q = None if quanta is None else np.ascontiguousarray(quanta, fdt)
     tot = C.c_longlong(0)
-    err = L.hs_encode(a2.ctypes.data, dt, n_stream, stream_size, level, None if q is None else q.ctypes.data,
-                      out.ctypes.data, cap, starts.ctypes.data, nbytes.ctypes.data, offs.ctypes.data,
-                      gains.ctypes.data, C.byref(tot))
+    args = [a2.ctypes.data, dt, n_stream, stream_size, level, None if q is None else q.ctypes.data, out.ctypes.data, cap,
+            starts.ctypes.data, nbytes.ctypes.data, offs.ctypes.data, gains.ctypes.data, C.byref(tot)]
+    if records:
+        sb, pb = C.c_int(0), C.c_int(0)
+        L.hs_record_sizes(C.byref(sb), C.byref(pb))
+        assert (sb.value, pb.value) == (FRAME_STATS.itemsize, FRAME_PLAN.itemsize), "FrameStats / FramePlan layout changed"
+        nf = -(-stream_size // (1152 if level <= 2 else 4096))
+        stats = np.zeros((n_stream, nf, nch), FRAME_STATS)
+        plans = np.zeros((n_stream, nf, nch), FRAME_PLAN)
+        fixed = np.zeros((n_stream, nf), np.uint8)
+        err = L.hs_encode_records(*args, stats.ctypes.data, plans.ctypes.data, fixed.ctypes.data)
+    else:
+        err = L.hs_encode(*args)
     if err:
         raise RuntimeError(f"Encoding failed, return code = {err}")
-    return out[:tot.value].copy(), starts, nbytes, offs, gains
+    res = (out[:tot.value].copy(), starts, nbytes, offs, gains)
+    return res + (stats, plans, fixed.astype(bool)) if records else res
 
 
 def _inputs(compressed, starts, nbytes):
