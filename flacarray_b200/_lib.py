@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get("FLACARRAY_B200_SO") or os.path.join(_HERE, "libflacarray_b200.so")   # (override: kernel experiments)
 _SOURCES = [os.path.join(_HERE, "csrc", f) for f in
             ("fa_api.cu", "fa_simt.h", "fa_bits.h", "fa_quant.h", "fa_encode.h", "fa_decode.h", "fa_decode_tile.h", "fa_stats.h",
-             "fa_combine.h", "fa_flags.h")]
+             "fa_combine.h", "fa_flags.h", "fa_project.h")]
 _HEADER = os.path.join(os.path.dirname(_HERE), "include", "flacarray_b200.h")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
@@ -114,6 +114,10 @@ def lib():
         L.fab_flag_count.argtypes = [_vp, _vp, _i32, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp]
         L.fab_flag_write.restype = _i32
         L.fab_flag_write.argtypes = [_vp, _vp, _i32, _i64, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp]
+        L.fab_project_rows_workspace_bytes.restype = _i64
+        L.fab_project_rows_workspace_bytes.argtypes = [_i64, _i64, _i64]
+        L.fab_project_rows.restype = _i32
+        L.fab_project_rows.argtypes = [_vp, _vp, _i32, _i64, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp]
         L.fab_float_to_int.restype = _i32
         L.fab_float_to_int.argtypes = [_vp, _vp, _i32, _i64, _i64, _vp, _vp, _vp, _vp, _vp]
         L.fab_stream_std.restype = _i32
@@ -135,7 +139,7 @@ EXPORTED = [
     "float32_to_int32", "float64_to_int64", "int64_to_float64", "int32_to_float32",
     "fab_create", "fab_destroy", "fab_last_error", "fab_launch_count", "fab_encode_bound", "fab_encode",
     "fab_encode_workspace_bytes", "fab_decode_workspace_bytes", "fab_set_workspace",
-    "fab_decode", "fab_decode_isolated", "fab_verify", "fab_decode_windows", "fab_decode_windows_workspace_bytes", "fab_row_stats", "fab_row_stats_workspace_bytes", "fab_combine_rows", "fab_flag_ranges_workspace_bytes", "fab_flag_count", "fab_flag_write", "fab_stream_std", "fab_float_to_int", "fab_int_to_float", "fab_finish", "fab_profile", "fab_profile_ms",
+    "fab_decode", "fab_decode_isolated", "fab_verify", "fab_decode_windows", "fab_decode_windows_workspace_bytes", "fab_row_stats", "fab_row_stats_workspace_bytes", "fab_combine_rows", "fab_flag_ranges_workspace_bytes", "fab_flag_count", "fab_flag_write", "fab_project_rows_workspace_bytes", "fab_project_rows", "fab_stream_std", "fab_float_to_int", "fab_int_to_float", "fab_finish", "fab_profile", "fab_profile_ms",
 ]
 
 

@@ -16,7 +16,7 @@ import numpy as np
 
 from .compress import array_compress
 from .decompress import (array_combine, array_decompress_slice, array_decompress_windows, array_flag_ranges, array_verify,
-                         stats_slice)
+                         project_slice, stats_slice)
 from .libflacarray import is_torch
 from .mpi import global_array_properties, global_bytes
 from .utils import log
@@ -421,6 +421,40 @@ class FlacArray:
                                  stream_offsets=self._stream_offsets, stream_gains=self._stream_gains, lo=lo, hi=hi,
                                  pad=pad, keep=keep, first_stream_sample=first, last_stream_sample=last,
                                  is_int64=self._is_int64, on_error=on_error)
+
+    def project(self, templates, keep=None, stream_slice=None, keep_indices=False, on_error="raise"):
+        """Per-stream projections of the local data onto templates without decompressing it into memory
+        (array_project): P[s, t] = sum_i T[t, i] * x_s[i] over the samples `stream_slice` selects (normalised as stats()
+        does).  With cm = combine(), project(cm) / (cm @ cm) is each stream's coupling to the common mode; Legendre or
+        polynomial templates give baseline coefficients, sine / cosine pairs lock-in amplitudes.  `templates`: (n,) or
+        (n_templates, n), numpy or torch.  `keep` selects streams as to_array does.  Returns float64 projections with
+        to_array's shape, the sample axis replaced by the template axis (dropped for 1-D templates): a CUDA tensor when
+        the compressed bytes are on the device, else numpy; or (projections, indices) with `keep` and `keep_indices`.
+        on_error="fill" adds the int32 status last, as stats() does; failed streams get NaN."""
+        first, last = 0, self._stream_size
+        if stream_slice is not None:
+            first, last, step = stream_slice.indices(self._stream_size)
+            if step != 1:
+                raise ValueError("Only stream slices with a step size of 1 are supported")
+        out, indices, status = project_slice(
+            self._compressed,
+            self._stream_size,
+            self._stream_starts,
+            self._stream_nbytes,
+            templates,
+            stream_offsets=self._stream_offsets,
+            stream_gains=self._stream_gains,
+            keep=keep,
+            first_stream_sample=first,
+            last_stream_sample=last,
+            is_int64=self._is_int64,
+            no_flatten=(not self._flatten_single),
+            on_error=on_error,
+        )
+        res = (out, indices) if (keep is not None and keep_indices) else (out,)
+        if status is not None:
+            res = res + (status,)
+        return res[0] if len(res) == 1 else res
 
     def to_windows(self, streams, first, last):
         """Decompress many sample windows of local streams in one call.

@@ -25,6 +25,7 @@
 #include "fa_encode.h"
 #include "fa_encode_fixed.h"
 #include "fa_flags.h"
+#include "fa_project.h"
 #include "fa_quant.h"
 #include "fa_stats.h"
 
@@ -419,6 +420,21 @@ __global__ void __launch_bounds__(kFlagWarps * 32) k_flag_offsets(const FlagPara
 __global__ void __launch_bounds__(kFlagWarps * 32) k_flag_write(const FlagParams P, int64_t row0) {
     const int64_t pc = (int64_t)blockIdx.x * kFlagWarps + (threadIdx.x >> 5);
     if (pc < P.ppr) flag_write_warp(P, row0 + blockIdx.y, pc);
+}
+
+// ---- fab_project_rows (fa_project.h): pass 1 grid = (row tiles, pieces of one slab), one CTA per (row tile, piece), CH
+// templates per chunk; pass 2 one thread per (row, template)
+template <bool I64, bool FLT, int CH>
+__global__ void __launch_bounds__(kProjectThreads, 4) k_project_piece(const ProjectParams P, int64_t piece0) {
+    typedef typename std::conditional<I64, long long, int32_t>::type T;
+    __shared__ __align__(16) T rs[kProjectThreads * (kProjectSub + 1)];
+    __shared__ __align__(16) double ts[kProjectSub * CH];
+    project_piece_cta<I64, FLT, kProjectThreads, CH>(P, (int64_t)blockIdx.x * kProjectThreads, piece0 + blockIdx.y, rs, ts);
+}
+
+__global__ void __launch_bounds__(kProjectFoldThreads) k_project_fold(const ProjectParams P) {
+    const int64_t idx = (int64_t)blockIdx.x * kProjectFoldThreads + threadIdx.x;
+    if (idx < P.n_rows * P.n_tmpl) project_fold(P, idx);
 }
 
 // ---- fab_decode_windows ------------------------------------------------------------------------------
@@ -1448,6 +1464,73 @@ extern "C" int fab_flag_write(fab_ctx* ctx, const void* d_rows, int is_int64, in
         k_flag_write<<<grid, kFlagWarps * 32, 0, st>>>(P, r0);
         ctx->launches++;
     }
+    FAB_CUDA(ctx, cudaGetLastError());
+    return 0;
+}
+
+// =================================================================================================
+// Projections of decoded integer rows onto templates
+// =================================================================================================
+static_assert(kProjectPiece == FAB_PROJECT_PIECE, "the piece length is part of fab_project_rows' contract");
+
+extern "C" int64_t fab_project_rows_workspace_bytes(int64_t n_rows, int64_t n, int64_t n_tmpl) {
+    ProjectParams P{};
+    if (project_geometry(n_rows, n, n_tmpl, &P)) return -1;
+    return (int64_t)align256((size_t)project_partials(P) * sizeof(double));
+}
+
+template <bool I64, bool FLT>
+static void launch_project_piece(const ProjectParams& P, int ch, dim3 grid, int64_t piece0, cudaStream_t st) {
+    switch (ch) {
+        case 1: k_project_piece<I64, FLT, 1><<<grid, kProjectThreads, 0, st>>>(P, piece0); break;
+        case 2: k_project_piece<I64, FLT, 2><<<grid, kProjectThreads, 0, st>>>(P, piece0); break;
+        case 4: k_project_piece<I64, FLT, 4><<<grid, kProjectThreads, 0, st>>>(P, piece0); break;
+        case 8: k_project_piece<I64, FLT, 8><<<grid, kProjectThreads, 0, st>>>(P, piece0); break;
+        default: k_project_piece<I64, FLT, kProjectMaxChunk><<<grid, kProjectThreads, 0, st>>>(P, piece0); break;
+    }
+}
+
+extern "C" int fab_project_rows(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n,
+                                const void* d_offsets, const void* d_gains, const int32_t* d_status,
+                                const double* d_templates, int64_t n_tmpl, double* d_out, void* stream) {
+    if (!ctx) return FAB_ERROR_CUDA;
+    ProjectParams P{};
+    int rc = project_geometry(n_rows, n, n_tmpl, &P);
+    if (rc) return rc;
+    if (!d_rows || !d_templates || !d_out) {
+        ctx->last_error = "fab_project_rows: d_rows, d_templates and d_out must not be NULL";
+        return ERROR_ALLOC;
+    }
+    if ((d_offsets == nullptr) != (d_gains == nullptr) || ((uintptr_t)d_rows & (is_int64 ? 7 : 3)) != 0 ||
+        (((uintptr_t)d_templates | (uintptr_t)d_out) & 7) != 0 || ((uintptr_t)d_status & 3) != 0) {
+        ctx->last_error = "fab_project_rows: offsets and gains go together, and every array must be aligned to its "
+                          "element size";
+        return ERROR_CONVERT_TYPE;
+    }
+    const int64_t gx = (n_rows + kProjectThreads - 1) / kProjectThreads;
+    const int64_t gf = (n_rows * n_tmpl + kProjectFoldThreads - 1) / kProjectFoldThreads;
+    if (gx > 0x7FFFFFFFll || gf > 0x7FFFFFFFll) return ERROR_ALLOC;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char* scr;
+    rc = ctx_scratch(ctx, align256((size_t)project_partials(P) * sizeof(double)), &scr, st);
+    if (rc) return rc;
+    P.rows = d_rows; P.offsets = d_offsets; P.gains = d_gains; P.status = d_status;
+    P.tmpl = d_templates; P.part = (double*)scr; P.out = d_out;
+    const int ch = project_chunk(n_tmpl);
+    const bool flt = d_offsets != nullptr;
+    for (int64_t p0 = 0; p0 < P.npieces; p0 += 65535) {
+        const dim3 grid((unsigned)gx, (unsigned)std::min<int64_t>(65535, P.npieces - p0));
+        if (is_int64) {
+            if (flt) launch_project_piece<true, true>(P, ch, grid, p0, st);
+            else launch_project_piece<true, false>(P, ch, grid, p0, st);
+        } else {
+            if (flt) launch_project_piece<false, true>(P, ch, grid, p0, st);
+            else launch_project_piece<false, false>(P, ch, grid, p0, st);
+        }
+        ctx->launches++;
+    }
+    k_project_fold<<<(unsigned)gf, kProjectFoldThreads, 0, st>>>(P);
+    ctx->launches++;
     FAB_CUDA(ctx, cudaGetLastError());
     return 0;
 }

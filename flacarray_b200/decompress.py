@@ -4,13 +4,14 @@ flattening rules, error messages), plus on_error="fill" (per-stream fault isolat
 array_decompress_windows: many per-stream sample windows in one decode; array_verify: check streams without
 decoding them out; array_stats: per-stream and per-bin statistics without decoding the array out; array_combine:
 per-sample weighted sums across streams without decoding the array out; array_flag_ranges: per-stream ranges of samples
-outside thresholds without decoding the array out.  The FLAC decode, the int->float restore, the statistics, the sums and
-the range search run on the device."""
+outside thresholds without decoding the array out; array_project: per-stream projections onto templates without decoding
+the array out.  The FLAC decode, the int->float restore, the statistics, the sums, the range search and the projections
+run on the device."""
 import numpy as np
 
 from .libflacarray import (FlagRanges, StreamStats, check_bin, check_combine_args, check_flag_args, check_on_error,
-                           combine_flac, decode_flac, decode_flac_float, decode_windows, flag_ranges_flac, is_torch,
-                           stats_flac, verify_flac)
+                           check_project_args, combine_flac, decode_flac, decode_flac_float, decode_windows,
+                           flag_ranges_flac, is_torch, project_flac, stats_flac, verify_flac)
 from .utils import ensure_one_element, function_timer, keep_select, select_keep_indices
 
 
@@ -419,3 +420,91 @@ def array_flag_ranges(
             status[sel] = st
     res = FlagRanges(stream, first_out, last_out, nflagged.reshape(lead))
     return (res, status.reshape(lead)) if isolate else res
+
+
+def project_slice(compressed, stream_size, stream_starts, stream_nbytes, templates, stream_offsets=None,
+                  stream_gains=None, keep=None, first_stream_sample=None, last_stream_sample=None, is_int64=False,
+                  no_flatten=False, on_error="raise"):
+    """array_project with the index tuples of the kept streams and FlacArray's flattening rule: returns (projections,
+    indices, status), status None unless on_error="fill"."""
+    isolate = check_on_error(on_error)
+    if (stream_offsets is None) != (stream_gains is None):
+        raise RuntimeError("Offsets and gains must be given together")
+    restored = stream_offsets is not None
+    first = 0 if first_stream_sample is None else int(first_stream_sample)
+    last = int(stream_size) if last_stream_sample is None else int(last_stream_sample)
+    if first < 0 or last > stream_size:
+        raise ValueError(f"sample range [{first}, {last}) lies outside the stream of {stream_size} samples")
+    if last <= first:
+        raise ValueError(f"sample range [{first}, {last}) is empty")
+    n_tmpl, one_d = check_project_args(templates, last - first)
+
+    single = not (isinstance(stream_starts, np.ndarray) or is_torch(stream_starts)) or tuple(stream_starts.shape) == (1,)
+    if single:
+        fdt = np.float64 if is_int64 else np.float32
+        stream_starts = ensure_one_element(stream_starts, np.int64)
+        stream_nbytes = ensure_one_element(stream_nbytes, np.int64)
+        if restored:
+            stream_offsets = ensure_one_element(stream_offsets, fdt)
+            stream_gains = ensure_one_element(stream_gains, fdt)
+    starts, nbytes, indices = keep_select(keep, _host(stream_starts), _host(stream_nbytes))
+    offsets = select_keep_indices(None if not restored else _host(stream_offsets), indices)
+    gains = select_keep_indices(None if not restored else _host(stream_gains), indices)
+    lead = tuple(starts.shape)
+    tail = () if one_d else (n_tmpl,)
+    if starts.size == 0:
+        out = np.zeros(lead + tail)
+        if is_torch(compressed) and compressed.is_cuda:
+            import torch
+
+            out = torch.zeros(lead + tail, dtype=torch.float64, device=compressed.device)
+        status = np.zeros(lead, np.int32)
+    else:
+        out, status = project_flac(compressed, starts, nbytes, stream_size, first, last, templates, offsets, gains,
+                                   is_int64, isolate)
+        out = out.reshape(lead + tail)
+        status = None if status is None else status.reshape(lead)
+    if single and not no_flatten:
+        out = out.reshape(tail)
+    return out, indices, (status if isolate else None)
+
+
+@function_timer
+def array_project(
+    compressed,
+    stream_size,
+    stream_starts,
+    stream_nbytes,
+    templates,
+    stream_offsets=None,
+    stream_gains=None,
+    keep=None,
+    first_stream_sample=None,
+    last_stream_sample=None,
+    is_int64=False,
+    on_error="raise",
+):
+    """Per-stream projections onto templates (common-mode couplings, baseline coefficients, lock-in amplitudes) without
+    materialising the decoded array: P[s, t] = sum_i T[t, i] * x_s[i].
+
+    Streams and samples are selected as in array_decompress_slice (`keep`, [first_stream_sample, last_stream_sample),
+    offsets and gains both or neither).  `templates`: (n,) or (n_templates, n) real numbers over the n selected samples,
+    numpy or any torch tensor; they are copied once to the device as float64.  Returns float64 projections with the shape
+    array_decompress_slice's result would have, the sample axis replaced by the template axis (dropped for 1-D
+    templates): a CUDA tensor when the compressed bytes are on the device, else numpy.
+
+    With v the row array_decompress returns, widened to float64 (float32 exactly, int64 with round to nearest even), the
+    samples are cut into pieces of PROJECT_PIECE = 4096 counted from first_stream_sample, and in plain IEEE double
+    (multiply and add each rounded, no FMA):
+        per piece j: p_j = +0.0; p_j = p_j + T[t, i] * v[i] in ascending i;  then P = +0.0; P = P + p_j in piece order
+    so the result has the same bits whatever the residency or the grouping of streams into device calls.
+
+    on_error="fill" returns (projections, status) as array_stats does: a stream that cannot be decoded gets NaN.
+    Templates that are not real numbers or are boolean, that are neither 1-D nor 2-D, whose last axis is not n or that
+    hold no template, an empty sample range and an unknown on_error raise ValueError before any device is used.
+    """
+    out, _, status = project_slice(compressed, stream_size, stream_starts, stream_nbytes, templates,
+                                   stream_offsets=stream_offsets, stream_gains=stream_gains, keep=keep,
+                                   first_stream_sample=first_stream_sample, last_stream_sample=last_stream_sample,
+                                   is_int64=is_int64, on_error=on_error)
+    return (out, status) if status is not None else out

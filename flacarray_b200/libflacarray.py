@@ -1218,6 +1218,98 @@ def combine_flac(compressed, starts, nbytes, stream_size, first_sample, last_sam
 
 
 # -------------------------------------------------------------------------------------------------
+# Projections onto templates: per-stream inner products with a few templates, folded from the decoded integers on the
+# device (fab_project_rows; no reference equivalent)
+# -------------------------------------------------------------------------------------------------
+PROJECT_PIECE = 4096              # FAB_PROJECT_PIECE: samples per partial, part of the result's definition
+
+
+def check_project_args(templates, n):
+    """The number of templates and whether they came 1-D, for templates over n samples (numpy, array-like or any torch
+    tensor; nothing is copied).  Raises ValueError for templates that are not real numbers or are boolean, are neither
+    1-D nor 2-D, whose last axis is not n, or that hold no template."""
+    if is_torch(templates):
+        shape = tuple(templates.shape)
+        real = not (templates.dtype == torch.bool or templates.is_complex())
+        kind = str(templates.dtype)
+    else:
+        a = np.asarray(templates)
+        shape = a.shape
+        real = a.dtype.kind in "iuf"
+        kind = str(a.dtype)
+    if not real:
+        raise ValueError(f"templates must be real numbers, not {kind}")
+    if len(shape) not in (1, 2):
+        raise ValueError(f"templates must be 1-D (n,) or 2-D (n_templates, n), not of shape {shape}")
+    if shape[-1] != n:
+        raise ValueError(f"templates have {shape[-1]} samples for a range of {n}")
+    n_tmpl = 1 if len(shape) == 1 else shape[0]
+    if n_tmpl == 0:
+        raise ValueError("templates hold no template")
+    return n_tmpl, len(shape) == 1
+
+
+def _templates_on(templates, dev):
+    """The templates as one contiguous float64 [n_tmpl, n] CUDA tensor on dev (one copy)."""
+    if is_torch(templates):
+        t = templates.to(device=dev, dtype=torch.float64)
+    else:
+        t = to_device(np.ascontiguousarray(templates, np.float64), dev, torch.float64)
+    return t.reshape(-1, t.shape[-1]).contiguous()
+
+
+def project_device(rows, is_int64, n_rows, n, offsets, gains, status, templates, n_tmpl, out):
+    """Device-level fab_project_rows over CUDA tensors: out [n_rows, n_tmpl] float64."""
+    dev = rows.device
+    with torch.cuda.device(dev):
+        ctx = _lib.context(dev)
+        st = _stream(dev)
+        rc = _lib.lib().fab_project_rows(ctx.handle, _ptr(rows), 1 if is_int64 else 0, n_rows, n, _ptr(offsets),
+                                         _ptr(gains), _ptr(status), _ptr(templates), n_tmpl, _ptr(out), st)
+        if rc != 0:
+            _check(rc, ctx, st, "Projecting")
+
+
+def project_flac(compressed, starts, nbytes, stream_size, first_sample, last_sample, templates, offsets=None,
+                 gains=None, is_int64=False, isolate=False):
+    """Inner products of samples [first_sample, last_sample) of every stream with every template, without storing the
+    decoded array: groups of streams are decoded to integers on the device and fab_project_rows projects each group's
+    rows.  `templates` as check_project_args accepts them, over last_sample - first_sample samples.  Returns (out
+    [n_stream, n_tmpl] float64: a CUDA tensor for device bytes, else numpy; status): status is the int32 numpy
+    per-stream status with `isolate` (failed streams: NaN), else None and a failed decode raises."""
+    h_starts, h_nbytes, on_dev, hint = _stream_index(compressed, starts, nbytes)
+    n_stream = h_starts.size
+    n_decode = last_sample - first_sample
+    dev = compressed.device if on_dev else _device()
+    fdt = torch.float64 if is_int64 else torch.float32
+    restore = offsets is not None
+    with torch.cuda.device(dev):
+        t = _templates_on(templates, dev)
+        n_tmpl = t.shape[0]
+        out = torch.empty((n_stream, n_tmpl), dtype=torch.float64, device=dev)
+        status = _status_tensor(dev, n_stream) if isolate else None
+        d_off = to_device(offsets, dev, fdt).reshape(-1) if restore else None
+        d_gain = to_device(gains, dev, fdt).reshape(-1) if restore else None
+        row_bytes = n_decode * (8 if is_int64 else 4)
+        if on_dev:
+            ranges = _stats_ranges(n_stream, row_bytes, _STATS_GROUP_BYTES)
+        else:
+            ranges = _chunk_ranges(n_stream, row_bytes)
+        full = first_sample == 0 and last_sample == stream_size
+        for a, b, rows in _decode_groups(compressed, h_starts, h_nbytes, on_dev, hint, dev, ranges, stream_size,
+                                         -1 if full else first_sample, -1 if full else last_sample, is_int64,
+                                         status=status):
+            project_device(rows, is_int64, b - a, n_decode, None if d_off is None else d_off[a:b],
+                           None if d_gain is None else d_gain[a:b], None if status is None else status[a:b], t, n_tmpl,
+                           out[a:b])
+            del rows
+        st_h = to_host(status) if isolate else None
+        if not on_dev:
+            out = to_host(out)
+    return out, st_h
+
+
+# -------------------------------------------------------------------------------------------------
 # Ranges of out-of-threshold samples: glitch and saturation intervals per stream, found in the decoded integers on the
 # device (fab_flag_count / fab_flag_write; no reference equivalent)
 # -------------------------------------------------------------------------------------------------

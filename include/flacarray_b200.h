@@ -290,6 +290,30 @@ int fab_flag_write(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_row
                    int64_t* d_first_out, int64_t* d_last_out, void* stream);
 
 /*
+ * Projections of decoded integer rows onto templates (no reference equivalent): the reduction behind
+ * FlacArray.project() (common-mode couplings, baseline coefficients, lock-in amplitudes).  d_rows: [n_rows][n] int32
+ * (is_int64 = 0) or int64, e.g. the output of fab_decode without offsets / gains, aligned to its element size.
+ * d_templates: [n_tmpl][n] double.  d_out: [n_rows][n_tmpl] double.  With v_k[i] the integer (int64 converts with round
+ * to nearest even) or, when d_offsets and d_gains ([n_rows] float32 / float64, as fab_decode takes them; both NULL for
+ * integer rows) are given, the value fab_decode's restore produces in the array's type, widened to double, the samples
+ * are cut into pieces of FAB_PROJECT_PIECE counted from sample 0 (the last one may be shorter) and, in plain IEEE double
+ * (multiply and add each rounded, never an FMA):
+ *     for each piece j:  p_j = +0.0;  for i in piece j ascending:  p_j = p_j + d_templates[t][i] * v_k[i]
+ *     d_out[k][t] = +0.0;  for j ascending:  d_out[k][t] = d_out[k][t] + p_j
+ * so the result depends on the piece length only, not on how rows are grouped into calls.  d_status ([n_rows] int32,
+ * may be NULL): rows with a non-zero status get NaN.  Bad arguments return error bits (ERROR_ZERO_NSTREAM for n_rows or
+ * n_tmpl <= 0, ERROR_ZERO_STREAMSIZE for n <= 0, ERROR_ALLOC for NULL arrays, ERROR_CONVERT_TYPE for offsets without
+ * gains or a misaligned array) and launch nothing.  Workspace: fab_project_rows_workspace_bytes (one double per row,
+ * template and piece; -1 for invalid arguments); a caller-supplied workspace that is too small fails with ERROR_ALLOC.
+ * One launch per 65535 pieces and one more.
+ */
+#define FAB_PROJECT_PIECE 4096
+int64_t fab_project_rows_workspace_bytes(int64_t n_rows, int64_t n, int64_t n_tmpl);
+int fab_project_rows(fab_ctx* ctx, const void* d_rows, int is_int64, int64_t n_rows, int64_t n, const void* d_offsets,
+                     const void* d_gains, const int32_t* d_status, const double* d_templates, int64_t n_tmpl,
+                     double* d_out, void* stream);
+
+/*
  * Per-stream population standard deviation of float32 / float64 streams, in the input's type: the device side of
  * `precision` -> quanta (replaces np.std(data, axis=-1) in utils.py:282-296).  One read of the input, moments
  * accumulated in double precision; differs from numpy's pairwise single-precision sum by rounding only.
